@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- walker-steps/s of the emcee stretch-move hot path on N B200s.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload rosenbrock2d]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload rosenbrock2d] [--dump-outputs DIR]
 
 One "step" is one complete emcee job of the workload: BASELINE.json configs[1], the 2-D
 Rosenbrock density with 2^20 walkers and 10^4 iterations per walker (API niter = 10^4 * 2^20,
@@ -403,9 +403,27 @@ class Env:
         return mx.tolist(), sm.tolist()
 
 
-def run_workload(env, km, workload, steps, warmup, launch_mode=0, tensor_cores=None, e2e_steps=3):
+def dump_outputs(out_dir, chain, logp, ratio, budget=48_000_000):
+    """Writes what one emcee job returns to its caller -- the stored chain [nw, ns, d], its log-densities [nw, ns] and
+    the accept ratio of every walker -- as float64 .npy files under out_dir, with walker_index.npy naming the walkers
+    written.  When all walkers would exceed `budget` bytes, a fixed seeded sample of walkers (sorted; the same rows in
+    every file) is written, so that two builds run with the same arguments can be compared file for file."""
+    nw = len(ratio)
+    per_walker = 8 * (chain[0].size + logp[0].size + 2)
+    keep = np.arange(nw)
+    if nw * per_walker > budget:
+        keep = np.sort(np.random.default_rng(0).choice(nw, budget // per_walker, replace=False))
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = {"chain": chain[keep], "log_density": logp[keep], "accept_ratio": ratio[keep], "walker_index": keep}
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a.astype(np.float64))
+
+
+def run_workload(env, km, workload, steps, warmup, launch_mode=0, tensor_cores=None, e2e_steps=3, keep_outputs=False):
     """Times `steps` steps (complete emcee jobs) of one workload on every rank (independent ensembles).
-    Returns the pieces of a bench line: value / ms_per_step / roofline / e2e / clocks / launches."""
+    Returns the pieces of a bench line: value / ms_per_step / roofline / e2e / clocks / launches, and with
+    keep_outputs the (chain, log-densities, accept ratios) of the last timed step."""
     torch = env.torch
     wl = WORKLOADS[workload]
     rank, world, local = env.rank, env.world, env.local
@@ -457,6 +475,7 @@ def run_workload(env, km, workload, steps, warmup, launch_mode=0, tensor_cores=N
         ms, n = samplers[i].last_run_ms()
         kern_ms.append(ms)
         launches += n
+    outputs = samplers[-1].results() if keep_outputs else None
     for s in samplers:
         s.close()
 
@@ -495,7 +514,7 @@ def run_workload(env, km, workload, steps, warmup, launch_mode=0, tensor_cores=N
     (dev_ms, e2e_ms, _, _), (_, _, _, launches) = env.max_sum([dev_ms, e2e_s * 1e3, max(kern_ms), float(launches)])
     k_ms = statistics.mean(kern_ms)
     return {
-        "wl": wl, "tensor": tensor, "k_ms": k_ms,
+        "wl": wl, "tensor": tensor, "k_ms": k_ms, "outputs": outputs,
         "per_rank": {"kernel_ms": [round(v[0], 3) for v in per_rank], "ms_per_step": [round(v[1], 3) for v in per_rank],
                      "sm_mhz": [v[2] for v in per_rank]},
         "value": world * walker_steps_per_step * steps / (dev_ms * 1e-3),
@@ -629,7 +648,12 @@ def main():
     ap.add_argument("--traffic-child", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--tensor-cores", type=int, default=None, choices=[0, 1],
                     help="force the tcgen05 (1) or FP64 (0) log-density kernel of the dense plugins")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (chain, log-densities, accept ratios; "
+                         "rank 0) to DIR/*.npy as float64, a fixed seeded sample of walkers if all would exceed 48 MB")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         return run_reference(args, wl)
@@ -640,7 +664,11 @@ def main():
     env = Env()
     rank, world = env.rank, env.world
 
-    r = run_workload(env, km, args.workload, args.steps, args.warmup, args.launch_mode, args.tensor_cores)
+    r = run_workload(env, km, args.workload, args.steps, args.warmup, args.launch_mode, args.tensor_cores,
+                     keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *r["outputs"])
+    r["outputs"] = None
     default_run = args.workload == "rosenbrock2d" and args.launch_mode == 0 and args.tensor_cores is None
 
     others = []

@@ -12,6 +12,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -28,10 +29,10 @@ class _Density(C.Structure):
                 ("nparams", C.c_int64), ("data", C.POINTER(C.c_float)), ("ndata", C.c_int64)]
 
 
-def build(native: bool = False) -> Path:
-    """Compile the oracle.  native=True builds a -march=native copy on the machine it runs on
-    (used for the CPU baseline on the GPU box); the default is a portable x86-64-v3 build."""
-    out = _HERE / ("libkmc_oracle_native.so" if native else "libkmc_oracle.so")
+def build(native: bool = False, out_dir: Path = _HERE) -> Path:
+    """Compile the oracle into out_dir.  native=True builds a -march=native copy for the machine it
+    runs on (bench.py's CPU baseline); the default is a portable x86-64-v3 build."""
+    out = Path(out_dir) / ("libkmc_oracle_native.so" if native else "libkmc_oracle.so")
     src = _HERE / "kmc_oracle.c"
     if out.exists() and out.stat().st_mtime >= src.stat().st_mtime:
         return out
@@ -45,13 +46,16 @@ _libs: dict[bool, C.CDLL] = {}
 
 def lib(native: bool = False) -> C.CDLL:
     if native not in _libs:
-        try:
-            path = build(native)
-        except Exception:
-            if not native:
-                raise
-            path = build(False)
-        L = C.CDLL(str(path))
+        if native:
+            # the native build belongs to the host it runs on, and the tree may be read-only there (bench.py):
+            # it is compiled into a temporary directory, which goes once the library is loaded
+            with tempfile.TemporaryDirectory(prefix="kmc_oracle_") as tmp:
+                try:
+                    L = C.CDLL(str(build(True, Path(tmp))))
+                except Exception:
+                    L = C.CDLL(str(build(False)))
+        else:
+            L = C.CDLL(str(build(False)))
         L.kmo_g_pdf.restype = C.c_double
         L.kmo_g_pdf.argtypes = [C.c_double, C.c_double]
         L.kmo_cdf_g_inv.restype = C.c_double

@@ -1,11 +1,13 @@
 """CPU checks of bench.py's contract pieces that need no GPU: workloads = BASELINE.json's configs, the roofline arithmetic
-(SURVEY.md section 8d), the kernel labels, the reference arm's JSON line, and the order of operations in the rank barrier."""
+(SURVEY.md section 8d), the kernel labels, the reference arm's JSON line, the order of operations in the rank barrier and
+the files of --dump-outputs; and on a GPU, that those files hold what the last timed step computed."""
 import inspect
 import json
 import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
 import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -54,6 +56,57 @@ def test_rank_barrier_synchronizes_before_the_collective():
     code = [ln.strip() for ln in src.splitlines() if ln.strip() and not ln.strip().startswith("#")]
     assert code.index("self.torch.cuda.synchronize()") < code.index("self.dist.barrier()")
     assert code.count("self.torch.cuda.synchronize()") == 2            # and again after it
+
+
+def test_dump_outputs_writes_a_fixed_bounded_sample(tmp_path):
+    """--dump-outputs: float64 .npy files, all walkers while they fit the budget, else the same seeded walker sample in
+    every file and on every run."""
+    rng = np.random.default_rng(1)
+    chain, logp, ratio = rng.standard_normal((1000, 5, 2)), rng.standard_normal((1000, 5)), rng.random(1000)
+    bench.dump_outputs(tmp_path / "all", chain, logp, ratio)
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").glob("*.npy")}
+    assert np.array_equal(got["chain"], chain) and np.array_equal(got["log_density"], logp)
+    assert np.array_equal(got["accept_ratio"], ratio) and np.array_equal(got["walker_index"], np.arange(1000))
+    budget = 100 * 8 * (10 + 5 + 2)
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, chain, logp, ratio.astype(np.float32), budget=budget)
+    a = {p.stem: np.load(p) for p in (tmp_path / "a").glob("*.npy")}
+    b = {p.stem: np.load(p) for p in (tmp_path / "b").glob("*.npy")}
+    assert sorted(a) == ["accept_ratio", "chain", "log_density", "walker_index"]
+    assert all(a[k].dtype == np.float64 and np.array_equal(a[k], b[k]) for k in a)
+    assert sum(v.nbytes for v in a.values()) <= budget
+    keep = a["walker_index"].astype(np.int64)
+    assert len(keep) == 100 and np.all(np.diff(keep) > 0)
+    assert np.array_equal(a["chain"], chain[keep]) and np.array_equal(a["log_density"], logp[keep])
+    assert np.array_equal(a["accept_ratio"], ratio.astype(np.float32)[keep])
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_those_of_the_last_timed_step(km, tmp_path):
+    """bench.py --dump-outputs on the default workload: the files hold, bit for bit, the sampled walkers of the job of
+    the last timed step (seed (warmup + steps - 1) << 8 on rank 0), and the line reports the steps asked for."""
+    steps, warmup = 2, 1
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                          "--no-others", "--no-sharded", "--no-traffic", "--no-cpu-baseline",
+                          "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600,
+                         cwd=tmp_path)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps and line["warmup"] == warmup
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").glob("*.npy")}
+    assert sum(v.nbytes for v in got.values()) <= 64 << 20
+    wl = bench.WORKLOADS["rosenbrock2d"]
+    params, x0 = bench.make_inputs(wl, 1000)
+    nitw = wl["niter_walker"]
+    s = km.Sampler(km.LogDensity("rosenbrock", 2, params), x0, nitw, nitw // 2, wl["nthin"], 2.0,
+                   seed=(warmup + steps - 1) << 8)
+    s.run(-1)
+    th, lp, ar = s.results()
+    s.close()
+    keep = got["walker_index"].astype(np.int64)
+    assert len(keep) > 0 and np.array_equal(got["walker_index"], keep)
+    assert np.array_equal(got["chain"], th[keep]) and np.array_equal(got["log_density"], lp[keep])
+    assert np.array_equal(got["accept_ratio"], ar[keep])
 
 
 def test_reference_arm_line():
