@@ -218,6 +218,31 @@ int32_t kmc_make_theta0s(kmc_density_t density, const double *theta0, const doub
 int32_t kmc_ball_randn(uint64_t seed, int64_t walker0, int64_t nwalkers, int32_t k, int32_t j, int32_t d,
                        int32_t device, double *out);
 
+/* Metropolis: batched independent random-walk chains, the reference's `metropolis` (src/samplers.jl:9-128) ---------
+ * One kmc_sampler_t holds nchains independent chains (theta0s [nchains][d], deep-copied; p0 = pdf(theta0) evaluated on
+ * the device, no error if it is -Inf).  The user closure sample_ppdf becomes a symmetric Gaussian random walk,
+ * theta1 = theta0 .+ sigma .* n with n ~ N(0, I) (mul, then add): sigma [nsigma] with nsigma = 1 (scalar) or d, finite
+ * and > 0.  Accept iff p1 - p0 > log(u) (:103; strict, FP64, NaN rejects).  The kmc_emcee_opts are reused as is:
+ * niter_walker = niter and nburnin_walker = nburnin PER CHAIN, nthin, seed, mode, device, walker_id_base = id of chain 0
+ * (ids must stay below 2^32); a_scale is not read; launch_mode, exchange, shard_* and push_* must be 0.
+ * ns = (niter - nburnin) / nthin samples per chain, accept_ratio = naccept / (niter - nburnin), accepts counted after
+ * burn-in.  Draws of step t = ni + nburnin - 1 (0-based) of chain id c are a pure function of (seed, c, t): Philox4x32-10
+ * with counter (c, t lo, t hi, 0x4D48 << 16 | pair) -> Box-Muller normals 2 pair, 2 pair + 1 from words r0, r1; the
+ * accept uniform ((r2 & 0xFFFF) << 32 | r3) * 2^-48 of pair 0.  So chain c is the same chain whatever the batch size.
+ * These take a Metropolis handle and mean the same as for emcee: kmc_emcee_run (niters = steps), _sync, _destroy,
+ * _set_stream, _nsamples, _nlocal (= nchains), _device_ptrs, _copy_results, _copy_state, _chain_moments, _squash,
+ * _progress, _last_run_ms.  kmc_emcee_set_replay, _run_half, _ipc_export, _set_peers and _window_* return
+ * KMC_ERR_STATE on it. */
+int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
+                              const double *sigma, int64_t nsigma, const kmc_emcee_opts *opts, kmc_sampler_t *out);
+/* Replay mode: normals [niters][nchains][d] and accept uniforms [niters][nchains] for the steps from the sampler's
+ * current step on (sample_ppdf and the rand() of :103).  KMC_ERR_STATE on an emcee handle. */
+int32_t kmc_metropolis_set_replay(kmc_sampler_t s, const double *normals, const double *u, int64_t niters);
+/* The normals [niters][nchains][d] and uniforms [niters][nchains] the device draws for chain ids
+ * [chain0, chain0 + nchains) at steps [t0, t0 + niters). */
+int32_t kmc_metropolis_draws(uint64_t seed, int64_t chain0, int64_t nchains, int64_t t0, int64_t niters, int32_t d,
+                             int32_t device, double *normals, double *u);
+
 /* Library-owned multi-GPU (single process, SURVEY.md section 8b: opts {devices[], sharded / independent}) -------- */
 /* One emcee run over `ndev` devices of this process.  devices[] lists CUDA ordinals (an ordinal may repeat: its
  * sub-samplers then share that GPU, which is how the sharded path is tested on one GPU).  densities[] holds one plugin

@@ -7,6 +7,7 @@ Drop-in names, argument meaning and error behaviour of the reference
           init_blobs, reduce_blob!)                               :188-216
     make_theta0s(theta0, ball_radius, logdensity, nwalkers; ...)  :311-349
     squash_walkers(thetas, accept_ratio, logdensities, blobs; ...) :372-428
+    metropolis(pdf, sample_ppdf, theta0; niter, nburnin, nthin, ...) :9-128
 
 The one deliberate difference: `logdensity` is a device plugin descriptor (`LogDensity`) and
 not a closure -- user closures cannot cross the C-ABI onto the GPU and there is no CPU
@@ -416,6 +417,158 @@ def emcee(logdensity, theta0s, *, niter=10**5, nburnin=None, nthin=1, a_scale=2.
         s.close()
     if scalar_theta:
         thetas = thetas[:, :, 0]
+    return thetas, ratio, logp, None
+
+
+# ------------------------------------------------------------------------------------------
+# metropolis  (src/samplers.jl:9-128)
+
+class NormalProposal:
+    """The proposal of a random-walk Metropolis chain in place of the closure `sample_ppdf`:
+    theta1 = theta0 .+ sigma .* randn(d), sigma a scalar or one scale per component."""
+
+    def __init__(self, sigma):
+        self.sigma = np.ascontiguousarray(np.atleast_1d(np.asarray(sigma, dtype=np.float64)).ravel())
+
+    def __repr__(self):
+        return f"NormalProposal({self.sigma.tolist() if self.sigma.size > 1 else float(self.sigma[0])})"
+
+
+def normal_proposal(sigma) -> NormalProposal:
+    """Symmetric Gaussian random walk with scale sigma (scalar or length d; finite and > 0, checked at the call)."""
+    return NormalProposal(sigma)
+
+
+def _require_proposal(sample_ppdf) -> NormalProposal:
+    if not isinstance(sample_ppdf, NormalProposal):
+        raise TypeError(
+            "the CUDA backend takes a proposal descriptor (normal_proposal(sigma)) in place of the closure "
+            "sample_ppdf: user code cannot run on the device and there is no CPU fallback")
+    return sample_ppdf
+
+
+class Metropolis(Sampler):
+    """Owns a kmc_sampler_t of nchains independent random-walk Metropolis chains.  Counts are PER CHAIN.
+    Chain c draws with id chain_id_base + c, so it is the same chain whatever the batch it runs in.  Running, results,
+    state, squash, chain moments and progress are those of Sampler; there are no half-steps and nothing to exchange."""
+
+    def __init__(self, logdensity: LogDensity, theta0s, proposal, niter, nburnin, nthin=1, seed=0, mode=MODE_PHILOX,
+                 device=None, chain_id_base=0):
+        x = np.ascontiguousarray(np.asarray(theta0s, dtype=np.float64))
+        if x.ndim == 1:
+            x = x.reshape(-1, 1)
+        self.nw, self.d = x.shape
+        self.logdensity = logdensity
+        self.proposal = _require_proposal(proposal)
+        self.opts = EmceeOpts(int(niter), int(nburnin), int(nthin), 0.0, int(seed), int(mode),
+                              int(logdensity.device if device is None else device), int(chain_id_base),
+                              0, 0, 0, 0, 0, 0, 0, 0)
+        sig = self.proposal.sigma
+        h = C.c_void_p()
+        check(lib.kmc_metropolis_create(logdensity._h, _ptr(x), self.nw, self.d, _ptr(sig), sig.size,
+                                        C.byref(self.opts), C.byref(h)))
+        self._h = h
+        n = C.c_int64()
+        check(lib.kmc_emcee_nsamples(h, C.byref(n)))
+        self.ns = n.value
+        self.nl = self.nw
+
+    def set_replay(self, normals, u):
+        """normals [steps, nchains, d] and accept uniforms [steps, nchains] from the current step on."""
+        n = np.ascontiguousarray(normals, dtype=np.float64)
+        u = np.ascontiguousarray(u, dtype=np.float64)
+        if u.size % self.nw or n.size != u.size * self.d:
+            raise ValueError("replay arrays must hold [steps, nchains, d] normals and [steps, nchains] uniforms")
+        check(lib.kmc_metropolis_set_replay(self._h, _ptr(n), _ptr(u), u.size // self.nw))
+
+
+def metropolis_draws(seed: int, chain0: int, nchains: int, t0: int, nsteps: int, d: int, device: int = 0):
+    """The normals [nsteps, nchains, d] and accept uniforms [nsteps, nchains] the DEVICE draws for chain ids
+    [chain0, chain0 + nchains) at 0-based steps [t0, t0 + nsteps)."""
+    n, u = np.empty((int(nsteps), int(nchains), int(d))), np.empty((int(nsteps), int(nchains)))
+    check(lib.kmc_metropolis_draws(int(seed), int(chain0), int(nchains), int(t0), int(nsteps), int(d), int(device),
+                                   _ptr(n), _ptr(u)))
+    return n, u
+
+
+def metropolis_randn(seed: int, chains, steps, d: int):
+    """Host restatement of the Metropolis draws of chain ids `chains` at 0-based steps `steps`: (normals
+    [len(steps), len(chains), d], uniforms [len(steps), len(chains)]).  Philox counter (chain, t lo, t hi,
+    0x4D48 << 16 | pair); the uniform ((r2 & 0xFFFF) << 32 | r3) * 2^-48 of pair 0 is exact integer arithmetic; the
+    normals are numpy's Box-Muller of words r0, r1 (the device's log / sqrt / sincospi may differ by a few ulp)."""
+    c = np.atleast_1d(np.asarray(chains, dtype=np.uint64))
+    t = np.atleast_1d(np.asarray(steps, dtype=np.uint64))
+    pair = np.arange((d + 1) // 2, dtype=np.uint64)
+    m32 = np.uint64(0xFFFFFFFF)
+    r0, r1, r2, r3 = philox4x32_10(c[None, :, None], (t & m32)[:, None, None], (t >> np.uint64(32))[:, None, None],
+                                   np.uint64(0x4D480000) | pair[None, None, :], seed, seed >> 32)
+    u = (((r2[:, :, 0] & np.uint64(0xFFFF)) << np.uint64(32)) | r3[:, :, 0]).astype(np.float64) * 2.0 ** -48
+    u1 = (r0.astype(np.float64) + 1.0) * 2.0 ** -32
+    u2 = r1.astype(np.float64) * 2.0 ** -32
+    rad = np.sqrt(-2.0 * np.log(u1))
+    z = np.stack([rad * np.cos(2 * np.pi * u2), rad * np.sin(2 * np.pi * u2)], axis=-1).reshape(len(t), len(c), -1)
+    return z[:, :, :d], u
+
+
+def metropolis(logdensity, sample_ppdf, theta0, *, niter=10**5, nburnin=None, nthin=1, use_progress_meter=True,
+               hasblob=False, seed=0, replay=None, nchains=None):
+    """Random-walk Metropolis; same call shape and 4-tuple as the reference, on the device.
+
+    `sample_ppdf` is normal_proposal(sigma) (a Python callable raises TypeError).  niter / nburnin count the steps of
+    ONE chain; ns = (niter - nburnin) // nthin.
+    nchains=None: the reference call, one chain from theta0 (scalar or [d]): returns (thetas [ns] or [ns, d],
+    accept_ratio: float, logdensities [ns], None).
+    nchains=k: k independent chains from theta0 [k] or [k, d] (chain c draws with id c): returns ([k, ns(, d)], [k],
+    [k, ns], None) -- the per-walker layout of emcee, so squash_walkers, int_acorr, eff_samples and
+    evaluate_convergence take it directly.
+    `seed` keys the Philox draws; `replay=(normals [niter, k, d], u [niter, k])` uploads the draws instead.
+    """
+    _require_plugin(logdensity)
+    proposal = _require_proposal(sample_ppdf)
+    if hasblob:
+        raise NotImplementedError("hasblob=True is not supported by the CUDA backend: blobs are arbitrary host objects")
+    if nburnin is None:
+        nburnin = niter // 2
+    d = logdensity.d
+    th = np.asarray(theta0, dtype=np.float64)  # + ascontiguousarray in Metropolis: the deepcopy of theta0
+    if nchains is None:
+        scalar_theta = th.ndim == 0
+        if th.size != d or th.ndim > 1:
+            raise ValueError(f"theta0 must be a scalar or a vector of length d={d} for one chain")
+        k = 1
+    else:
+        k = int(nchains)
+        scalar_theta = th.ndim == 1
+        if k < 1 or th.shape not in [(k, d)] + ([(k,)] if d == 1 else []):
+            raise ValueError(f"with nchains={k}, theta0 must have shape ({k}, {d})" + (f" or ({k},)" if d == 1 else ""))
+    mode = MODE_REPLAY if replay is not None else MODE_PHILOX
+    s = Metropolis(logdensity, th.reshape(k, d), proposal, niter, nburnin, nthin, seed, mode)
+    try:
+        if replay is not None:
+            s.set_replay(*replay)
+        if use_progress_meter and niter > 0:    # coarse, never per step
+            chunks = min(20, niter)
+            done, t0 = 0, time.time()
+            for c in range(chunks):
+                upto = (niter * (c + 1)) // chunks
+                s.run(upto - done)
+                done = upto
+                it, mean, sd, outl = s.progress()
+                nn = max(1, it - nburnin if it > nburnin else it)
+                sys.stderr.write(
+                    f"\rmetropolis, niter={niter}, nchains={k}: {100 * done // niter:3d}%  "
+                    f"accept_ratio_mean={mean / nn:.3g} accept_ratio_std={sd / nn:.3g} "
+                    f"accept_ratio_outliers={outl} burnin_phase={it <= nburnin} [{time.time() - t0:.1f}s]")
+            sys.stderr.write("\n")
+        else:
+            s.run(-1)
+        thetas, logp, ratio = s.results()
+    finally:
+        s.close()
+    if scalar_theta:
+        thetas = thetas[:, :, 0]
+    if nchains is None:
+        return thetas[0], float(ratio[0]), logp[0], None
     return thetas, ratio, logp, None
 
 

@@ -364,6 +364,15 @@ cudaError_t eval_on_device(const kmc_density_s &dn, const double *X, long long n
     return cudaLaunchKernel(dn.ops.eval, dim3((unsigned)((npts + 255) / 256)), dim3(256), args, 0, st);
 }
 
+int eval_launches(const kmc_density_s &dn) {
+    const bool tc = dn.tc_ok && dn.tc_on;
+    switch (dn.ops.batch) {
+        case 1: return tc ? 2 : 1;                // (split + GEMM) or the FP64 kernel
+        case 2: return tc ? 3 : 2;                // (split + GEMM + finish) or (partial sums + finish)
+        default: return 1;
+    }
+}
+
 void cache_trim() {
     std::lock_guard<std::mutex> lk(g_cache.mu);
     for (auto &kv : g_cache.free_blocks) {
@@ -611,6 +620,8 @@ int32_t kmc_emcee_destroy(kmc_sampler_t s) {
     dev_free(s->rp_partner);
     dev_free(s->rp_z);
     dev_free(s->rp_u);
+    dev_free(s->rp_n);
+    dev_free(s->d_sigma);
     dev_free(s->scratch);
     for (void *q : s->ipc_opened) cudaIpcCloseMemHandle(q);
     cudaFree(s->flags);
@@ -871,6 +882,7 @@ int32_t kmc_emcee_set_stream(kmc_sampler_t s, void *cuda_stream) {
 int32_t kmc_emcee_set_replay(kmc_sampler_t s, const int64_t *partner, const double *z, const double *u,
                              int64_t niters) {
     if (!s || !partner || !z || !u || niters < 0) return fail(KMC_ERR_INVALID, "bad argument");
+    if (s->metro) return fail(KMC_ERR_STATE, "a Metropolis handle takes its draws through kmc_metropolis_set_replay");
     if (s->opts.mode != KMC_MODE_REPLAY) return fail(KMC_ERR_STATE, "sampler is not in replay mode");
     CU_TRY(cudaSetDevice(s->opts.device));
     CU_TRY(cudaStreamSynchronize(s->stream));
@@ -900,6 +912,7 @@ int32_t kmc_emcee_set_replay(kmc_sampler_t s, const int64_t *partner, const doub
 
 int32_t kmc_emcee_run_half(kmc_sampler_t s, int64_t nhalfsteps) {
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
+    if (s->metro) return fail(KMC_ERR_STATE, "a Metropolis handle has no half-steps: use kmc_emcee_run");
     const long long remaining = 2 * s->opts.niter_walker - s->hdone;
     if (nhalfsteps < 0 || nhalfsteps > remaining) nhalfsteps = remaining;
     s->last_launches = 0;
@@ -1114,6 +1127,7 @@ int32_t kmc_emcee_run_half(kmc_sampler_t s, int64_t nhalfsteps) {
 
 int32_t kmc_emcee_run(kmc_sampler_t s, int64_t niters) {
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
+    if (s->metro) return metro_run(s, niters);
     if (s->hdone & 1) return fail(KMC_ERR_STATE, "an outer iteration is half done: finish it with kmc_emcee_run_half");
     return kmc_emcee_run_half(s, niters < 0 ? -1 : 2 * niters);
 }
@@ -1121,6 +1135,7 @@ int32_t kmc_emcee_run(kmc_sampler_t s, int64_t niters) {
 int32_t kmc_emcee_ipc_export(kmc_sampler_t s, void *handle_x, void *handle_flags) {
     if (!s || !handle_x || !handle_flags) return fail(KMC_ERR_INVALID, "NULL argument");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "CUDA IPC handles are 64 bytes");
+    if (s->metro) return fail(KMC_ERR_STATE, "Metropolis chains are independent: nothing to exchange");
     CU_TRY(cudaSetDevice(s->opts.device));
     if (s->push) return fail(KMC_ERR_STATE, "a push-exchange sampler exports its window (kmc_emcee_window_export)");
     CU_TRY(cudaIpcGetMemHandle(reinterpret_cast<cudaIpcMemHandle_t *>(handle_x), s->x));
@@ -1131,6 +1146,7 @@ int32_t kmc_emcee_ipc_export(kmc_sampler_t s, void *handle_x, void *handle_flags
 int32_t kmc_emcee_set_peers(kmc_sampler_t s, const void *handles_x, const void *handles_flags, int32_t nranks,
                             int32_t rank) {
     if (!s || !handles_x || !handles_flags) return fail(KMC_ERR_INVALID, "NULL argument");
+    if (s->metro) return fail(KMC_ERR_STATE, "Metropolis chains are independent: nothing to exchange");
     if (nranks < 1 || nranks > 8 || rank < 0 || rank >= nranks) return fail(KMC_ERR_INVALID, "bad rank / nranks (max 8)");
     if (s->push) return fail(KMC_ERR_STATE, "a push-exchange sampler attaches windows (kmc_emcee_window_attach)");
     if (s->scnt * nranks != s->nhalf || s->sbeg != (long long)rank * s->scnt)
@@ -1159,6 +1175,7 @@ int32_t kmc_emcee_set_peers(kmc_sampler_t s, const void *handles_x, const void *
 
 int32_t kmc_emcee_window_export(kmc_sampler_t s, void *handle) {
     if (!s || !handle) return fail(KMC_ERR_INVALID, "NULL argument");
+    if (s->metro) return fail(KMC_ERR_STATE, "Metropolis chains are independent: nothing to exchange");
     if (!s->push) return fail(KMC_ERR_STATE, "not a push-exchange sampler (opts.exchange = KMC_EXCHANGE_PUSH)");
     CU_TRY(cudaSetDevice(s->opts.device));
     CU_TRY(cudaIpcGetMemHandle(reinterpret_cast<cudaIpcMemHandle_t *>(handle), s->window));
@@ -1167,6 +1184,7 @@ int32_t kmc_emcee_window_export(kmc_sampler_t s, void *handle) {
 
 int32_t kmc_emcee_window_attach(kmc_sampler_t s, const void *handles, int32_t nranks, int32_t rank) {
     if (!s || !handles) return fail(KMC_ERR_INVALID, "NULL argument");
+    if (s->metro) return fail(KMC_ERR_STATE, "Metropolis chains are independent: nothing to exchange");
     if (!s->push) return fail(KMC_ERR_STATE, "not a push-exchange sampler (opts.exchange = KMC_EXCHANGE_PUSH)");
     if (nranks != s->G || rank != s->rank)
         return fail(KMC_ERR_INVALID, "the sampler's shard is rank %d of %d, got rank %d of %d", s->rank, s->G, rank, nranks);
@@ -1237,7 +1255,7 @@ int32_t kmc_emcee_progress(kmc_sampler_t s, int64_t *iters_done, double *naccept
     CU_TRY(cudaMemcpyAsync(&houtl, outl, sizeof houtl, cudaMemcpyDeviceToHost, s->stream));
     CU_TRY(cudaStreamSynchronize(s->stream));
     CU_TRY(cudaGetLastError());
-    if (iters_done) *iters_done = (s->hdone / 2);
+    if (iters_done) *iters_done = s->metro ? s->tdone : (s->hdone / 2);
     if (naccept_mean) *naccept_mean = mean;
     if (naccept_std) *naccept_std = sd;
     if (outliers) *outliers = (int64_t)houtl;
@@ -1297,11 +1315,15 @@ int32_t kmc_emcee_copy_results(kmc_sampler_t s, double *thetas, double *logp, do
         dev_free(stage);
         if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "copy_results failed: %s", cudaGetErrorString(e));
     }
-    if (accept_ratio) {  // this sampler's walkers: its slice of half 0, then of half 1
+    if (accept_ratio) {  // this sampler's walkers: its slice of half 0, then of half 1 (Metropolis: every chain)
         std::vector<unsigned> h(nl);
-        CU_TRY(cudaMemcpy(h.data(), s->nacc + s->loff, sizeof(unsigned) * s->scnt, cudaMemcpyDeviceToHost));
-        CU_TRY(cudaMemcpy(h.data() + s->scnt, s->nacc + s->hoff + s->loff, sizeof(unsigned) * s->scnt,
-                          cudaMemcpyDeviceToHost));
+        if (s->metro) {
+            CU_TRY(cudaMemcpy(h.data(), s->nacc, sizeof(unsigned) * nl, cudaMemcpyDeviceToHost));
+        } else {
+            CU_TRY(cudaMemcpy(h.data(), s->nacc + s->loff, sizeof(unsigned) * s->scnt, cudaMemcpyDeviceToHost));
+            CU_TRY(cudaMemcpy(h.data() + s->scnt, s->nacc + s->hoff + s->loff, sizeof(unsigned) * s->scnt,
+                              cudaMemcpyDeviceToHost));
+        }
         const double den = (double)(s->opts.niter_walker - s->opts.nburnin_walker);  // :291
         for (long long w = 0; w < nl; ++w) accept_ratio[w] = (double)h[w] / den;
     }

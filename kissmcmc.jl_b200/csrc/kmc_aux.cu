@@ -511,14 +511,7 @@ namespace {
 
 __device__ __forceinline__ void ball_normals(const kmc::PhiloxKeys &ks, unsigned walker, unsigned pair, unsigned kj,
                                              double &z0, double &z1) {
-    const kmc::Philox4 r = kmc::philox4x32_10(walker, pair, kj, 0x4D540000u, ks);
-    const double u1 = ((double)r.r0 + 1.0) * 0x1p-32;  // (0, 1]
-    const double u2 = (double)r.r1 * 0x1p-32;          // [0, 1)
-    const double rad = sqrt(-2.0 * log(u1));
-    double sn, cs;
-    sincospi(2.0 * u2, &sn, &cs);
-    z0 = rad * cs;
-    z1 = rad * sn;
+    kmc::philox_normals(ks, walker, pair, kj, 0x4D540000u, z0, z1);
 }
 
 // out[i][c] = the standard normals of walker widx[i] (or w0 + i), try (k, j)

@@ -121,6 +121,22 @@ __device__ __forceinline__ void draw(const PhiloxKeys &ks, uint32_t walker, uint
 #endif
 }
 
+// Two counter-based standard normals from one Philox block: words r0, r1 -> uniforms in (0, 1] and [0, 1) ->
+// Box-Muller.  c3 carries the stream tag that keeps the users of this helper apart (make_theta0s: 0x4D54 << 16,
+// metropolis: 0x4D48 << 16 | pair); the block is returned so that a caller can use r2 and r3 too.
+__device__ __forceinline__ Philox4 philox_normals(const PhiloxKeys &ks, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
+                                                  double &z0, double &z1) {
+    const Philox4 r = philox4x32_10(c0, c1, c2, c3, ks);
+    const double u1 = ((double)r.r0 + 1.0) * 0x1p-32;  // (0, 1]
+    const double u2 = (double)r.r1 * 0x1p-32;          // [0, 1)
+    const double rad = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    z0 = rad * cs;
+    z1 = rad * sn;
+    return r;
+}
+
 // ------------------------------------------------------------------ log-density plugins
 // Each plugin is a POD passed BY VALUE in the kernel arguments, so its parameters sit in the
 // constant bank and feed the FP64 pipe directly (no loads).  logpdf() follows the operation

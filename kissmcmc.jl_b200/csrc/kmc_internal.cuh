@@ -119,6 +119,12 @@ struct kmc_sampler_s {
     unsigned chunk = 0, rounds = 0, nchunks = 0, cap = 0, lag = 0;
     double *peer_recv[8] = {};
     int share = 1;  // sub-samplers sharing this device (kmc_emcee_create_multi with a repeated ordinal)
+    // Metropolis handle (kmc_metropolis_create): nw = nl = nstate = chains, scnt = chains (one "half"), steps in tdone
+    bool metro = false;
+    long long tdone = 0;
+    std::vector<double> sigma;     // [d] proposal scales: the fused kernel's by-value argument
+    double *d_sigma = nullptr;     // batched plugins: the same in device memory
+    double *rp_n = nullptr;        // replay normals [steps][chains][d] (rp_u holds the uniforms)
 };
 
 
@@ -146,5 +152,10 @@ inline unsigned push_default_lag(unsigned nchunks, int push_lag) {
 // Batched log-density of npts device-resident points with the density's plugin (any plugin), on stream st.
 cudaError_t eval_on_device(const kmc_density_s &dn, const double *X, long long npts, double *out, BatchScratch &sc,
                            cudaStream_t st);
+// Kernels eval_on_device launches for this density.
+int eval_launches(const kmc_density_s &dn);
+
+// kmc_emcee_run of a Metropolis handle (kmc_metro.cu).
+int32_t metro_run(kmc_sampler_s *s, long long nsteps);
 
 }  // namespace kmc_host

@@ -1,0 +1,201 @@
+// kmc_metro.cu -- C-ABI of the batched Metropolis sampler (the reference's `metropolis`, src/samplers.jl:9-128):
+// handle creation, replay upload, the draws entry point and the run dispatch.  A Metropolis run is a kmc_sampler_t,
+// so the result, state, statistics and squash entry points of kmc_api.cu / kmc_aux.cu serve it unchanged.
+#include <cmath>
+#include <cstring>
+
+#include "kmc_internal.cuh"
+#include "kmc_metropolis.cuh"
+
+using namespace kmc_host;
+
+namespace kmc_host {
+
+int32_t metro_run(kmc_sampler_s *s, long long nsteps) {
+    const long long remaining = s->opts.niter_walker - s->tdone;
+    if (nsteps < 0 || nsteps > remaining) nsteps = remaining;
+    s->last_launches = 0;
+    s->timed = false;
+    if (nsteps <= 0) return KMC_OK;
+    const bool replay = s->opts.mode == KMC_MODE_REPLAY;
+    const long long t0 = s->tdone, t1 = s->tdone + nsteps;
+    if (replay && (t0 < s->rp_t0 || t1 > s->rp_t0 + s->rp_niters))
+        return fail(KMC_ERR_STATE, "replay draws cover steps [%lld, %lld), asked to run steps [%lld, %lld)", s->rp_t0,
+                    s->rp_t0 + s->rp_niters, t0, t1);
+    CU_TRY(cudaSetDevice(s->opts.device));
+    kmc::MhParams p{};
+    p.x = s->x;
+    p.lp = s->lp;
+    p.nacc = s->nacc;
+    p.chain_x = s->chain_x;
+    p.chain_lp = s->chain_lp;
+    p.rp_n = s->rp_n;
+    p.rp_u = s->rp_u;
+    p.rp_t0 = s->rp_t0;
+    p.nchains = s->nw;
+    p.nburnin = s->opts.nburnin_walker;
+    p.nthin = s->opts.nthin;
+    p.keys = kmc::philox_keys(s->opts.seed);
+    p.id_base = (unsigned)s->opts.walker_id_base;
+    const int d = s->d;
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    if (!s->dn->ops.batch) {  // the whole range in one launch, state in registers
+        p.t0 = t0;
+        p.t1 = t1;
+        void *args[] = {&p, s->dn->params.data(), s->sigma.data()};
+        const unsigned grid = (unsigned)((s->nw + kmc::kMhThreads - 1) / kmc::kMhThreads);
+        CU_TRY(cudaLaunchKernel(s->dn->ops.mh[replay ? 1 : 0], dim3(grid), dim3(kmc::kMhThreads), args, 0, s->stream));
+        s->last_launches = 1;
+    } else {  // propose -> batched log-density -> accept, per step
+        const long long npair = (d + 1) / 2;
+        const unsigned gp = (unsigned)((s->nw * npair + 255) / 256), ga = (unsigned)((s->nw * 32 + 255) / 256);
+        const int per_step = 2 + eval_launches(*s->dn);
+        for (long long t = t0; t < t1; ++t) {
+            p.t0 = t;
+            p.t1 = t + 1;
+            const long long ni = t + 1 - s->opts.nburnin_walker;
+            const int store = (ni > 0 && ni % s->opts.nthin == 0) ? 1 : 0;
+            const long long sidx = store ? ni / s->opts.nthin - 1 : 0;
+            if (replay) kmc::mh_propose_kernel<true><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
+            else kmc::mh_propose_kernel<false><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
+            CU_TRY(eval_on_device(*s->dn, s->bb.Y, s->nw, s->bb.p1, s->bsc, s->stream));
+            kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, ni, store, sidx);
+            s->last_launches += per_step;
+        }
+        CU_TRY(cudaGetLastError());
+    }
+    CU_TRY(cudaEventRecord(s->ev1, s->stream));
+    s->timed = true;
+    s->tdone = t1;
+    return KMC_OK;
+}
+
+}  // namespace kmc_host
+
+extern "C" {
+
+int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
+                              const double *sigma, int64_t nsigma, const kmc_emcee_opts *opts, kmc_sampler_t *out) {
+    if (!out) return fail(KMC_ERR_INVALID, "out is NULL");
+    *out = nullptr;
+    if (!density || !theta0s || !sigma || !opts) return fail(KMC_ERR_INVALID, "NULL argument");
+    if (d != density->d) return fail(KMC_ERR_INVALID, "d=%d does not match the density (d=%d)", d, density->d);
+    if (nchains < 1) return fail(KMC_ERR_INVALID, "nchains must be >= 1");
+    if (opts->walker_id_base < 0 || opts->walker_id_base + nchains > (1LL << 32))
+        return fail(KMC_ERR_INVALID, "chain ids [%lld, %lld) do not fit the 32-bit Philox counter word",
+                    (long long)opts->walker_id_base, (long long)(opts->walker_id_base + nchains));
+    if (opts->nthin < 1) return fail(KMC_ERR_INVALID, "nthin must be >= 1");
+    if (opts->niter_walker < 0 || opts->nburnin_walker < 0) return fail(KMC_ERR_INVALID, "niter and nburnin must be >= 0");
+    if (opts->mode != KMC_MODE_PHILOX && opts->mode != KMC_MODE_REPLAY)
+        return fail(KMC_ERR_INVALID, "unknown mode %d", opts->mode);
+    if (opts->launch_mode || opts->exchange || opts->shard_begin || opts->shard_count || opts->push_chunk ||
+        opts->push_cap || opts->push_lag)
+        return fail(KMC_ERR_INVALID, "launch_mode, exchange, shard_* and push_* must be 0 for Metropolis");
+    if (nsigma != 1 && nsigma != d) return fail(KMC_ERR_INVALID, "sigma has %lld entries: give 1 or d=%d", (long long)nsigma, d);
+    for (int64_t k = 0; k < nsigma; ++k)
+        if (!(std::isfinite(sigma[k]) && sigma[k] > 0.0))
+            return fail(KMC_ERR_INVALID, "sigma[%lld] = %g: proposal scales must be finite and > 0", (long long)k, sigma[k]);
+    if (!density->ops.batch && !density->ops.mh[0])
+        return fail(KMC_ERR_UNSUPPORTED, "no Metropolis kernel for this plugin and d=%d", d);
+    if (density->ops.batch && opts->device != density->device)
+        return fail(KMC_ERR_INVALID, "the density's parameters / data live on device %d, the sampler was asked for device %d",
+                    density->device, opts->device);
+
+    CU_TRY(cudaSetDevice(opts->device));
+    auto *s = new kmc_sampler_s;
+    s->metro = true;
+    s->dn = density;
+    s->opts = *opts;
+    s->nw = s->nl = s->nstate = s->scnt = nchains;  // squash reads the counters as one block of scnt
+    s->d = d;
+    const long long nspan = opts->niter_walker - opts->nburnin_walker;
+    s->ns = nspan > 0 ? nspan / opts->nthin : 0;  // ns = (niter - nburnin) / nthin
+    s->sigma.assign(d, 0.0);
+    for (int k = 0; k < d; ++k) s->sigma[k] = sigma[nsigma == 1 ? 0 : k];
+
+    auto bail = [&](int32_t rc) {
+        kmc_emcee_destroy(s);
+        return rc;
+    };
+#define CU_TRY_S(expr)                                                                                                    \
+    do {                                                                                                                  \
+        cudaError_t e_ = (expr);                                                                                          \
+        if (e_ != cudaSuccess)                                                                                            \
+            return bail(fail(KMC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__)); \
+    } while (0)
+    CU_TRY_S(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
+    s->stream = s->own_stream;
+    CU_TRY_S(cudaEventCreate(&s->ev0));
+    CU_TRY_S(cudaEventCreate(&s->ev1));
+    CU_TRY_S(dev_alloc(&s->x, sizeof(double) * nchains * d, opts->device));
+    CU_TRY_S(dev_alloc(&s->lp, sizeof(double) * nchains, opts->device));
+    CU_TRY_S(dev_alloc(&s->nacc, sizeof(unsigned) * nchains, opts->device));
+    CU_TRY_S(dev_alloc(&s->scratch, 4 * sizeof(unsigned long long), opts->device));
+    if (s->ns > 0) {
+        CU_TRY_S(dev_alloc(&s->chain_x, sizeof(double) * s->ns * nchains * d, opts->device));
+        CU_TRY_S(dev_alloc(&s->chain_lp, sizeof(double) * s->ns * nchains, opts->device));
+    }
+    CU_TRY_S(cudaMemsetAsync(s->nacc, 0, sizeof(unsigned) * nchains, s->stream));
+    CU_TRY_S(cudaMemcpyAsync(s->x, theta0s, sizeof(double) * nchains * d, cudaMemcpyHostToDevice, s->stream));  // deep copy
+    if (density->ops.batch) {  // per-step buffers: proposals, their log-densities, accept uniforms
+        CU_TRY_S(dev_alloc(&s->bb.Y, sizeof(double) * nchains * d, opts->device));
+        CU_TRY_S(dev_alloc(&s->bb.u, sizeof(double) * nchains, opts->device));
+        CU_TRY_S(dev_alloc(&s->bb.p1, sizeof(double) * nchains, opts->device));
+        CU_TRY_S(dev_alloc(&s->d_sigma, sizeof(double) * d, opts->device));
+        CU_TRY_S(cudaMemcpyAsync(s->d_sigma, s->sigma.data(), sizeof(double) * d, cudaMemcpyHostToDevice, s->stream));
+    }
+    CU_TRY_S(eval_on_device(*density, s->x, nchains, s->lp, s->bsc, s->stream));  // p0 = pdf(theta0)
+    CU_TRY_S(cudaStreamSynchronize(s->stream));
+#undef CU_TRY_S
+    *out = s;
+    return KMC_OK;
+}
+
+int32_t kmc_metropolis_set_replay(kmc_sampler_t s, const double *normals, const double *u, int64_t niters) {
+    if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
+    if (!s->metro) return fail(KMC_ERR_STATE, "not a Metropolis handle: use kmc_emcee_set_replay");
+    if (s->opts.mode != KMC_MODE_REPLAY) return fail(KMC_ERR_STATE, "sampler is not in replay mode");
+    if (niters < 0 || (niters > 0 && (!normals || !u))) return fail(KMC_ERR_INVALID, "bad argument");
+    CU_TRY(cudaSetDevice(s->opts.device));
+    CU_TRY(cudaStreamSynchronize(s->stream));
+    dev_free(s->rp_n);
+    dev_free(s->rp_u);
+    s->rp_n = s->rp_u = nullptr;
+    s->rp_niters = 0;
+    const long long n = niters * s->nw;
+    if (n > 0) {
+        CU_TRY(dev_alloc(&s->rp_n, sizeof(double) * n * s->d, s->opts.device));
+        CU_TRY(dev_alloc(&s->rp_u, sizeof(double) * n, s->opts.device));
+        CU_TRY(cudaMemcpy(s->rp_n, normals, sizeof(double) * n * s->d, cudaMemcpyHostToDevice));
+        CU_TRY(cudaMemcpy(s->rp_u, u, sizeof(double) * n, cudaMemcpyHostToDevice));
+    }
+    s->rp_t0 = s->tdone;
+    s->rp_niters = niters;
+    return KMC_OK;
+}
+
+int32_t kmc_metropolis_draws(uint64_t seed, int64_t chain0, int64_t nchains, int64_t t0, int64_t niters, int32_t d,
+                             int32_t device, double *normals, double *u) {
+    if (chain0 < 0 || nchains < 0 || chain0 + nchains > (1LL << 32) || t0 < 0 || niters < 0 || d < 1)
+        return fail(KMC_ERR_INVALID, "bad argument");
+    const long long n = nchains * niters;
+    if (n == 0) return KMC_OK;
+    if (!normals || !u) return fail(KMC_ERR_INVALID, "NULL output");
+    CU_TRY(cudaSetDevice(device));
+    double *dn = nullptr, *du = nullptr;
+    CU_TRY(dev_alloc(&dn, sizeof(double) * n * d, device));
+    cudaError_t e = dev_alloc(&du, sizeof(double) * n, device);
+    if (e == cudaSuccess) {
+        const long long ne = n * ((d + 1) / 2);
+        kmc::mh_draws_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(kmc::philox_keys(seed), (unsigned)chain0, nchains, t0,
+                                                                     niters, d, dn, du);
+        e = cudaMemcpy(normals, dn, sizeof(double) * n * d, cudaMemcpyDeviceToHost);
+    }
+    if (e == cudaSuccess) e = cudaMemcpy(u, du, sizeof(double) * n, cudaMemcpyDeviceToHost);
+    dev_free(dn);
+    dev_free(du);
+    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "metropolis_draws failed: %s", cudaGetErrorString(e));
+    return KMC_OK;
+}
+
+}  // extern "C"

@@ -17,6 +17,7 @@ struct Ops {
     int min_blocks = 1;          // CTAs per SM the kernels are compiled for
     int batch = 0;               // 0: fused thread-per-walker kernels; 1: wide Gaussian; 2: logistic (kmc_batched.cuh)
     const void *eval = nullptr;
+    const void *mh[2] = {nullptr, nullptr};  // [replay] metropolis_kernel (kmc_metropolis.cuh)
     size_t dn_bytes = 0;
     int nparams = 0;
 };
@@ -33,6 +34,7 @@ bool ops_lognormal(int d, Ops &o);
 #ifdef KMC_OPS_IMPL  // only the kmc_ops_*.cu translation units instantiate kernels
 #include "kmc_kernels.cuh"
 #include "kmc_push.cuh"
+#include "kmc_metropolis.cuh"
 
 namespace kmc_host {
 
@@ -58,6 +60,8 @@ Ops make_ops() {
     o.block = kmc::max_threads<D>();
     o.min_blocks = kmc::min_blocks<D>();
     o.eval = (const void *)kmc::density_eval_kernel<Dn, D>;
+    o.mh[0] = (const void *)kmc::metropolis_kernel<Dn, D, false>;
+    o.mh[1] = (const void *)kmc::metropolis_kernel<Dn, D, true>;
     o.dn_bytes = sizeof(Dn<D>);
     o.nparams = Dn<D>::nparams;
     return o;

@@ -6,8 +6,10 @@
 #     emcee(logdensity, theta0s; niter, nburnin, nthin, a_scale, use_progress_meter, hasblob, ...)
 #     make_theta0s(theta0, ball_radius, logdensity, nwalkers; ...)
 #     squash_walkers(thetas, accept_ratio, logdensities, blobs; ...)   (unchanged: host side)
+#     metropolis(logdensity, sample_ppdf, theta0; niter, nburnin, nthin, ...)
 #
-# with ONE difference: `logdensity` is a `LogDensity` plugin descriptor instead of a closure
+# with ONE difference: `logdensity` is a `LogDensity` plugin descriptor instead of a closure (and metropolis's
+# `sample_ppdf` a `NormalProposal`)
 # (closures cannot cross the C-ABI onto the GPU; there is no CPU fallback and no CUDA.jl).
 #
 # NOTE: Julia is not installed in the build image, so this module has not been executed
@@ -16,7 +18,7 @@
 module CUDABackend
 
 export LogDensity, exponential, rosenbrock, gaussian, lognormal, logistic, set_option!, info, emcee, emcee_squashed,
-       make_theta0s, g_pdf, cdf_g_inv, sample_g
+       make_theta0s, g_pdf, cdf_g_inv, sample_g, NormalProposal, normal_proposal, metropolis
 
 using LinearAlgebra: cholesky, Symmetric, diag, inv
 import ..KissMCMC: squash_walkers   # host-side, reused as is (src/samplers.jl:372-428)
@@ -342,6 +344,75 @@ function make_theta0s(theta0::T, ball_radius, ld::LogDensity, nwalkers; ball_rad
         (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Int32, Int32, UInt64, Ptr{Float64}, Ref{Int64}),
         ld.handle, th0, br, nwalkers, ball_radius_halfing_steps, ntries, seed, out, nf))
     return T <: Number ? [out[1, c] for c in 1:nf[]] : [T(out[:, c]) for c in 1:nf[]]
+end
+
+# ------------------------------------------------------------------ metropolis (src/samplers.jl:9-128)
+"Symmetric Gaussian random walk `theta1 = theta0 .+ sigma .* randn(d)` in place of the closure `sample_ppdf`."
+struct NormalProposal
+    sigma::Vector{Float64}       # one scale, or one per component; finite and > 0 (checked by the library)
+end
+normal_proposal(sigma::Real) = NormalProposal(Float64[sigma])
+normal_proposal(sigma::AbstractVector{<:Real}) = NormalProposal(Float64.(sigma))
+
+"""
+    metropolis(logdensity::LogDensity, proposal::NormalProposal, theta0; niter=10^5, nburnin=niter÷2, nthin=1,
+               use_progress_meter=true, hasblob=false, seed=0, nchains=nothing, device=logdensity.device)
+
+Same semantics and 4-tuple as `KissMCMC.metropolis`: `(thetas::Vector{T}, accept_ratio::Float64,
+logdensities::Vector{Float64}, nothing)`; `niter` counts the steps of one chain.  With `nchains=k`, `theta0` is a
+vector of k starting points and every element of the tuple holds one entry per independent chain (chain c draws
+with id c - 1, so it is the same chain whatever k is).
+"""
+function metropolis(ld::LogDensity, proposal::NormalProposal, theta0; niter=10^5, nburnin=niter ÷ 2, nthin=1,
+                    use_progress_meter=true, hasblob=false, seed::Integer=0, nchains=nothing,
+                    device::Integer=ld.device)
+    hasblob && error("hasblob=true is not supported by the CUDA backend (blobs are host objects)")
+    starts = nchains === nothing ? [deepcopy(theta0)] : deepcopy(theta0)
+    nchains === nothing || @assert length(starts) == nchains "theta0 must hold nchains starting points"
+    x0 = to_matrix(starts)                                                  # d x nchains
+    d, k = size(x0)
+    opts = Ref(EmceeOpts(niter, nburnin, nthin, 0.0, UInt64(seed), MODE_PHILOX, device, 0, 0, 0, 0, 0, 0, 0, 0, 0))
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    sig = proposal.sigma
+    GC.@preserve x0 sig check(ccall((:kmc_metropolis_create, LIB[]), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Int64, Ref{EmceeOpts}, Ref{Ptr{Cvoid}}),
+        ld.handle, x0, k, d, sig, length(sig), opts, h))
+    s = h[]
+    try
+        if use_progress_meter && niter > 0                 # coarse: at most 20 polls, never per step
+            done = 0
+            for c in 1:min(20, niter)
+                upto = (niter * c) ÷ min(20, niter)
+                check(ccall((:kmc_emcee_run, LIB[]), Int32, (Ptr{Cvoid}, Int64), s, upto - done))
+                done = upto
+                it, m, sd, outl = Ref{Int64}(0), Ref{Float64}(0), Ref{Float64}(0), Ref{Int64}(0)
+                check(ccall((:kmc_emcee_progress, LIB[]), Int32,
+                    (Ptr{Cvoid}, Ref{Int64}, Ref{Float64}, Ref{Float64}, Ref{Int64}), s, it, m, sd, outl))
+                nn = max(1, it[] > nburnin ? it[] - nburnin : it[])
+                print(stderr, "\rmetropolis, niter=$niter, nchains=$k: $(100done ÷ niter)%  ",
+                      "accept_ratio_mean=$(round(m[]/nn, sigdigits=3)) accept_ratio_std=$(round(sd[]/nn, sigdigits=3)) ",
+                      "accept_ratio_outliers=$(outl[]) burnin_phase=$(it[] <= nburnin)")
+            end
+            println(stderr)
+        else
+            check(ccall((:kmc_emcee_run, LIB[]), Int32, (Ptr{Cvoid}, Int64), s, -1))
+        end
+        nsr = Ref{Int64}(0)
+        check(ccall((:kmc_emcee_nsamples, LIB[]), Int32, (Ptr{Cvoid}, Ref{Int64}), s, nsr))
+        ns = nsr[]
+        th = Array{Float64,3}(undef, d, ns, k)
+        lp = Matrix{Float64}(undef, ns, k)
+        ar = Vector{Float64}(undef, k)
+        GC.@preserve th lp ar check(ccall((:kmc_emcee_copy_results, LIB[]), Int32,
+            (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), s, th, lp, ar))
+        scalar = first(starts) isa Real
+        thetas = scalar ? [th[1, :, c] for c in 1:k] : [[th[:, i, c] for i in 1:ns] for c in 1:k]
+        logdensities = [lp[:, c] for c in 1:k]
+        nchains === nothing && return thetas[1], ar[1], logdensities[1], nothing
+        return thetas, ar, logdensities, nothing
+    finally
+        ccall((:kmc_emcee_destroy, LIB[]), Int32, (Ptr{Cvoid},), s)
+    end
 end
 
 end # module
