@@ -187,6 +187,11 @@ int32_t kmc_emcee_copy_results(kmc_sampler_t s, double *thetas, double *logp,
  * reduced on the device: mean [d], unbiased variance [d], number of samples.  Avoids copying
  * chains of 10^9+ samples to the host. */
 int32_t kmc_emcee_chain_moments(kmc_sampler_t s, double *mean, double *var, int64_t *count);
+/* Covariance of the same rows as kmc_emcee_chain_moments (emcee or Metropolis handle): mean [d], unbiased covariance
+ * cov [d][d] (ddof = 1, row-major, symmetric), number of samples; shifted by the first stored sample.  A fixed grid
+ * and a fixed-order final sum: the result's bits depend only on the stored chain.  d <= 128, else
+ * KMC_ERR_UNSUPPORTED.  The pilot-run estimate a correlated Metropolis proposal is tuned from. */
+int32_t kmc_emcee_chain_covariance(kmc_sampler_t s, double *mean, double *cov, int64_t *count);
 /* Current ensemble: theta [nw][d], logp [nw], naccept [nw]; any may be NULL. */
 int32_t kmc_emcee_copy_state(kmc_sampler_t s, double *theta, double *logp, int64_t *naccept);
 
@@ -235,6 +240,15 @@ int32_t kmc_ball_randn(uint64_t seed, int64_t walker0, int64_t nwalkers, int32_t
  * KMC_ERR_STATE on it. */
 int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
                               const double *sigma, int64_t nsigma, const kmc_emcee_opts *opts, kmc_sampler_t *out);
+/* The same with a correlated Gaussian random walk (the reference's closure drawing from MvNormal): chol [d][d] is
+ * the lower-triangular Cholesky factor L of the proposal covariance, row-major (Julia's column-major
+ * cholesky(Sigma).U has this layout).  With z the step's normals (the same draws as above): for i = 0 .. d-1,
+ * s = 0.0; s = s + L[i][j] * z[j] for j = 0 .. i ascending (mul, then add, never fused); theta1[i] = theta0[i] + s.
+ * L = diag(sigma) gives the chains of kmc_metropolis_create bit for bit.  KMC_ERR_INVALID as kmc_metropolis_create,
+ * and if an entry is not finite, a diagonal entry is <= 0 or an entry above the diagonal is non-zero.  The handle is
+ * a Metropolis handle like any other; kmc_metropolis_set_replay takes the normals z. */
+int32_t kmc_metropolis_create_chol(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
+                                   const double *chol, const kmc_emcee_opts *opts, kmc_sampler_t *out);
 /* Replay mode: normals [niters][nchains][d] and accept uniforms [niters][nchains] for the steps from the sampler's
  * current step on (sample_ppdf and the rand() of :103).  KMC_ERR_STATE on an emcee handle. */
 int32_t kmc_metropolis_set_replay(kmc_sampler_t s, const double *normals, const double *u, int64_t niters);

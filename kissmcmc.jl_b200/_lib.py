@@ -28,7 +28,8 @@ SYMBOLS = [
     "kmc_emcee_create_multi", "kmc_multi_destroy", "kmc_multi_run", "kmc_multi_sync", "kmc_multi_last_run_ms",
     "kmc_multi_shape", "kmc_multi_copy_results",
     "kmc_g_pdf", "kmc_cdf_g_inv", "kmc_sample_g", "kmc_emcee_squash", "kmc_make_theta0s", "kmc_ball_randn",
-    "kmc_metropolis_create", "kmc_metropolis_set_replay", "kmc_metropolis_draws",
+    "kmc_metropolis_create", "kmc_metropolis_set_replay", "kmc_metropolis_draws", "kmc_metropolis_create_chol",
+    "kmc_emcee_chain_covariance",
 ]
 
 
@@ -102,6 +103,9 @@ lib.kmc_make_theta0s.argtypes = [C.c_void_p, _dp, _dp, C.c_int64, C.c_int32, C.c
 lib.kmc_ball_randn.argtypes = [C.c_uint64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _dp]
 lib.kmc_metropolis_create.argtypes = [C.c_void_p, _dp, C.c_int64, C.c_int32, _dp, C.c_int64, C.POINTER(EmceeOpts),
                                       C.POINTER(C.c_void_p)]
+lib.kmc_metropolis_create_chol.argtypes = [C.c_void_p, _dp, C.c_int64, C.c_int32, _dp, C.POINTER(EmceeOpts),
+                                           C.POINTER(C.c_void_p)]
+lib.kmc_emcee_chain_covariance.argtypes = [C.c_void_p, _dp, _dp, _i64p]
 lib.kmc_metropolis_set_replay.argtypes = [C.c_void_p, _dp, _dp, C.c_int64]
 lib.kmc_metropolis_draws.argtypes = [C.c_uint64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, _dp,
                                      _dp]

@@ -256,6 +256,13 @@ class Sampler:
         check(lib.kmc_emcee_chain_moments(self._h, _ptr(mean), _ptr(var), C.byref(n)))
         return mean, var, n.value
 
+    def chain_covariance(self):
+        """(mean[d], cov[d, d], nsamples) of the whole stored chain (the rows of chain_moments; unbiased, ddof=1),
+        reduced on the device in a fixed order: the same chain gives the same bits.  d <= 128."""
+        mean, cov, n = np.empty(self.d), np.empty((self.d, self.d)), C.c_int64()
+        check(lib.kmc_emcee_chain_covariance(self._h, _ptr(mean), _ptr(cov), C.byref(n)))
+        return mean, cov, n.value
+
     def state(self):
         """Current ensemble (x, logp, naccept); a push-exchange sampler returns the rows it holds
         (its slice of half 0, then of half 1)."""
@@ -425,17 +432,44 @@ def emcee(logdensity, theta0s, *, niter=10**5, nburnin=None, nthin=1, a_scale=2.
 
 class NormalProposal:
     """The proposal of a random-walk Metropolis chain in place of the closure `sample_ppdf`:
-    theta1 = theta0 .+ sigma .* randn(d), sigma a scalar or one scale per component."""
+    theta1 = theta0 .+ sigma .* randn(d), sigma a scalar or one scale per component; or, with `chol` (the lower
+    Cholesky factor L of the proposal covariance, d x d), the correlated walk theta1 = theta0 .+ L * randn(d).
+    `chol` is None for the diagonal walk and `sigma` is None for the correlated one."""
 
-    def __init__(self, sigma):
-        self.sigma = np.ascontiguousarray(np.atleast_1d(np.asarray(sigma, dtype=np.float64)).ravel())
+    def __init__(self, sigma, chol=None):
+        self.sigma = None if sigma is None else np.ascontiguousarray(
+            np.atleast_1d(np.asarray(sigma, dtype=np.float64)).ravel())
+        self.chol = None if chol is None else np.ascontiguousarray(np.asarray(chol, dtype=np.float64))
+        if self.chol is not None and (self.chol.ndim != 2 or self.chol.shape[0] != self.chol.shape[1]):
+            raise ValueError(f"chol must be a square d x d matrix, got shape {self.chol.shape}")
 
     def __repr__(self):
+        if self.chol is not None:
+            return f"NormalProposal(chol={self.chol.tolist()})"
         return f"NormalProposal({self.sigma.tolist() if self.sigma.size > 1 else float(self.sigma[0])})"
 
 
-def normal_proposal(sigma) -> NormalProposal:
-    """Symmetric Gaussian random walk with scale sigma (scalar or length d; finite and > 0, checked at the call)."""
+def normal_proposal(sigma=None, *, cov=None, chol=None) -> NormalProposal:
+    """Symmetric Gaussian random walk.  Give exactly one of
+    sigma  scale, scalar or length d (finite and > 0, checked at the call): theta1 = theta0 .+ sigma .* randn(d);
+    cov    proposal covariance, d x d symmetric positive definite (e.g. 2.38^2 / d times a pilot run's
+           chain_covariance()), factored here with numpy's Cholesky;
+    chol   its lower Cholesky factor L (lower-triangular, positive diagonal, checked at the call):
+           theta1 = theta0 .+ L * randn(d), each component summed in ascending order without FMA."""
+    if sum(a is not None for a in (sigma, cov, chol)) != 1:
+        raise ValueError("normal_proposal takes exactly one of sigma, cov= and chol=")
+    if cov is not None:
+        c = np.asarray(cov, dtype=np.float64)
+        if c.ndim != 2 or c.shape[0] != c.shape[1] or not np.all(np.isfinite(c)):
+            raise ValueError(f"cov must be a finite square d x d matrix, got shape {c.shape}")
+        if not np.allclose(c, c.T, rtol=1e-12, atol=1e-14 * np.abs(c).max()):
+            raise ValueError("cov is not symmetric")
+        try:
+            chol = np.linalg.cholesky(0.5 * (c + c.T))
+        except np.linalg.LinAlgError:
+            raise ValueError("cov is not positive definite") from None
+    if chol is not None:
+        return NormalProposal(None, chol=chol)
     return NormalProposal(sigma)
 
 
@@ -450,7 +484,8 @@ def _require_proposal(sample_ppdf) -> NormalProposal:
 class Metropolis(Sampler):
     """Owns a kmc_sampler_t of nchains independent random-walk Metropolis chains.  Counts are PER CHAIN.
     Chain c draws with id chain_id_base + c, so it is the same chain whatever the batch it runs in.  Running, results,
-    state, squash, chain moments and progress are those of Sampler; there are no half-steps and nothing to exchange."""
+    state, squash, chain moments / covariance and progress are those of Sampler; there are no half-steps and nothing
+    to exchange.  A proposal with `chol` creates the handle with kmc_metropolis_create_chol."""
 
     def __init__(self, logdensity: LogDensity, theta0s, proposal, niter, nburnin, nthin=1, seed=0, mode=MODE_PHILOX,
                  device=None, chain_id_base=0):
@@ -463,10 +498,17 @@ class Metropolis(Sampler):
         self.opts = EmceeOpts(int(niter), int(nburnin), int(nthin), 0.0, int(seed), int(mode),
                               int(logdensity.device if device is None else device), int(chain_id_base),
                               0, 0, 0, 0, 0, 0, 0, 0)
-        sig = self.proposal.sigma
         h = C.c_void_p()
-        check(lib.kmc_metropolis_create(logdensity._h, _ptr(x), self.nw, self.d, _ptr(sig), sig.size,
-                                        C.byref(self.opts), C.byref(h)))
+        if self.proposal.chol is not None:
+            L = self.proposal.chol
+            if L.shape != (self.d, self.d):
+                raise ValueError(f"the proposal's Cholesky factor is {L.shape[0]} x {L.shape[1]}, the density has d={self.d}")
+            check(lib.kmc_metropolis_create_chol(logdensity._h, _ptr(x), self.nw, self.d, _ptr(L), C.byref(self.opts),
+                                                 C.byref(h)))
+        else:
+            sig = self.proposal.sigma
+            check(lib.kmc_metropolis_create(logdensity._h, _ptr(x), self.nw, self.d, _ptr(sig), sig.size,
+                                            C.byref(self.opts), C.byref(h)))
         self._h = h
         n = C.c_int64()
         check(lib.kmc_emcee_nsamples(h, C.byref(n)))
@@ -514,7 +556,8 @@ def metropolis(logdensity, sample_ppdf, theta0, *, niter=10**5, nburnin=None, nt
                hasblob=False, seed=0, replay=None, nchains=None):
     """Random-walk Metropolis; same call shape and 4-tuple as the reference, on the device.
 
-    `sample_ppdf` is normal_proposal(sigma) (a Python callable raises TypeError).  niter / nburnin count the steps of
+    `sample_ppdf` is normal_proposal(sigma), normal_proposal(cov=...) or normal_proposal(chol=...) (a Python
+    callable raises TypeError).  niter / nburnin count the steps of
     ONE chain; ns = (niter - nburnin) // nthin.
     nchains=None: the reference call, one chain from theta0 (scalar or [d]): returns (thetas [ns] or [ns, d],
     accept_ratio: float, logdensities [ns], None).

@@ -622,6 +622,8 @@ int32_t kmc_emcee_destroy(kmc_sampler_t s) {
     dev_free(s->rp_u);
     dev_free(s->rp_n);
     dev_free(s->d_sigma);
+    dev_free(s->d_chol);
+    dev_free(s->d_z);
     dev_free(s->scratch);
     for (void *q : s->ipc_opened) cudaIpcCloseMemHandle(q);
     cudaFree(s->flags);

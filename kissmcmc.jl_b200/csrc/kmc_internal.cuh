@@ -125,6 +125,11 @@ struct kmc_sampler_s {
     std::vector<double> sigma;     // [d] proposal scales: the fused kernel's by-value argument
     double *d_sigma = nullptr;     // batched plugins: the same in device memory
     double *rp_n = nullptr;        // replay normals [steps][chains][d] (rp_u holds the uniforms)
+    // correlated proposal (kmc_metropolis_create_chol): y = x + L z
+    bool chol = false;
+    std::vector<double> chol_packed;  // [d (d + 1) / 2] L by rows: the fused kernel's by-value argument
+    double *d_chol = nullptr;         // batched plugins: L [d][d] in device memory
+    double *d_z = nullptr;            // batched plugins: the step's normals [chains][d]
 };
 
 

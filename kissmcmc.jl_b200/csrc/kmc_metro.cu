@@ -42,22 +42,31 @@ int32_t metro_run(kmc_sampler_s *s, long long nsteps) {
     if (!s->dn->ops.batch) {  // the whole range in one launch, state in registers
         p.t0 = t0;
         p.t1 = t1;
-        void *args[] = {&p, s->dn->params.data(), s->sigma.data()};
+        void *args[] = {&p, s->dn->params.data(), s->chol ? s->chol_packed.data() : s->sigma.data()};
         const unsigned grid = (unsigned)((s->nw + kmc::kMhThreads - 1) / kmc::kMhThreads);
-        CU_TRY(cudaLaunchKernel(s->dn->ops.mh[replay ? 1 : 0], dim3(grid), dim3(kmc::kMhThreads), args, 0, s->stream));
+        const void *k = s->chol ? s->dn->ops.mh_chol[replay ? 1 : 0] : s->dn->ops.mh[replay ? 1 : 0];
+        CU_TRY(cudaLaunchKernel(k, dim3(grid), dim3(kmc::kMhThreads), args, 0, s->stream));
         s->last_launches = 1;
     } else {  // propose -> batched log-density -> accept, per step
         const long long npair = (d + 1) / 2;
         const unsigned gp = (unsigned)((s->nw * npair + 255) / 256), ga = (unsigned)((s->nw * 32 + 255) / 256);
-        const int per_step = 2 + eval_launches(*s->dn);
+        const dim3 gt((unsigned)((s->nw + kmc::kMhTri - 1) / kmc::kMhTri), (unsigned)((d + kmc::kMhTri - 1) / kmc::kMhTri));
+        const int per_step = (s->chol ? 3 : 2) + eval_launches(*s->dn);
         for (long long t = t0; t < t1; ++t) {
             p.t0 = t;
             p.t1 = t + 1;
             const long long ni = t + 1 - s->opts.nburnin_walker;
             const int store = (ni > 0 && ni % s->opts.nthin == 0) ? 1 : 0;
             const long long sidx = store ? ni / s->opts.nthin - 1 : 0;
-            if (replay) kmc::mh_propose_kernel<true><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
-            else kmc::mh_propose_kernel<false><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
+            if (s->chol) {  // Z, U; then Y = X + L Z
+                if (replay) kmc::mh_normals_kernel<true><<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
+                else kmc::mh_normals_kernel<false><<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
+                kmc::mh_chol_kernel<<<gt, dim3(kmc::kMhTri, 8), 0, s->stream>>>(s->x, s->d_chol, s->d_z, s->nw, d, s->bb.Y);
+            } else if (replay) {
+                kmc::mh_propose_kernel<true><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
+            } else {
+                kmc::mh_propose_kernel<false><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
+            }
             CU_TRY(eval_on_device(*s->dn, s->bb.Y, s->nw, s->bb.p1, s->bsc, s->stream));
             kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, ni, store, sidx);
             s->last_launches += per_step;
@@ -72,13 +81,12 @@ int32_t metro_run(kmc_sampler_s *s, long long nsteps) {
 
 }  // namespace kmc_host
 
-extern "C" {
-
-int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
-                              const double *sigma, int64_t nsigma, const kmc_emcee_opts *opts, kmc_sampler_t *out) {
+// kmc_metropolis_create (chol == NULL: y = x + sigma .* z) and kmc_metropolis_create_chol (sigma == NULL: y = x + L z).
+static int32_t metro_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d, const double *sigma,
+                            int64_t nsigma, const double *chol, const kmc_emcee_opts *opts, kmc_sampler_t *out) {
     if (!out) return fail(KMC_ERR_INVALID, "out is NULL");
     *out = nullptr;
-    if (!density || !theta0s || !sigma || !opts) return fail(KMC_ERR_INVALID, "NULL argument");
+    if (!density || !theta0s || !(sigma || chol) || !opts) return fail(KMC_ERR_INVALID, "NULL argument");
     if (d != density->d) return fail(KMC_ERR_INVALID, "d=%d does not match the density (d=%d)", d, density->d);
     if (nchains < 1) return fail(KMC_ERR_INVALID, "nchains must be >= 1");
     if (opts->walker_id_base < 0 || opts->walker_id_base + nchains > (1LL << 32))
@@ -91,10 +99,23 @@ int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int6
     if (opts->launch_mode || opts->exchange || opts->shard_begin || opts->shard_count || opts->push_chunk ||
         opts->push_cap || opts->push_lag)
         return fail(KMC_ERR_INVALID, "launch_mode, exchange, shard_* and push_* must be 0 for Metropolis");
-    if (nsigma != 1 && nsigma != d) return fail(KMC_ERR_INVALID, "sigma has %lld entries: give 1 or d=%d", (long long)nsigma, d);
-    for (int64_t k = 0; k < nsigma; ++k)
-        if (!(std::isfinite(sigma[k]) && sigma[k] > 0.0))
-            return fail(KMC_ERR_INVALID, "sigma[%lld] = %g: proposal scales must be finite and > 0", (long long)k, sigma[k]);
+    if (chol) {  // d x d row-major, lower-triangular with a positive diagonal: a full covariance fails here
+        for (int i = 0; i < d; ++i)
+            for (int j = 0; j < d; ++j) {
+                const double v = chol[(size_t)i * d + j];
+                if (!std::isfinite(v)) return fail(KMC_ERR_INVALID, "chol[%d][%d] = %g is not finite", i, j, v);
+                if (j > i && v != 0.0)
+                    return fail(KMC_ERR_INVALID, "chol[%d][%d] = %g: the factor must be lower-triangular (row-major)", i, j, v);
+                if (j == i && !(v > 0.0))
+                    return fail(KMC_ERR_INVALID, "chol[%d][%d] = %g: the diagonal must be > 0", i, j, v);
+            }
+    } else {
+        if (nsigma != 1 && nsigma != d)
+            return fail(KMC_ERR_INVALID, "sigma has %lld entries: give 1 or d=%d", (long long)nsigma, d);
+        for (int64_t k = 0; k < nsigma; ++k)
+            if (!(std::isfinite(sigma[k]) && sigma[k] > 0.0))
+                return fail(KMC_ERR_INVALID, "sigma[%lld] = %g: proposal scales must be finite and > 0", (long long)k, sigma[k]);
+    }
     if (!density->ops.batch && !density->ops.mh[0])
         return fail(KMC_ERR_UNSUPPORTED, "no Metropolis kernel for this plugin and d=%d", d);
     if (density->ops.batch && opts->device != density->device)
@@ -111,7 +132,14 @@ int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int6
     const long long nspan = opts->niter_walker - opts->nburnin_walker;
     s->ns = nspan > 0 ? nspan / opts->nthin : 0;  // ns = (niter - nburnin) / nthin
     s->sigma.assign(d, 0.0);
-    for (int k = 0; k < d; ++k) s->sigma[k] = sigma[nsigma == 1 ? 0 : k];
+    if (chol) {
+        s->chol = true;
+        s->chol_packed.resize((size_t)d * (d + 1) / 2);
+        for (int i = 0; i < d; ++i)
+            for (int j = 0; j <= i; ++j) s->chol_packed[(size_t)i * (i + 1) / 2 + j] = chol[(size_t)i * d + j];
+    } else {
+        for (int k = 0; k < d; ++k) s->sigma[k] = sigma[nsigma == 1 ? 0 : k];
+    }
 
     auto bail = [&](int32_t rc) {
         kmc_emcee_destroy(s);
@@ -143,12 +171,29 @@ int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int6
         CU_TRY_S(dev_alloc(&s->bb.p1, sizeof(double) * nchains, opts->device));
         CU_TRY_S(dev_alloc(&s->d_sigma, sizeof(double) * d, opts->device));
         CU_TRY_S(cudaMemcpyAsync(s->d_sigma, s->sigma.data(), sizeof(double) * d, cudaMemcpyHostToDevice, s->stream));
+        if (chol) {
+            CU_TRY_S(dev_alloc(&s->d_chol, sizeof(double) * d * d, opts->device));
+            CU_TRY_S(dev_alloc(&s->d_z, sizeof(double) * nchains * d, opts->device));
+            CU_TRY_S(cudaMemcpyAsync(s->d_chol, chol, sizeof(double) * d * d, cudaMemcpyHostToDevice, s->stream));
+        }
     }
     CU_TRY_S(eval_on_device(*density, s->x, nchains, s->lp, s->bsc, s->stream));  // p0 = pdf(theta0)
     CU_TRY_S(cudaStreamSynchronize(s->stream));
 #undef CU_TRY_S
     *out = s;
     return KMC_OK;
+}
+
+extern "C" {
+
+int32_t kmc_metropolis_create(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
+                              const double *sigma, int64_t nsigma, const kmc_emcee_opts *opts, kmc_sampler_t *out) {
+    return metro_create(density, theta0s, nchains, d, sigma, nsigma, nullptr, opts, out);
+}
+
+int32_t kmc_metropolis_create_chol(kmc_density_t density, const double *theta0s, int64_t nchains, int32_t d,
+                                   const double *chol, const kmc_emcee_opts *opts, kmc_sampler_t *out) {
+    return metro_create(density, theta0s, nchains, d, nullptr, 0, chol, opts, out);
 }
 
 int32_t kmc_metropolis_set_replay(kmc_sampler_t s, const double *normals, const double *u, int64_t niters) {
@@ -195,6 +240,42 @@ int32_t kmc_metropolis_draws(uint64_t seed, int64_t chain0, int64_t nchains, int
     dev_free(dn);
     dev_free(du);
     if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "metropolis_draws failed: %s", cudaGetErrorString(e));
+    return KMC_OK;
+}
+
+int32_t kmc_emcee_chain_covariance(kmc_sampler_t s, double *mean, double *cov, int64_t *count) {
+    if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
+    const long long nrows = s->ns * s->nl;  // the rows kmc_emcee_chain_moments reduces
+    const int d = s->d;
+    if (count) *count = nrows;
+    if (d > kmc::kCovMaxD) return fail(KMC_ERR_UNSUPPORTED, "chain covariance supports d <= %d, got d=%d", kmc::kCovMaxD, d);
+    if (nrows < 1) return fail(KMC_ERR_STATE, "no samples stored");
+    CU_TRY(cudaSetDevice(s->opts.device));
+    const int P = (d + 1) * (d + 2) / 2;  // upper triangle over the d components and the constant column
+    double *part = nullptr, *sums = nullptr;
+    CU_TRY(dev_alloc(&part, sizeof(double) * ((size_t)kmc::kCovGrid + 1) * P, s->opts.device));
+    sums = part + (size_t)kmc::kCovGrid * P;
+    std::vector<double> h(P), shift(d);
+    kmc::mh_cov_partial_kernel<<<kmc::kCovGrid, kmc::kCovThreads, 0, s->stream>>>(s->chain_x, nrows, d, part);
+    kmc::mh_cov_final_kernel<<<(P + 255) / 256, 256, 0, s->stream>>>(part, P, kmc::kCovGrid, sums);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h.data(), sums, sizeof(double) * P, cudaMemcpyDeviceToHost, s->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
+    dev_free(part);
+    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "chain covariance failed: %s", cudaGetErrorString(e));
+    const int dc = d + 1;
+    auto at = [&](int a, int b) { return h[(size_t)a * dc - (size_t)a * (a - 1) / 2 + (b - a)]; };  // a <= b
+    const double n = (double)nrows;
+    for (int a = 0; a < d; ++a) {
+        const double sa = at(a, d);
+        if (mean) mean[a] = shift[a] + sa / n;
+        if (cov)
+            for (int b = a; b < d; ++b) {
+                const double v = nrows > 1 ? (at(a, b) - sa * at(b, d) / n) / (n - 1.0) : 0.0;
+                cov[(size_t)a * d + b] = cov[(size_t)b * d + a] = v;
+            }
+    }
     return KMC_OK;
 }
 

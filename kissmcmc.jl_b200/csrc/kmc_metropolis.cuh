@@ -7,10 +7,16 @@
 //   metropolis_kernel   fused plugins at their compiled d: one thread per chain, theta / log-density / accept count
 //                       in registers for a range of steps [t0, t1) -- proposal, plugin, accept test (:103), update,
 //                       thinned store, burn-in counter reset -- and written back once at the end of the launch.
+//   metropolis_chol_kernel  the same loop with the correlated proposal Y = x + L z (L lower-triangular, by value).
 //   mh_propose_kernel   every other plugin, per step: draws + Y = x + sigma .* n ...
+//     (correlated:      mh_normals_kernel draws Z and U, then mh_chol_kernel forms Y = X + L Z)
 //   <density>           ... P1 = plugin(Y) through eval_on_device (FP64, or tcgen05 if the density opted in) ...
 //   mh_accept_kernel    ... accept test, update, counters, store.
 //   mh_draws_kernel     the normals and uniforms of chains x steps (what a replay of the host loop needs).
+//
+// The correlated proposal's arithmetic, which the CPU oracle restates bit for bit: for i = 0 .. d-1,
+// s = 0.0; s = s + L[i][j] * z[j] for j = 0 .. i ascending (mul, then add; never an FMA); y[i] = x[i] + s.
+// With L = diag(sigma) this is bit-identical to x + sigma .* z: the added products are signed zeros.
 //
 // Draws of step t (0-based: t = ni + nburnin - 1) of chain id c: Philox4x32-10, key = seed, counter
 // (c, t lo, t hi, 0x4D48 << 16 | pair) for pair = 0 .. ceil(d/2)-1; normals 2 pair and 2 pair + 1 are the Box-Muller
@@ -49,6 +55,18 @@ struct MhSigma {
     double s[D];
 };
 
+// Lower-triangular Cholesky factor, packed by rows: L[i][j] (j <= i) at i (i + 1) / 2 + j.  By value, like MhSigma.
+template <int D>
+struct MhChol {
+    double l[D * (D + 1) / 2];
+};
+
+// The fused kernels' arguments (MhParams, the plugin, the proposal) share the 4 KB kernel-parameter space.
+template <class Dn, class Prop>
+struct MhParamsFit {
+    static constexpr bool value = sizeof(MhParams) + sizeof(Dn) + sizeof(Prop) <= 4096;
+};
+
 __device__ __forceinline__ double mh_uniform(const Philox4 &r) {
     return (double)(((unsigned long long)(r.r2 & 0xFFFFu) << 32) | r.r3) * 0x1p-48;  // exact: 48-bit integer * 2^-48
 }
@@ -59,9 +77,44 @@ __device__ __forceinline__ Philox4 mh_pair(const PhiloxKeys &ks, unsigned cid, u
     return philox_normals(ks, cid, (unsigned)t, (unsigned)(t >> 32), kMhTag | pair, z0, z1);
 }
 
-// Fused plugins: one thread per chain for steps [t0, t1).
-template <template <int> class Dn, int D, bool REPLAY>
-static __global__ void __launch_bounds__(kMhThreads) metropolis_kernel(const MhParams p, const Dn<D> dn, const MhSigma<D> sg) {
+// Components k, k + 1 (k even; k + 1 skipped at D) of the proposal from the normals z0, z1 of pair k / 2.
+template <int D>
+__device__ __forceinline__ void mh_propose_pair(const MhSigma<D> &sg, const double *x, double *y, int k, double z0,
+                                                double z1) {
+    y[k] = dadd(x[k], dmul(sg.s[k], z0));  // theta0 .+ sigma .* n: mul, then add
+    if (k + 1 < D) y[k + 1] = dadd(x[k + 1], dmul(sg.s[k + 1], z1));
+}
+
+// Correlated: y[i] (i > k + 1) holds the partial sum over j < k of row i until its own pair comes.  Pairs arrive in
+// ascending order, z0 before z1, so every row adds its products in ascending j.
+template <int D>
+__device__ __forceinline__ void mh_propose_pair(const MhChol<D> &ch, const double *x, double *y, int k, double z0,
+                                                double z1) {
+    if (k == 0) {
+#pragma unroll
+        for (int i = 0; i < D; ++i) y[i] = 0.0;
+    }
+#pragma unroll
+    for (int i = k; i < D; ++i) y[i] = dadd(y[i], dmul(ch.l[i * (i + 1) / 2 + k], z0));
+#pragma unroll
+    for (int i = k + 1; i < D; ++i) y[i] = dadd(y[i], dmul(ch.l[i * (i + 1) / 2 + k + 1], z1));
+    y[k] = dadd(x[k], y[k]);
+    if (k + 1 < D) y[k + 1] = dadd(x[k + 1], y[k + 1]);
+}
+
+template <class Prop>
+struct MhIsChol {
+    static constexpr bool value = false;
+};
+template <int D>
+struct MhIsChol<MhChol<D>> {
+    static constexpr bool value = true;
+};
+
+// Fused plugins: one thread per chain for steps [t0, t1).  Prop is MhSigma<D> (y = x + sigma .* z) or MhChol<D>
+// (y = x + L z, formed pair by pair as the Philox pairs arrive: y[i] needs only z[0 .. i]).
+template <template <int> class Dn, int D, bool REPLAY, class Prop>
+__device__ __forceinline__ void metropolis_chain(const MhParams &p, const Dn<D> &dn, const Prop &sg) {
     const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= p.nchains) return;
     double x[D];
@@ -77,8 +130,15 @@ static __global__ void __launch_bounds__(kMhThreads) metropolis_kernel(const MhP
         double y[D], u;
         if constexpr (REPLAY) {
             const size_t slot = (size_t)(t - p.rp_t0) * p.nchains + c;
+            if constexpr (MhIsChol<Prop>::value) {
 #pragma unroll
-            for (int k = 0; k < D; ++k) y[k] = dadd(x[k], dmul(sg.s[k], __ldcs(p.rp_n + slot * D + k)));
+                for (int k = 0; k < D; k += 2)
+                    mh_propose_pair<D>(sg, x, y, k, __ldcs(p.rp_n + slot * D + k),
+                                       k + 1 < D ? __ldcs(p.rp_n + slot * D + k + 1) : 0.0);
+            } else {
+#pragma unroll
+                for (int k = 0; k < D; ++k) y[k] = dadd(x[k], dmul(sg.s[k], __ldcs(p.rp_n + slot * D + k)));
+            }
             u = __ldcs(p.rp_u + slot);
         } else {
 #pragma unroll
@@ -86,8 +146,7 @@ static __global__ void __launch_bounds__(kMhThreads) metropolis_kernel(const MhP
                 double z0, z1;
                 const Philox4 r = mh_pair(p.keys, cid, (unsigned long long)t, (unsigned)pr, z0, z1);
                 if (pr == 0) u = mh_uniform(r);
-                y[2 * pr] = dadd(x[2 * pr], dmul(sg.s[2 * pr], z0));  // theta0 .+ sigma .* n: mul, then add
-                if (2 * pr + 1 < D) y[2 * pr + 1] = dadd(x[2 * pr + 1], dmul(sg.s[2 * pr + 1], z1));
+                mh_propose_pair<D>(sg, x, y, 2 * pr, z0, z1);
             }
         }
         const double p1 = dn.logpdf(y);
@@ -110,6 +169,19 @@ static __global__ void __launch_bounds__(kMhThreads) metropolis_kernel(const MhP
     store_row<D>(p.x + c * D, x);
     p.lp[c] = lp;
     p.nacc[c] = na;
+}
+
+template <template <int> class Dn, int D, bool REPLAY>
+static __global__ void __launch_bounds__(kMhThreads) metropolis_kernel(const MhParams p, const Dn<D> dn, const MhSigma<D> sg) {
+    static_assert(MhParamsFit<Dn<D>, MhSigma<D>>::value, "kernel parameters of metropolis_kernel exceed 4 KB");
+    metropolis_chain<Dn, D, REPLAY>(p, dn, sg);
+}
+
+template <template <int> class Dn, int D, bool REPLAY>
+static __global__ void __launch_bounds__(kMhThreads) metropolis_chol_kernel(const MhParams p, const Dn<D> dn,
+                                                                            const MhChol<D> ch) {
+    static_assert(MhParamsFit<Dn<D>, MhChol<D>>::value, "kernel parameters of metropolis_chol_kernel exceed 4 KB");
+    metropolis_chain<Dn, D, REPLAY>(p, dn, ch);
 }
 
 // Batched plugins, stage 1 of a step: Y = x + sigma .* n and the accept uniform.  One thread per (chain, pair).
@@ -136,6 +208,70 @@ static __global__ void __launch_bounds__(256) mh_propose_kernel(const MhParams p
     yc[k] = dadd(xc[k], dmul(sigma[k], z0));
     if (k + 1 < d) yc[k + 1] = dadd(xc[k + 1], dmul(sigma[k + 1], z1));
     if (pr == 0) U[c] = u;
+}
+
+// Batched plugins with a correlated proposal, stage 1a: the normals Z [nchains][d] and the accept uniform of step t.
+template <bool REPLAY>
+static __global__ void __launch_bounds__(256) mh_normals_kernel(const MhParams p, long long t, int d,
+                                                                double *__restrict__ Z, double *__restrict__ U) {
+    const int npair = (d + 1) / 2;
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= p.nchains * npair) return;
+    const long long c = e / npair;
+    const int pr = (int)(e - c * npair), k = 2 * pr;
+    double *zc = Z + c * d;
+    double z0, z1, u = 0.0;
+    if constexpr (REPLAY) {
+        const size_t slot = (size_t)(t - p.rp_t0) * p.nchains + c;
+        z0 = __ldcs(p.rp_n + slot * d + k);
+        z1 = k + 1 < d ? __ldcs(p.rp_n + slot * d + k + 1) : 0.0;
+        if (pr == 0) u = __ldcs(p.rp_u + slot);
+    } else {
+        const Philox4 r = mh_pair(p.keys, p.id_base + (unsigned)c, (unsigned long long)t, (unsigned)pr, z0, z1);
+        if (pr == 0) u = mh_uniform(r);
+    }
+    zc[k] = z0;
+    if (k + 1 < d) zc[k + 1] = z1;
+    if (pr == 0) U[c] = u;
+}
+
+// Stage 1b: Y = X + L Z, L [d][d] row-major lower-triangular.  A CTA owns kMhTri rows i x kMhTri chains; thread
+// (tx, ty) owns row i0 + tx of chains c0 + ty + 8 r.  It walks the k-tiles up to its diagonal in ascending order with
+// no split-K, so every output adds its products in the order of the proposal contract (s = 0; s += L[i][j] z[j] for
+// j = 0 .. i; y = x + s), and skips the tiles above the diagonal.
+constexpr int kMhTri = 32;
+static __global__ void __launch_bounds__(256) mh_chol_kernel(const double *__restrict__ X, const double *__restrict__ L,
+                                                             const double *__restrict__ Z, long long nchains, int d,
+                                                             double *__restrict__ Y) {
+    constexpr int R = kMhTri / 8;
+    __shared__ double Ls[kMhTri][kMhTri + 1], Zs[kMhTri][kMhTri + 1];
+    const int tx = threadIdx.x, ty = threadIdx.y, tid = ty * kMhTri + tx;
+    const int i0 = blockIdx.y * kMhTri, i = i0 + tx;  // chain tiles on x: grid.y (<= 65535) only counts row tiles
+    const long long c0 = (long long)blockIdx.x * kMhTri;
+    double s[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) s[r] = 0.0;
+    for (int j0 = 0; j0 <= i0; j0 += kMhTri) {
+        for (int e = tid; e < kMhTri * kMhTri; e += 256) {  // coalesced along j
+            const int a = e / kMhTri, b = e % kMhTri;
+            Ls[a][b] = (i0 + a < d && j0 + b < d) ? L[(size_t)(i0 + a) * d + j0 + b] : 0.0;
+            Zs[a][b] = (c0 + a < nchains && j0 + b < d) ? Z[(c0 + a) * d + j0 + b] : 0.0;
+        }
+        __syncthreads();
+        const int jn = min(kMhTri, i - j0 + 1);  // j <= i: the diagonal tile stops at the thread's own row
+        for (int jj = 0; jj < jn; ++jj) {
+            const double l = Ls[tx][jj];
+#pragma unroll
+            for (int r = 0; r < R; ++r) s[r] = dadd(s[r], dmul(l, Zs[ty + 8 * r][jj]));
+        }
+        __syncthreads();
+    }
+    if (i >= d) return;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const long long c = c0 + ty + 8 * r;
+        if (c < nchains) Y[c * d + i] = dadd(X[c * d + i], s[r]);
+    }
 }
 
 // Batched plugins, stage 3 of a step: one warp per chain, lanes stride over the components.
@@ -179,6 +315,60 @@ static __global__ void mh_draws_kernel(PhiloxKeys ks, unsigned chain0, long long
     normals[row * d + 2 * pr] = z0;
     if (2 * pr + 1 < d) normals[row * d + 2 * pr + 1] = z1;
     if (pr == 0) u[row] = mh_uniform(r);
+}
+
+// Covariance of the stored chain (kmc_emcee_chain_covariance): the nrows rows of chain [nrows][d], shifted by row 0
+// like chain_moments_kernel, with a constant column v[d] = 1 appended so that one upper triangle over d + 1 columns
+// holds both sum(v_a v_b) and sum(v_a).  A fixed grid of kCovGrid CTAs each reduces a fixed contiguous row range into
+// its own partials, and mh_cov_final_kernel adds the partials of the CTAs in ascending order: no atomics, so the
+// result's bits depend only on the stored chain.
+constexpr int kCovMaxD = 128, kCovGrid = 256, kCovThreads = 256, kCovRows = 16;
+constexpr int kCovPerThread = ((kCovMaxD + 1) * (kCovMaxD + 2) / 2 + kCovThreads - 1) / kCovThreads;
+
+static __global__ void __launch_bounds__(kCovThreads) mh_cov_partial_kernel(const double *__restrict__ chain,
+                                                                            long long nrows, int d,
+                                                                            double *__restrict__ part /* [grid][P] */) {
+    __shared__ double V[kCovRows][kCovMaxD + 1];
+    const int dc = d + 1, P = dc * (dc + 1) / 2;
+    short ia[kCovPerThread], ib[kCovPerThread];
+    double acc[kCovPerThread];
+#pragma unroll
+    for (int k = 0; k < kCovPerThread; ++k) {  // entry e -> (a, b), a <= b, row-major upper triangle
+        int e = threadIdx.x + k * kCovThreads, a = 0;
+        if (e >= P) e = 0;
+        while (e >= dc - a) e -= dc - a++;
+        ia[k] = (short)a;
+        ib[k] = (short)(a + e);
+        acc[k] = 0.0;
+    }
+    const long long r0 = nrows * blockIdx.x / gridDim.x, r1 = nrows * (blockIdx.x + 1) / gridDim.x;
+    for (long long rb = r0; rb < r1; rb += kCovRows) {
+        const int nr = (int)min((long long)kCovRows, r1 - rb);
+        for (int e = threadIdx.x; e < nr * dc; e += kCovThreads) {
+            const int r = e / dc, a = e - r * dc;
+            V[r][a] = a < d ? chain[(rb + r) * d + a] - chain[a] : 1.0;
+        }
+        __syncthreads();
+        for (int r = 0; r < nr; ++r) {
+#pragma unroll
+            for (int k = 0; k < kCovPerThread; ++k)  // the guard is uniform: small d skips the unused slots
+                if (k * kCovThreads < P) acc[k] = fma(V[r][ia[k]], V[r][ib[k]], acc[k]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int k = 0; k < kCovPerThread; ++k) {
+        const int e = threadIdx.x + k * kCovThreads;
+        if (e < P) part[(size_t)blockIdx.x * P + e] = acc[k];
+    }
+}
+
+static __global__ void mh_cov_final_kernel(const double *__restrict__ part, int P, int ngrid, double *__restrict__ out) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= P) return;
+    double s = 0.0;
+    for (int g = 0; g < ngrid; ++g) s += part[(size_t)g * P + e];
+    out[e] = s;
 }
 
 }  // namespace kmc

@@ -18,6 +18,7 @@ struct Ops {
     int batch = 0;               // 0: fused thread-per-walker kernels; 1: wide Gaussian; 2: logistic (kmc_batched.cuh)
     const void *eval = nullptr;
     const void *mh[2] = {nullptr, nullptr};  // [replay] metropolis_kernel (kmc_metropolis.cuh)
+    const void *mh_chol[2] = {nullptr, nullptr};  // [replay] metropolis_chol_kernel: correlated proposal
     size_t dn_bytes = 0;
     int nparams = 0;
 };
@@ -62,6 +63,8 @@ Ops make_ops() {
     o.eval = (const void *)kmc::density_eval_kernel<Dn, D>;
     o.mh[0] = (const void *)kmc::metropolis_kernel<Dn, D, false>;
     o.mh[1] = (const void *)kmc::metropolis_kernel<Dn, D, true>;
+    o.mh_chol[0] = (const void *)kmc::metropolis_chol_kernel<Dn, D, false>;
+    o.mh_chol[1] = (const void *)kmc::metropolis_chol_kernel<Dn, D, true>;
     o.dn_bytes = sizeof(Dn<D>);
     o.nparams = Dn<D>::nparams;
     return o;

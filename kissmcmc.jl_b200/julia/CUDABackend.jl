@@ -9,7 +9,7 @@
 #     metropolis(logdensity, sample_ppdf, theta0; niter, nburnin, nthin, ...)
 #
 # with ONE difference: `logdensity` is a `LogDensity` plugin descriptor instead of a closure (and metropolis's
-# `sample_ppdf` a `NormalProposal`)
+# `sample_ppdf` a `NormalProposal` or `MvNormalProposal`)
 # (closures cannot cross the C-ABI onto the GPU; there is no CPU fallback and no CUDA.jl).
 #
 # NOTE: Julia is not installed in the build image, so this module has not been executed
@@ -18,7 +18,7 @@
 module CUDABackend
 
 export LogDensity, exponential, rosenbrock, gaussian, lognormal, logistic, set_option!, info, emcee, emcee_squashed,
-       make_theta0s, g_pdf, cdf_g_inv, sample_g, NormalProposal, normal_proposal, metropolis
+       make_theta0s, g_pdf, cdf_g_inv, sample_g, NormalProposal, MvNormalProposal, normal_proposal, metropolis
 
 using LinearAlgebra: cholesky, Symmetric, diag, inv
 import ..KissMCMC: squash_walkers   # host-side, reused as is (src/samplers.jl:372-428)
@@ -354,18 +354,39 @@ end
 normal_proposal(sigma::Real) = NormalProposal(Float64[sigma])
 normal_proposal(sigma::AbstractVector{<:Real}) = NormalProposal(Float64.(sigma))
 
+"Correlated Gaussian random walk `theta1 = theta0 .+ L * randn(d)`, L the lower Cholesky factor of the covariance."
+struct MvNormalProposal
+    chol::Matrix{Float64}        # the column-major UPPER factor U = L': its memory is L row-major, as the library takes it
+end
+normal_proposal(Sigma::AbstractMatrix{<:Real}) = MvNormalProposal(Matrix{Float64}(cholesky(Symmetric(Float64.(Sigma))).U))
+
+# kmc_metropolis_create(_chol) for either proposal
+create_metropolis(ld, x0, k, d, p::NormalProposal, opts, h) =
+    GC.@preserve x0 p check(ccall((:kmc_metropolis_create, LIB[]), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Int64, Ref{EmceeOpts}, Ref{Ptr{Cvoid}}),
+        ld.handle, x0, k, d, p.sigma, length(p.sigma), opts, h))
+function create_metropolis(ld, x0, k, d, p::MvNormalProposal, opts, h)
+    size(p.chol) == (d, d) || error("the proposal's Cholesky factor is $(size(p.chol)), the density has d=$d")
+    GC.@preserve x0 p check(ccall((:kmc_metropolis_create_chol, LIB[]), Int32,
+        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Ref{EmceeOpts}, Ref{Ptr{Cvoid}}),
+        ld.handle, x0, k, d, p.chol, opts, h))
+end
+
 """
-    metropolis(logdensity::LogDensity, proposal::NormalProposal, theta0; niter=10^5, nburnin=niter÷2, nthin=1,
+    metropolis(logdensity::LogDensity, proposal, theta0; niter=10^5, nburnin=niter÷2, nthin=1,
                use_progress_meter=true, hasblob=false, seed=0, nchains=nothing, device=logdensity.device)
+
+`proposal` is `normal_proposal(sigma)` (diagonal) or `normal_proposal(Sigma::AbstractMatrix)` (correlated, factored
+with `cholesky`).
 
 Same semantics and 4-tuple as `KissMCMC.metropolis`: `(thetas::Vector{T}, accept_ratio::Float64,
 logdensities::Vector{Float64}, nothing)`; `niter` counts the steps of one chain.  With `nchains=k`, `theta0` is a
 vector of k starting points and every element of the tuple holds one entry per independent chain (chain c draws
 with id c - 1, so it is the same chain whatever k is).
 """
-function metropolis(ld::LogDensity, proposal::NormalProposal, theta0; niter=10^5, nburnin=niter ÷ 2, nthin=1,
-                    use_progress_meter=true, hasblob=false, seed::Integer=0, nchains=nothing,
-                    device::Integer=ld.device)
+function metropolis(ld::LogDensity, proposal::Union{NormalProposal,MvNormalProposal}, theta0; niter=10^5,
+                    nburnin=niter ÷ 2, nthin=1, use_progress_meter=true, hasblob=false, seed::Integer=0,
+                    nchains=nothing, device::Integer=ld.device)
     hasblob && error("hasblob=true is not supported by the CUDA backend (blobs are host objects)")
     starts = nchains === nothing ? [deepcopy(theta0)] : deepcopy(theta0)
     nchains === nothing || @assert length(starts) == nchains "theta0 must hold nchains starting points"
@@ -373,10 +394,7 @@ function metropolis(ld::LogDensity, proposal::NormalProposal, theta0; niter=10^5
     d, k = size(x0)
     opts = Ref(EmceeOpts(niter, nburnin, nthin, 0.0, UInt64(seed), MODE_PHILOX, device, 0, 0, 0, 0, 0, 0, 0, 0, 0))
     h = Ref{Ptr{Cvoid}}(C_NULL)
-    sig = proposal.sigma
-    GC.@preserve x0 sig check(ccall((:kmc_metropolis_create, LIB[]), Int32,
-        (Ptr{Cvoid}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Int64, Ref{EmceeOpts}, Ref{Ptr{Cvoid}}),
-        ld.handle, x0, k, d, sig, length(sig), opts, h))
+    create_metropolis(ld, x0, k, d, proposal, opts, h)
     s = h[]
     try
         if use_progress_meter && niter > 0                 # coarse: at most 20 polls, never per step

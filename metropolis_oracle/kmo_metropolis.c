@@ -20,24 +20,29 @@
  *       if ni > 0 && rem(ni, nthin) == 0: store (theta0, p0) as sample ni/nthin
  *       if ni == 0: naccept = 0
  *   accept_ratio = naccept / (niter - nburnin)
+ *
+ * kmo_metropolis_chol is the same loop with the correlated proposal of kmc_metropolis_create_chol (L lower-triangular,
+ * [d][d] row-major):
+ *       for i in 0..d-1: s = 0.0; for j in 0..i: s = s + L[i][j] * n_t[j];  theta1[i] = theta0[i] + s
  */
 #include "../oracle/kmc_oracle.c"
 
 /*
  *  x        [nchains][d] in/out: theta0 of every chain, the final state on return
  *  lp       [nchains] out: the final log-density
- *  sigma    [nsigma], nsigma = 1 or d
+ *  sigma    [nsigma], nsigma = 1 or d (chol == NULL); chol [d][d] lower-triangular, row-major (sigma == NULL)
  *  normals  [niter][nchains][d], u [niter][nchains]: the draws of step t of chain c at [t][c]
  *  chain_x  [nchains][ns][d], chain_lp [nchains][ns] (may be NULL), ns = (niter - nburnin) / nthin
  *  naccept, accept_ratio [nchains] out
  *  min_margin: min over finite decisions of |(p1 - p0) - log(u)| (how far any decision was from a tie)
  */
-int kmo_metropolis(const kmo_density *dn, double *x, double *lp, int64_t nchains, int64_t niter, int64_t nburnin,
-                   int64_t nthin, const double *sigma, int64_t nsigma, const double *normals, const double *u,
-                   double *chain_x, double *chain_lp, int64_t *naccept, double *accept_ratio, double *min_margin,
-                   int32_t nthreads) {
+static int kmo_metropolis_loop(const kmo_density *dn, double *x, double *lp, int64_t nchains, int64_t niter,
+                               int64_t nburnin, int64_t nthin, const double *sigma, int64_t nsigma, const double *chol,
+                               const double *normals, const double *u, double *chain_x, double *chain_lp,
+                               int64_t *naccept, double *accept_ratio, double *min_margin, int32_t nthreads) {
     const int d = dn->d;
-    if (nchains < 1 || nthin < 1 || niter < 0 || nburnin < 0 || d < 1 || d > 4096 || (nsigma != 1 && nsigma != d))
+    if (nchains < 1 || nthin < 1 || niter < 0 || nburnin < 0 || d < 1 || d > 4096 ||
+        (!chol && nsigma != 1 && nsigma != d))
         return 1;
     const int64_t ns = niter > nburnin ? (niter - nburnin) / nthin : 0;
     double margin = INFINITY;
@@ -55,7 +60,15 @@ int kmo_metropolis(const kmo_density *dn, double *x, double *lp, int64_t nchains
         int64_t t = 0;
         for (int64_t ni = 1 - nburnin; ni <= niter - nburnin; ++ni, ++t) {
             const double *n = normals + (t * nchains + c) * d;
-            for (int k = 0; k < d; ++k) y[k] = th[k] + sigma[nsigma == 1 ? 0 : k] * n[k];
+            if (chol) {
+                for (int i = 0; i < d; ++i) {
+                    double s = 0.0;
+                    for (int j = 0; j <= i; ++j) s = s + chol[(int64_t)i * d + j] * n[j];
+                    y[i] = th[i] + s;
+                }
+            } else {
+                for (int k = 0; k < d; ++k) y[k] = th[k] + sigma[nsigma == 1 ? 0 : k] * n[k];
+            }
             const double p1 = kmo_logpdf(dn, y);
             const double lhs = p1 - p0, lu = log(u[t * nchains + c]);
             if (lhs > lu) {
@@ -80,4 +93,20 @@ int kmo_metropolis(const kmo_density *dn, double *x, double *lp, int64_t nchains
     }
     if (min_margin) *min_margin = margin;
     return 0;
+}
+
+int kmo_metropolis(const kmo_density *dn, double *x, double *lp, int64_t nchains, int64_t niter, int64_t nburnin,
+                   int64_t nthin, const double *sigma, int64_t nsigma, const double *normals, const double *u,
+                   double *chain_x, double *chain_lp, int64_t *naccept, double *accept_ratio, double *min_margin,
+                   int32_t nthreads) {
+    return kmo_metropolis_loop(dn, x, lp, nchains, niter, nburnin, nthin, sigma, nsigma, NULL, normals, u, chain_x,
+                               chain_lp, naccept, accept_ratio, min_margin, nthreads);
+}
+
+int kmo_metropolis_chol(const kmo_density *dn, double *x, double *lp, int64_t nchains, int64_t niter, int64_t nburnin,
+                        int64_t nthin, const double *chol, const double *normals, const double *u, double *chain_x,
+                        double *chain_lp, int64_t *naccept, double *accept_ratio, double *min_margin, int32_t nthreads) {
+    if (!chol) return 1;
+    return kmo_metropolis_loop(dn, x, lp, nchains, niter, nburnin, nthin, NULL, 0, chol, normals, u, chain_x, chain_lp,
+                               naccept, accept_ratio, min_margin, nthreads);
 }
