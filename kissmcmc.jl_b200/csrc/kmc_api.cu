@@ -109,20 +109,20 @@ bool find_ops(int kind, int d, Ops &o) {
             if (ops_exponential(d, o)) return true;
             if (d > 4096) return false;
             o = Ops();
-            o.batch = 3;  // any other dimension: batched half-step with a thread-per-point sum
+            o.batch = BATCH_EXP;  // any other dimension: batched half-step with a thread-per-point sum
             o.nparams = 0;
             return true;
         case kmc::KIND_GAUSSIAN:
             if (ops_gaussian(d, o)) return true;
             if (d > kmc::kHugeMaxD) return false;
             o = Ops();
-            o.batch = 1;  // dense contraction over the active half (d > 128: FP64 from L2, no tensor-core path)
+            o.batch = BATCH_GAUSSIAN;  // dense contraction over the active half (d > 128: FP64 from L2, no tensor-core path)
             o.nparams = d + d * d + 1;
             return true;
         case kmc::KIND_LOGISTIC:
             if (d > kLogisticMaxD) return false;  // 32 points' theta in shared memory; tcgen05 path up to d = 64
             o = Ops();
-            o.batch = 2;
+            o.batch = BATCH_LOGISTIC;
             o.nparams = 1;
             return true;
         case kmc::KIND_ROSENBROCK: return ops_rosenbrock(d, o);
@@ -139,6 +139,14 @@ int kind_of(const char *name) {
     if (!strcmp(name, "lognormal")) return kmc::KIND_LOGNORMAL;
     if (!strcmp(name, "logistic")) return kmc::KIND_LOGISTIC;
     return -1;
+}
+
+// CTAs of `kern` resident per SM, or 0 if the query fails (its error is cleared).
+int occupancy(const void *kern, int block, size_t smem) {
+    int n = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, block, smem) == cudaSuccess) return n;
+    cudaGetLastError();
+    return 0;
 }
 
 // Batched log-density of npts device-resident points (K4 for the batched plugins; stage 2 of
@@ -209,8 +217,8 @@ TcPlan tc_plan(const kmc_density_s &dn, long long npts) {
 }
 
 cudaError_t batch_scratch_reserve(BatchScratch &sc, const kmc_density_s &dn, long long npts) {
-    if (dn.ops.batch != 2) return cudaSuccess;
-    const bool tcp = dn.tc_ok && dn.tc_on;
+    if (dn.ops.batch != BATCH_LOGISTIC) return cudaSuccess;
+    const bool tcp = dn.tc();
     const TcPlan pl = tcp ? tc_plan(dn, npts) : TcPlan{};
     if (tcp) {
         const size_t pneed = sizeof(__nv_bfloat16) * kmc::tc::PIECES * (size_t)pl.lp.wpad * dn.kp;
@@ -270,7 +278,7 @@ cudaError_t launch_gauss_tc(const kmc_density_s &dn, BatchScratch &sc, long long
 cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long long npts, double *out,
                               BatchScratch &sc, cudaStream_t st) {
     const int d = dn.d;
-    if (dn.ops.batch == 1 && dn.tc_ok && dn.tc_on) {  // tcgen05 Mahalanobis GEMM
+    if (dn.ops.batch == BATCH_GAUSSIAN && dn.tc()) {  // tcgen05 Mahalanobis GEMM
         cudaError_t e = gauss_pieces_reserve(sc, dn, npts);
         if (e != cudaSuccess) return e;
         const long long wpad = ((npts + kmc::tc::BM - 1) / kmc::tc::BM) * kmc::tc::BM;
@@ -279,7 +287,7 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
                                                                                     wpad, d);
         return launch_gauss_tc(dn, sc, npts, out, st);
     }
-    if (dn.ops.batch == 1 && d > kmc::kWideMaxD) {
+    if (dn.ops.batch == BATCH_GAUSSIAN && d > kmc::kWideMaxD) {
         const int dpad = (d + 127) / 128 * 128;
         const size_t per_warp = sizeof(double) * (size_t)d * kmc::kWidePts;
         const int wpb = (int)std::max<size_t>(1, std::min<size_t>(kmc::kWideThreads / 32, (size_t)(200 * 1024) / per_warp));
@@ -292,7 +300,7 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
         kmc::gaussian_huge_logp_kernel<<<grid, wpb * 32, smem, st>>>(X, out, npts, d, dpad, dn.d_params, dn.d_At);
         return cudaGetLastError();
     }
-    if (dn.ops.batch == 1) {
+    if (dn.ops.batch == BATCH_GAUSSIAN) {
         const size_t smem = sizeof(double) * ((size_t)d * 128 + (size_t)(kmc::kWideThreads / 32) * d * kmc::kWidePts);
         cudaError_t e = cudaFuncSetAttribute(kmc::gaussian_wide_logp_kernel,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -303,11 +311,11 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
         kmc::gaussian_wide_logp_kernel<<<grid, kmc::kWideThreads, smem, st>>>(X, out, npts, d, dn.d_params, dn.d_At);
         return cudaGetLastError();
     }
-    if (dn.ops.batch == 3) {
+    if (dn.ops.batch == BATCH_EXP) {
         kmc::exponential_wide_logp_kernel<<<(unsigned)((npts + 255) / 256), 256, 0, st>>>(X, out, npts, d);
         return cudaGetLastError();
     }
-    if (dn.ops.batch == 2 && dn.tc_ok && dn.tc_on) {  // tcgen05 logits GEMM + fused softplus row sums
+    if (dn.ops.batch == BATCH_LOGISTIC && dn.tc()) {  // tcgen05 logits GEMM + fused softplus row sums
         cudaError_t e = batch_scratch_reserve(sc, dn, npts);
         if (e != cudaSuccess) return e;
         TcPlan pl = tc_plan(dn, npts);
@@ -335,7 +343,7 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
             X, sc.part, dn.d_xty, out, npts, d, pl.lp.nchunks, 0.5 / (sg * sg));
         return cudaGetLastError();
     }
-    if (dn.ops.batch == 2) {
+    if (dn.ops.batch == BATCH_LOGISTIC) {
         cudaError_t e = batch_scratch_reserve(sc, dn, npts);
         if (e != cudaSuccess) return e;
         const long long rows = (dn.ndata + kLogitChunks - 1) / kLogitChunks;
@@ -365,10 +373,9 @@ cudaError_t eval_on_device(const kmc_density_s &dn, const double *X, long long n
 }
 
 int eval_launches(const kmc_density_s &dn) {
-    const bool tc = dn.tc_ok && dn.tc_on;
     switch (dn.ops.batch) {
-        case 1: return tc ? 2 : 1;                // (split + GEMM) or the FP64 kernel
-        case 2: return tc ? 3 : 2;                // (split + GEMM + finish) or (partial sums + finish)
+        case BATCH_GAUSSIAN: return dn.tc() ? 2 : 1;  // (split + GEMM) or the FP64 kernel
+        case BATCH_LOGISTIC: return dn.tc() ? 3 : 2;  // (split + GEMM + finish) or (partial sums + finish)
         default: return 1;
     }
 }
@@ -382,6 +389,185 @@ void cache_trim() {
     g_cache.free_blocks.clear();
     g_cache.cached_bytes = 0;
 }
+
+int32_t sampler_init(kmc_sampler_s *s, const double *theta0s) {
+    const int d = s->d, dev = s->opts.device;
+    CU_TRY(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
+    s->stream = s->own_stream;
+    CU_TRY(cudaEventCreate(&s->ev0));
+    CU_TRY(cudaEventCreate(&s->ev1));
+    if (!s->x) CU_TRY(dev_alloc(&s->x, sizeof(double) * s->nstate * d, dev));
+    CU_TRY(dev_alloc(&s->lp, sizeof(double) * s->nstate, dev));
+    CU_TRY(dev_alloc(&s->nacc, sizeof(unsigned) * s->nstate, dev));
+    CU_TRY(dev_alloc(&s->scratch, 4 * sizeof(unsigned long long), dev));
+    if (s->ns > 0) {
+        CU_TRY(dev_alloc(&s->chain_x, sizeof(double) * s->ns * s->nl * d, dev));
+        CU_TRY(dev_alloc(&s->chain_lp, sizeof(double) * s->ns * s->nl, dev));
+    }
+    CU_TRY(cudaMemsetAsync(s->nacc, 0, sizeof(unsigned) * s->nstate, s->stream));
+    if (s->push) {  // only this shard's rows: its slice of half 0, then of half 1
+        CU_TRY(cudaMemcpyAsync(s->x, theta0s + (size_t)s->sbeg * d, sizeof(double) * s->scnt * d,
+                               cudaMemcpyHostToDevice, s->stream));
+        CU_TRY(cudaMemcpyAsync(s->x + (size_t)s->scnt * d, theta0s + (size_t)(s->nhalf + s->sbeg) * d,
+                               sizeof(double) * s->scnt * d, cudaMemcpyHostToDevice, s->stream));
+    } else {  // deep copy
+        CU_TRY(cudaMemcpyAsync(s->x, theta0s, sizeof(double) * s->nstate * d, cudaMemcpyHostToDevice, s->stream));
+    }
+    if (s->dn->ops.batch) {  // per-step buffers of the active shard: proposals, their log-densities, accept uniforms
+        CU_TRY(dev_alloc(&s->bb.Y, sizeof(double) * s->scnt * d, dev));
+        CU_TRY(dev_alloc(&s->bb.u, sizeof(double) * s->scnt, dev));
+        CU_TRY(dev_alloc(&s->bb.p1, sizeof(double) * s->scnt, dev));
+    }
+    CU_TRY(eval_on_device(*s->dn, s->x, s->nstate, s->lp, s->bsc, s->stream));  // p0 = pdf(theta0), :209-210
+    return KMC_OK;
+}
+
+namespace {
+
+// Half-steps [h0, h1) in p: the burn-in and thinning phase of h0, and the barrier epochs used so far.
+void set_range(kmc::RunParams &p, const kmc_sampler_s *s, long long h0, long long h1) {
+    p.h0 = h0;
+    p.h1 = h1;
+    const long long t = h0 >> 1;
+    p.n0 = t + 1 - s->opts.nburnin_walker;  // :245  n = (1-nburnin_walker) + t
+    long long ph = p.n0 % p.nthin;
+    if (ph < 0) ph += p.nthin;
+    p.phase0 = ph;
+    p.sidx0 = p.n0 >= 1 ? (p.n0 - 1) / p.nthin : 0;
+    p.bar_base = s->bar_base;
+}
+
+// The emcee run paths.  Each enqueues half-steps [h0, h1) of p, recording ev0 where its timed window starts, advances the
+// barrier bookkeeping of a persistent kernel and reports its kernel launches.
+
+// Sharded ensemble, owner-computes pushes (kmc_push.cuh): one persistent kernel for the whole range.
+int32_t run_push(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long h1, long long &launches) {
+    if (s->G > 1 && !s->attached)
+        return fail(KMC_ERR_STATE, "push exchange: attach the peers' windows first (kmc_emcee_window_attach)");
+    kmc::PushParams q{};
+    q.recv = reinterpret_cast<double *>(s->window + s->win_recv);
+    q.flags = reinterpret_cast<unsigned long long *>(s->window + s->win_flags);
+    for (int r = 0; r < s->G; ++r) {
+        q.peer_recv[r] = s->peer_recv[r];
+        q.peer_flags[r] = s->peer_flags[r];
+        q.peer_x[r] = s->peer_x[r];
+    }
+    q.task_ctr = s->task_ctr;
+    q.notes = s->notes;
+    q.S = (unsigned)s->scnt;
+    q.G = (unsigned)s->G;
+    q.rank = (unsigned)s->rank;
+    q.chunk = s->chunk;
+    q.rounds = s->rounds;
+    q.nchunks = s->nchunks;
+    q.cap = s->cap;
+    q.lag = s->lag;
+    q.batch = 1;  // measured on 8 B200s (profiles/r2_call13.log, r2_call14.log): notes posted singly, as soon as the
+    q.age = 2;    // newest message is two tasks old, beat every batched / later variant (flag latency gates the consumers)
+    set_range(p, s, h0, h1);
+    CU_TRY(cudaMemsetAsync(s->task_ctr, 0, 4 * sizeof(unsigned long long), s->stream));
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    void *args[] = {&p, &q, s->dn->params.data()};
+    CU_TRY(cudaLaunchCooperativeKernel(s->dn->ops.run_push, dim3(s->grid), dim3(s->block), args, s->smem_bytes, s->stream));
+    s->bar_base += (unsigned long long)(h1 - h0 - 1) * s->grid;
+    launches = 1;
+    return KMC_OK;
+}
+
+// Dense Gaussian on tcgen05, launch_mode 0: the whole range in one persistent fused kernel, K2G (fused_variant 2: the
+// matrix resident in TMEM) or K2F (fused_variant 1: the matrix in shared memory).
+int32_t run_fused_gauss(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long h1, long long &launches) {
+    kmc_density_s &dn = *s->dn;
+    const bool replay = s->opts.mode == KMC_MODE_REPLAY, k2g = dn.fused_variant == 2;
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    kmc::tc::Fused2Params f2{};
+    f2.mu = dn.d_params;
+    f2.apieces = reinterpret_cast<const unsigned *>(dn.d_Abf);
+    f2.lognorm = dn.params[s->d + (size_t)s->d * s->d];
+    f2.d = s->d;
+    kmc::tc::FusedParams f1{f2.mu, f2.lognorm, f2.d};
+    const void *kern = k2g ? (replay ? (const void *)kmc::tc::gaussian_fused2_kernel<true>
+                                     : (const void *)kmc::tc::gaussian_fused2_kernel<false>)
+                           : (replay ? (const void *)kmc::tc::gaussian_fused_kernel<true>
+                                     : (const void *)kmc::tc::gaussian_fused_kernel<false>);
+    const size_t smem = (k2g ? sizeof(kmc::tc::Fused2Smem) : sizeof(kmc::tc::FusedSmem)) + 1024;
+    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const long long ntiles = (s->scnt + kmc::tc::BM - 1) / kmc::tc::BM;
+    const unsigned grid = (unsigned)std::min<long long>(ntiles, dn.nsm);
+    set_range(p, s, h0, h1);
+    void *args2[] = {&p, &f2}, *args1[] = {&dn.mapA, &p, &f1};
+    CU_TRY(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(kmc::tc::kFusedThreads), k2g ? args2 : args1, smem, s->stream));
+    s->bar_base += (unsigned long long)(h1 - h0 - 1) * grid;
+    launches = 1;
+    return KMC_OK;
+}
+
+// Batched plugins: propose -> batched log-density -> accept, per half-step.  The dense Gaussian on tcgen05 (launch_mode
+// 1) writes no Y: the proposals go straight into bf16 pieces and accept recomputes the accepted rows.
+int32_t run_batched(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long h1, long long &launches) {
+    kmc_density_s &dn = *s->dn;
+    const bool replay = s->opts.mode == KMC_MODE_REPLAY, gtc = dn.ops.batch == BATCH_GAUSSIAN && dn.tc();
+    const unsigned grid = (unsigned)((s->scnt * 32 + 255) / 256);
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    if (gtc) CU_TRY(gauss_pieces_reserve(s->bsc, dn, s->scnt));
+    const long long wpad = ((s->scnt + kmc::tc::BM - 1) / kmc::tc::BM) * kmc::tc::BM;
+    const unsigned gridp = (unsigned)((wpad * 32 + 255) / 256);
+    auto propose = replay ? kmc::propose_kernel<true> : kmc::propose_kernel<false>;
+    auto accept = replay ? kmc::accept_kernel<true> : kmc::accept_kernel<false>;
+    auto propose_pieces = replay ? kmc::propose_pieces_kernel<true> : kmc::propose_pieces_kernel<false>;
+    auto accept_recompute = replay ? kmc::accept_recompute_kernel<true> : kmc::accept_recompute_kernel<false>;
+    for (long long h = h0; h < h1; ++h) {
+        set_range(p, s, h, h + 1);
+        const int store = (p.n0 > 0 && p.phase0 == 0) ? 1 : 0;
+        if (gtc) {
+            propose_pieces<<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, dn.d_params, s->bsc.pieces, wpad);
+            CU_TRY(launch_gauss_tc(dn, s->bsc, s->scnt, s->bb.p1, s->stream));
+            accept_recompute<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
+        } else {
+            propose<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d);
+            CU_TRY(eval_on_device(dn, s->bb.Y, s->scnt, s->bb.p1, s->bsc, s->stream));
+            accept<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
+        }
+    }
+    CU_TRY(cudaGetLastError());
+    launches = (h1 - h0) * (gtc ? 3 : 2 + eval_launches(dn));
+    return KMC_OK;
+}
+
+// Fused plugins, launch_mode 1: one walker per thread, one half-step per launch.
+int32_t run_per_half(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long h1, long long &launches) {
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    const void *kern = s->dn->ops.run[s->opts.mode == KMC_MODE_REPLAY ? 1 : 0][0];
+    const int blk = s->dn->ops.block >= 256 ? 256 : s->dn->ops.block;
+    p.per_cta = (unsigned)blk;
+    const unsigned grid = (unsigned)((s->scnt + blk - 1) / blk);
+    void *args[] = {&p, s->dn->params.data()};
+    for (long long h = h0; h < h1; ++h) {
+        set_range(p, s, h, h + 1);
+        CU_TRY(cudaLaunchKernel(kern, dim3(grid), dim3(blk), args, 0, s->stream));
+    }
+    launches = h1 - h0;
+    return KMC_OK;
+}
+
+// Fused plugins, launch_mode 0: the whole range in one persistent kernel with the geometry chosen at creation.
+int32_t run_persistent(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long h1, long long &launches) {
+    const bool peer = s->npeers >= 1;
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    const void *kern = s->use_bulk ? s->dn->ops.run_bulk[peer ? 1 : 0]
+                       : peer      ? s->dn->ops.run_peer
+                                   : s->dn->ops.run[s->opts.mode == KMC_MODE_REPLAY ? 1 : 0][s->use_smem ? 1 : 0];
+    set_range(p, s, h0, h1);
+    void *args[] = {&p, s->dn->params.data()};
+    CU_TRY(cudaLaunchCooperativeKernel(kern, dim3(s->grid), dim3(s->block), args,
+                                       (s->use_bulk || (!peer && s->use_smem)) ? s->smem_bytes : 0, s->stream));
+    s->bar_base += (unsigned long long)(h1 - h0 - 1) * s->grid * (peer ? 2 : 1);
+    if (peer) s->epoch += (unsigned long long)(h1 - h0 - 1);
+    launches = 1;
+    return KMC_OK;
+}
+
+}  // namespace
 
 }  // namespace kmc_host
 
@@ -439,9 +625,14 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
     if (ops.batch) {  // batched plugins keep parameters (and data) in device memory
         if (nparams) h->params.assign(params, params + nparams);
         cudaError_t e = cudaSetDevice(device);
+        if (e == cudaSuccess) {
+            int nsm = 0;
+            cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
+            h->nsm = nsm > 0 ? nsm : 148;
+        }
         if (e == cudaSuccess && nparams) e = dev_alloc(&h->d_params, sizeof(double) * nparams, device);
         if (e == cudaSuccess && nparams) e = cudaMemcpy(h->d_params, params, sizeof(double) * nparams, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && ops.batch == 1) {  // A^T padded to a multiple of 128 rows for the FP64 kernels
+        if (e == cudaSuccess && ops.batch == BATCH_GAUSSIAN) {  // A^T padded to a multiple of 128 rows for the FP64 kernels
             const size_t dpad = (size_t)(d + 127) / 128 * 128;
             std::vector<double> At((size_t)d * dpad, 0.0);
             for (int i = 0; i < d; ++i)
@@ -449,12 +640,7 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
             e = dev_alloc(&h->d_At, sizeof(double) * At.size(), device);
             if (e == cudaSuccess) e = cudaMemcpy(h->d_At, At.data(), sizeof(double) * At.size(), cudaMemcpyHostToDevice);
         }
-        if (e == cudaSuccess && ops.batch == 1) {
-            int nsm = 0;
-            cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-            h->nsm = nsm > 0 ? nsm : 148;
-        }
-        if (e == cudaSuccess && ops.batch == 1 && d <= kmc::kWideMaxD) {  // matrix pieces for the tcgen05 Mahalanobis GEMM
+        if (e == cudaSuccess && ops.batch == BATCH_GAUSSIAN && d <= kmc::kWideMaxD) {  // matrix pieces for the tcgen05 Mahalanobis GEMM
             e = dev_alloc(&h->d_Abf, sizeof(__nv_bfloat16) * kmc::tc::PIECES * kmc::tc::GN * kmc::tc::GK, device);
             if (e == cudaSuccess) {
                 const long long ne = (long long)kmc::tc::GN * kmc::tc::GK;
@@ -465,9 +651,8 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
             if (e == cudaSuccess)
                 h->tc_ok = make_map_bf16_k128(&h->mapA, h->d_Abf, (unsigned long long)kmc::tc::PIECES * kmc::tc::GN,
                                               kmc::tc::GN);
-            h->tc_on = false;  // exact FP64 kernel by default; opt in with set_option("tensor_cores", 1)
         }
-        if (e == cudaSuccess && ops.batch == 2) {
+        if (e == cudaSuccess && ops.batch == BATCH_LOGISTIC) {
             const long long N = data_bytes / (long long)(sizeof(float) * (d + 1));
             if (!data || N < 1 || N * (long long)(sizeof(float) * (d + 1)) != data_bytes) {
                 kmc_density_destroy(h);
@@ -484,11 +669,6 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
             if (e == cudaSuccess)
                 e = cudaMemcpy(h->d_y, (const float *)data + N * d, sizeof(float) * N, cudaMemcpyHostToDevice);
             // tcgen05 path: d <= 64 (zero-padded to K = 32 or 64) and every X value exactly representable in bf16
-            {
-                int nsm = 0;
-                cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-                h->nsm = nsm > 0 ? nsm : 148;
-            }
             if (e == cudaSuccess && d <= 64) {
                 h->kp = d <= 32 ? 32 : 64;
                 const uint32_t *xb = reinterpret_cast<const uint32_t *>(data);
@@ -512,7 +692,6 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
                     }
                     if (e == cudaSuccess)
                         h->tc_ok = make_map_bf16_k(&h->mapX, h->d_Xbf, (unsigned long long)N, kmc::tc::BN, h->kp);
-                    h->tc_on = false;  // exact FP64 kernel by default; opt in with set_option("tensor_cores", 1)
                 }
             }
         }
@@ -545,7 +724,7 @@ int32_t kmc_density_set_option(kmc_density_t h, const char *key, double value) {
 int32_t kmc_density_get_info(kmc_density_t h, const char *key, double *value) {
     if (!h || !key || !value) return fail(KMC_ERR_INVALID, "NULL argument");
     if (!strcmp(key, "tensor_cores")) {
-        *value = (h->tc_ok && h->tc_on) ? 1.0 : 0.0;
+        *value = h->tc() ? 1.0 : 0.0;
         return KMC_OK;
     }
     if (!strcmp(key, "tensor_cores_available")) {
@@ -585,15 +764,7 @@ int32_t kmc_density_eval(kmc_density_t h, const double *thetas, int64_t nw, doub
     cudaError_t e = dev_alloc(&dl, sizeof(double) * nw, h->device);
     if (e == cudaSuccess) e = cudaMemcpy(dx, thetas, sizeof(double) * nw * h->d, cudaMemcpyHostToDevice);
     BatchScratch sc;
-    if (e == cudaSuccess) {
-        if (h->ops.batch) {
-            e = launch_batch_logp(*h, dx, nw, dl, sc, nullptr);
-        } else {
-            long long nwl = nw;
-            void *args[] = {&dx, &dl, &nwl, h->params.data()};
-            e = cudaLaunchKernel(h->ops.eval, dim3((unsigned)((nw + 255) / 256)), dim3(256), args, 0, nullptr);
-        }
-    }
+    if (e == cudaSuccess) e = eval_on_device(*h, dx, nw, dl, sc, nullptr);
     if (e == cudaSuccess) e = cudaMemcpy(logp_out, dl, sizeof(double) * nw, cudaMemcpyDeviceToHost);
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     dev_free(dx);
@@ -663,7 +834,7 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
                     density->device, opts->device);
 
     CU_TRY(cudaSetDevice(opts->device));
-    auto *s = new kmc_sampler_s;
+    SamplerPtr s(new kmc_sampler_s, kmc_emcee_destroy);
     s->dn = density;
     s->opts = *opts;
     s->nw = nwalkers;
@@ -672,18 +843,14 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
     s->sbeg = opts->shard_count > 0 ? opts->shard_begin : 0;
     s->scnt = opts->shard_count > 0 ? opts->shard_count : s->nhalf;
     s->nl = 2 * s->scnt;
-    if (s->sbeg < 0 || s->sbeg + s->scnt > s->nhalf) {
-        delete s;
+    if (s->sbeg < 0 || s->sbeg + s->scnt > s->nhalf)
         return fail(KMC_ERR_INVALID, "shard [%lld, %lld) is outside the half-ensemble [0, %lld)", s->sbeg,
                     s->sbeg + s->scnt, (long long)(nwalkers / 2));
-    }
     const long long nspan = opts->niter_walker - opts->nburnin_walker;
     s->ns = nspan > 0 ? nspan / opts->nthin : 0;  // :234
     s->push = opts->exchange == KMC_EXCHANGE_PUSH;
-    if (opts->exchange != KMC_EXCHANGE_REPLICA && opts->exchange != KMC_EXCHANGE_PUSH) {
-        delete s;
+    if (opts->exchange != KMC_EXCHANGE_REPLICA && opts->exchange != KMC_EXCHANGE_PUSH)
         return fail(KMC_ERR_INVALID, "unknown exchange %d", opts->exchange);
-    }
     if (s->push) {  // owner-computes push exchange: equal shards, fused plugin with 16-byte-multiple rows, Philox draws
         const char *why = nullptr;
         if (opts->shard_count <= 0 || s->nhalf % s->scnt || s->sbeg % s->scnt) why = "equal shards: rank r owns [r*S, (r+1)*S) of each half";
@@ -693,10 +860,7 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
         else if (opts->push_chunk < 0 || opts->push_chunk > kmc::kPushMaxChunk) why = "push_chunk within the kernel's maximum";
         else if (opts->push_cap < 0 || opts->push_cap > kmc::kPushMaxCap) why = "push_cap within the kernel's maximum";
         else if (opts->push_lag < -1) why = "push_lag >= -1";
-        if (why) {
-            delete s;
-            return fail(KMC_ERR_UNSUPPORTED, "the push exchange needs %s", why);
-        }
+        if (why) return fail(KMC_ERR_UNSUPPORTED, "the push exchange needs %s", why);
         s->G = (int)(s->nhalf / s->scnt);
         s->rank = (int)(s->sbeg / s->scnt);
         // default: a chunk sends ~one task-width of rows per destination (kPushThreads walkers per rank), capped by the
@@ -717,82 +881,42 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
     s->hoff = s->push ? s->scnt : s->nhalf;
     s->loff = s->push ? 0 : s->sbeg;
 
-    auto bail = [&](int32_t rc) {
-        kmc_emcee_destroy(s);
-        return rc;
-    };
-#define CU_TRY_S(expr)                                                                              \
-    do {                                                                                            \
-        cudaError_t e_ = (expr);                                                                    \
-        if (e_ != cudaSuccess)                                                                      \
-            return bail(fail(KMC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), \
-                             __FILE__, __LINE__));                                                  \
-    } while (0)
-
-    CU_TRY_S(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
-    s->stream = s->own_stream;
-    CU_TRY_S(cudaEventCreate(&s->ev0));
-    CU_TRY_S(cudaEventCreate(&s->ev1));
     if (s->push) {  // one window: [chunk flags | receive ring | positions], exported as ONE CUDA IPC handle
         auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
         s->win_flags = 0;
         s->win_recv = up(sizeof(unsigned long long) * (size_t)s->G * s->nchunks);
         s->win_x = s->win_recv + up(2 * (size_t)s->G * s->nchunks * (kmc::kPushHeader + sizeof(double) * s->cap * d));
         s->win_bytes = s->win_x + up(sizeof(double) * (size_t)s->nstate * d);
-        CU_TRY_S(cudaMalloc(&s->window, s->win_bytes));
-        CU_TRY_S(cudaMemsetAsync(s->window, 0, s->win_recv, s->stream));  // flags = 0: nothing has landed
+        CU_TRY(cudaMalloc(&s->window, s->win_bytes));
         s->x = reinterpret_cast<double *>(s->window + s->win_x);
-        push_set_peer(s, s->rank, s->window);
-        CU_TRY_S(dev_alloc(&s->task_ctr, 4 * sizeof(unsigned long long), opts->device));
+    }
+    if (const int32_t rc = sampler_init(s.get(), theta0s); rc != KMC_OK) return rc;
+    if (s->push) {
+        CU_TRY(cudaMemsetAsync(s->window, 0, s->win_recv, s->stream));  // flags = 0: nothing has landed
+        push_set_peer(s.get(), s->rank, s->window);
+        CU_TRY(dev_alloc(&s->task_ctr, 4 * sizeof(unsigned long long), opts->device));
         if (s->G > 1) {  // the publisher's inbox: one note per push task, epochs only grow
             const size_t nb = sizeof(unsigned) * (size_t)s->nchunks * (s->G - 1);
-            CU_TRY_S(dev_alloc(&s->notes, nb, opts->device));
-            CU_TRY_S(cudaMemsetAsync(s->notes, 0, nb, s->stream));
+            CU_TRY(dev_alloc(&s->notes, nb, opts->device));
+            CU_TRY(cudaMemsetAsync(s->notes, 0, nb, s->stream));
         }
-    } else {
-        CU_TRY_S(dev_alloc(&s->x, sizeof(double) * s->nw * d, opts->device));
     }
-    CU_TRY_S(dev_alloc(&s->lp, sizeof(double) * s->nstate, opts->device));
-    CU_TRY_S(dev_alloc(&s->nacc, sizeof(unsigned) * s->nstate, opts->device));
-    CU_TRY_S(dev_alloc(&s->barrier, sizeof(unsigned long long), opts->device));
-    CU_TRY_S(dev_alloc(&s->scratch, 4 * sizeof(unsigned long long), opts->device));
-    CU_TRY_S(cudaMalloc(&s->flags, 8 * sizeof(unsigned long long)));  // own allocation: exported through CUDA IPC
-    CU_TRY_S(cudaMemsetAsync(s->flags, 0, 8 * sizeof(unsigned long long), s->stream));
-    if (s->ns > 0) {
-        CU_TRY_S(dev_alloc(&s->chain_x, sizeof(double) * s->ns * s->nl * d, opts->device));
-        CU_TRY_S(dev_alloc(&s->chain_lp, sizeof(double) * s->ns * s->nl, opts->device));
+    CU_TRY(dev_alloc(&s->barrier, sizeof(unsigned long long), opts->device));
+    CU_TRY(cudaMemsetAsync(s->barrier, 0, sizeof(unsigned long long), s->stream));
+    CU_TRY(cudaMalloc(&s->flags, 8 * sizeof(unsigned long long)));  // own allocation: exported through CUDA IPC
+    CU_TRY(cudaMemsetAsync(s->flags, 0, 8 * sizeof(unsigned long long), s->stream));
+    if (density->ops.batch) {  // the half-step's stretch factors and partners
+        CU_TRY(dev_alloc(&s->bb.z, sizeof(double) * s->scnt, opts->device));
+        CU_TRY(dev_alloc(&s->bb.j, sizeof(unsigned) * s->scnt, opts->device));
     }
-    CU_TRY_S(cudaMemsetAsync(s->nacc, 0, sizeof(unsigned) * s->nstate, s->stream));
-    CU_TRY_S(cudaMemsetAsync(s->barrier, 0, sizeof(unsigned long long), s->stream));
-    if (s->push) {  // only this shard's rows: its slice of half 0, then of half 1
-        CU_TRY_S(cudaMemcpyAsync(s->x, theta0s + (size_t)s->sbeg * d, sizeof(double) * s->scnt * d,
-                                 cudaMemcpyHostToDevice, s->stream));
-        CU_TRY_S(cudaMemcpyAsync(s->x + (size_t)s->scnt * d, theta0s + (size_t)(s->nhalf + s->sbeg) * d,
-                                 sizeof(double) * s->scnt * d, cudaMemcpyHostToDevice, s->stream));
-    } else {
-        CU_TRY_S(cudaMemcpyAsync(s->x, theta0s, sizeof(double) * s->nw * d, cudaMemcpyHostToDevice, s->stream));
-    }
-    if (density->ops.batch) {  // initial log-densities, :209-210, and the proposal buffers of the active shard
-        CU_TRY_S(launch_batch_logp(*density, s->x, s->nw, s->lp, s->bsc, s->stream));
-        CU_TRY_S(dev_alloc(&s->bb.Y, sizeof(double) * s->scnt * d, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.z, sizeof(double) * s->scnt, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.u, sizeof(double) * s->scnt, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.p1, sizeof(double) * s->scnt, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.j, sizeof(unsigned) * s->scnt, opts->device));
-    } else {
-        long long nwl = s->nstate;
-        void *args[] = {&s->x, &s->lp, &nwl, density->params.data()};
-        CU_TRY_S(cudaLaunchKernel(density->ops.eval, dim3((unsigned)((s->nstate + 255) / 256)), dim3(256), args, 0,
-                                  s->stream));
-    }
-    CU_TRY_S(cudaDeviceGetAttribute(&s->nsm, cudaDevAttrMultiProcessorCount, opts->device));
+    CU_TRY(cudaDeviceGetAttribute(&s->nsm, cudaDevAttrMultiProcessorCount, opts->device));
     if (s->push) {  // one persistent kernel, tasks handed out dynamically: as many CTAs as fit
         const void *kp = density->ops.run_push;
         const size_t psm = kmc::push_smem_bytes(d, s->cap);
-        CU_TRY_S(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
+        CU_TRY(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psm));
         int occ = 0;
-        CU_TRY_S(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kp, kmc::kPushThreads, psm));
-        if (occ < 1) return bail(fail(KMC_ERR_CUDA, "the push kernel does not fit on the device"));
+        CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kp, kmc::kPushThreads, psm));
+        if (occ < 1) return fail(KMC_ERR_CUDA, "the push kernel does not fit on the device");
         s->grid = (unsigned)(occ * s->nsm);
         s->block = kmc::kPushThreads;
         s->smem_bytes = psm;
@@ -812,19 +936,14 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
                 cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->smem_bytes);
                 if (e != cudaSuccess) { cudaGetLastError(); fits = false; return rounds; }
             }
-            int per_sm = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, (int)s->block, s->smem_bytes) != cudaSuccess) {
-                cudaGetLastError();
-                per_sm = 0;
-            }
-            fits = (long long)per_sm * s->nsm >= (long long)s->grid;
+            fits = (long long)occupancy(kern, (int)s->block, s->smem_bytes) * s->nsm >= (long long)s->grid;
             return rounds;
         };
         bool fits = false;
         s->use_smem = false;
         if (opts->launch_mode == 0 && density->ops.run[r][1] && opts->shard_count == 0) {  // shared-memory-resident state if it fits
             int max_optin = 0;
-            CU_TRY_S(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, opts->device));
+            CU_TRY(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, opts->device));
             const unsigned rounds = geometry(density->ops.run[r][1], kmc::kSmemThreads, kmc::kSmemCtas, density->ops.smem_per_walker, fits);
             s->use_smem = fits && rounds <= (unsigned)kmc::kRounds && s->smem_bytes <= (size_t)max_optin;
         }
@@ -833,10 +952,9 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
             const void *kb0 = density->ops.run_bulk[0], *kb1 = density->ops.run_bulk[1];
             cudaFuncSetAttribute(kb0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)density->ops.bulk_smem);
             cudaFuncSetAttribute(kb1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)density->ops.bulk_smem);
-            int occ = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kb1, kmc::kBulkThreads, density->ops.bulk_smem) !=
-                    cudaSuccess || occ < 1) {
-                cudaGetLastError();
+            const int occ = occupancy(kb1, kmc::kBulkThreads, density->ops.bulk_smem);
+            if (occ < 1) {
+                cudaGetLastError();  // and the attribute calls' errors
                 s->use_bulk = false;
             } else {
                 const long long want = (s->scnt + kmc::kBulkThreads - 1) / kmc::kBulkThreads;
@@ -849,27 +967,16 @@ int32_t kmc_emcee_create(kmc_density_t density, const double *theta0s, int64_t n
             }
         }
         if (!s->use_smem && !s->use_bulk) {
-            int occ = 0;  // as many CTAs per SM as the kernel's registers allow (at least what it was compiled for)
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, density->ops.run[r][0], density->ops.block, 0) != cudaSuccess) {
-                cudaGetLastError();
-                occ = 0;
-            }
-            if (opts->shard_count > 0 && density->ops.run_peer) {  // a sharded sampler may switch to the peer kernel
-                int occ_p = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_p, density->ops.run_peer, density->ops.block, 0) !=
-                    cudaSuccess) {
-                    cudaGetLastError();
-                    occ_p = 0;
-                }
-                occ = std::min(occ, occ_p);
-            }
+            // as many CTAs per SM as the kernel's registers allow (at least what it was compiled for)
+            int occ = occupancy(density->ops.run[r][0], density->ops.block, 0);
+            if (opts->shard_count > 0 && density->ops.run_peer)  // a sharded sampler may switch to the peer kernel
+                occ = std::min(occ, occupancy(density->ops.run_peer, density->ops.block, 0));
             geometry(density->ops.run[r][0], density->ops.block, std::max(occ, 1), 0, fits);
-            if (!fits) return bail(fail(KMC_ERR_CUDA, "kernel does not fit on the device"));
+            if (!fits) return fail(KMC_ERR_CUDA, "kernel does not fit on the device");
         }
     }
-    CU_TRY_S(cudaStreamSynchronize(s->stream));
-#undef CU_TRY_S
-    *out = s;
+    CU_TRY(cudaStreamSynchronize(s->stream));
+    *out = s.release();
     return KMC_OK;
 }
 
@@ -915,216 +1022,61 @@ int32_t kmc_emcee_set_replay(kmc_sampler_t s, const int64_t *partner, const doub
 int32_t kmc_emcee_run_half(kmc_sampler_t s, int64_t nhalfsteps) {
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
     if (s->metro) return fail(KMC_ERR_STATE, "a Metropolis handle has no half-steps: use kmc_emcee_run");
-    const long long remaining = 2 * s->opts.niter_walker - s->hdone;
-    if (nhalfsteps < 0 || nhalfsteps > remaining) nhalfsteps = remaining;
-    s->last_launches = 0;
-    s->timed = false;
-    if (nhalfsteps <= 0) return KMC_OK;
-    const bool replay = s->opts.mode == KMC_MODE_REPLAY;
-    const long long hbeg = s->hdone, hend = s->hdone + nhalfsteps;
-    if (replay && (hbeg < 2 * s->rp_t0 || hend > 2 * (s->rp_t0 + s->rp_niters)))
-        return fail(KMC_ERR_STATE, "replay draws cover iterations [%lld, %lld), asked to run half-steps [%lld, %lld)",
-                    s->rp_t0, s->rp_t0 + s->rp_niters, hbeg, hend);
-    CU_TRY(cudaSetDevice(s->opts.device));
-
-    kmc::RunParams p{};
-    p.x = s->x;
-    p.lp = s->lp;
-    p.nacc = s->nacc;
-    p.chain_x = s->chain_x;
-    p.chain_lp = s->chain_lp;
-    p.rp_partner = s->rp_partner;
-    p.rp_z = s->rp_z;
-    p.rp_u = s->rp_u;
-    p.rp_t0 = s->rp_t0;
-    p.nw = s->nw;
-    p.nhalf = (unsigned)s->nhalf;
-    p.shard_begin = (unsigned)s->sbeg;
-    p.shard_end = (unsigned)(s->sbeg + s->scnt);
-    p.chain_nw = s->nl;
-    p.nthin = s->opts.nthin;
-    p.ns = s->ns;
-    const double a = s->opts.a_scale;
-    p.sia = std::sqrt(1.0 / a);
-    p.span = std::sqrt(a) - p.sia;
-    p.nm1 = (double)(s->d - 1);
-    p.nm1f = (float)(s->d - 1);
-    p.margin = (float)((p.nm1 + 64.0) * 2e-6);
-    p.keys = kmc::philox_keys(s->opts.seed);
-    p.id_base[0] = (unsigned)s->opts.walker_id_base;
-    p.id_base[1] = (unsigned)(s->opts.walker_id_base + s->nhalf);
-    const unsigned nh = (unsigned)s->nhalf;
-    p.lemire_t = (unsigned)(0u - nh) % nh;
-    p.barrier = s->barrier;
-
-    auto set_range = [&](long long h0, long long h1) {
-        p.h0 = h0;
-        p.h1 = h1;
-        const long long t = h0 >> 1;
-        p.n0 = t + 1 - s->opts.nburnin_walker;  // :245  n = (1-nburnin_walker) + t
-        long long ph = p.n0 % p.nthin;
-        if (ph < 0) ph += p.nthin;
-        p.phase0 = ph;
-        p.sidx0 = p.n0 >= 1 ? (p.n0 - 1) / p.nthin : 0;
-        p.bar_base = s->bar_base;
-    };
-
-    void *args[] = {&p, s->dn->params.data()};
-    p.per_cta = s->per_cta;
-    const bool peer = s->npeers >= 1;  // set_peers was called (a single rank exercises the bulk-copy gathers alone)
-    if (peer) {
-        if (replay || s->dn->ops.batch || s->opts.launch_mode != 0 || !s->dn->ops.run_peer)
-            return fail(KMC_ERR_UNSUPPORTED, "peer mode needs a fused (non-batched) plugin, Philox draws and launch_mode 0");
-        // The ranks meet at a flag barrier BETWEEN the half-steps of one launch only: a second launch could gather from a
-        // peer that is still writing the last half-step of the first.  The pull mode therefore runs the whole job in ONE
-        // launch (the push exchange, kmc_emcee_window_*, has no such restriction).
-        if (s->npeers > 1 && (hbeg != 0 || hend != 2 * s->opts.niter_walker))
-            return fail(KMC_ERR_STATE, "peer (pull) mode runs the whole job in one launch: call kmc_emcee_run(s, -1) once");
-        for (int r = 0; r < s->npeers; ++r) {
-            p.peer_x[r] = s->peer_x[r];
-            p.peer_flags[r] = s->peer_flags[r];
-        }
-        p.npeers = s->npeers;
-        p.rank = s->rank;
-        p.epoch_base = s->epoch;
-    }
-    if (s->push) {  // sharded ensemble, owner-computes pushes (kmc_push.cuh): one persistent kernel for the whole range
-        if (s->G > 1 && !s->attached)
-            return fail(KMC_ERR_STATE, "push exchange: attach the peers' windows first (kmc_emcee_window_attach)");
-        kmc::PushParams q{};
-        q.recv = reinterpret_cast<double *>(s->window + s->win_recv);
-        q.flags = reinterpret_cast<unsigned long long *>(s->window + s->win_flags);
-        for (int r = 0; r < s->G; ++r) {
-            q.peer_recv[r] = s->peer_recv[r];
-            q.peer_flags[r] = s->peer_flags[r];
-            q.peer_x[r] = s->peer_x[r];
-        }
-        q.task_ctr = s->task_ctr;
-        q.notes = s->notes;
-        q.S = (unsigned)s->scnt;
-        q.G = (unsigned)s->G;
-        q.rank = (unsigned)s->rank;
-        q.chunk = s->chunk;
-        q.rounds = s->rounds;
-        q.nchunks = s->nchunks;
-        q.cap = s->cap;
-        q.lag = s->lag;
-        q.batch = 1;  // measured on 8 B200s (profiles/r2_call13.log, r2_call14.log): notes posted singly, as soon as the
-        q.age = 2;    // newest message is two tasks old, beat every batched / later variant (flag latency gates the consumers)
-        set_range(hbeg, hend);
-        CU_TRY(cudaMemsetAsync(s->task_ctr, 0, 4 * sizeof(unsigned long long), s->stream));
-        CU_TRY(cudaEventRecord(s->ev0, s->stream));
-        void *pargs[] = {&p, &q, s->dn->params.data()};
-        CU_TRY(cudaLaunchCooperativeKernel(s->dn->ops.run_push, dim3(s->grid), dim3(s->block), pargs, s->smem_bytes,
-                                           s->stream));
-        s->bar_base += (unsigned long long)(hend - hbeg - 1) * s->grid;
-        s->last_launches = 1;
-        CU_TRY(cudaEventRecord(s->ev1, s->stream));
-        s->timed = true;
-        s->hdone = hend;
-        return KMC_OK;
-    }
-    CU_TRY(cudaEventRecord(s->ev0, s->stream));
-    if (s->dn->ops.batch) {  // propose -> batched log-density -> accept, per half-step
-        const unsigned grid = (unsigned)((s->scnt * 32 + 255) / 256);
-        const bool gtc = s->dn->ops.batch == 1 && s->dn->tc_ok && s->dn->tc_on;  // Y-free tcgen05 Gaussian pipeline
-        if (gtc && s->opts.launch_mode == 0 && s->dn->fused_variant == 2) {  // K2G: K2F with the matrix resident in TMEM
-            kmc::tc::Fused2Params fpar{};
-            fpar.mu = s->dn->d_params;
-            fpar.apieces = reinterpret_cast<const unsigned *>(s->dn->d_Abf);
-            fpar.lognorm = s->dn->params[s->d + (size_t)s->d * s->d];
-            fpar.d = s->d;
-            const size_t smem = sizeof(kmc::tc::Fused2Smem) + 1024;
-            const void *kern = replay ? (const void *)kmc::tc::gaussian_fused2_kernel<true>
-                                      : (const void *)kmc::tc::gaussian_fused2_kernel<false>;
-            CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const long long ntiles = (s->scnt + kmc::tc::BM - 1) / kmc::tc::BM;
-            const unsigned fgrid = (unsigned)std::min<long long>(ntiles, s->dn->nsm);
-            set_range(hbeg, hend);
-            void *fargs[] = {&p, &fpar};
-            CU_TRY(cudaLaunchCooperativeKernel(kern, dim3(fgrid), dim3(kmc::tc::kFusedThreads), fargs, smem, s->stream));
-            s->bar_base += (unsigned long long)(hend - hbeg - 1) * fgrid;
-            s->last_launches += 1;
-            CU_TRY(cudaEventRecord(s->ev1, s->stream));
-            s->timed = true;
-            s->hdone = hend;
-            return KMC_OK;
-        }
-        if (gtc && s->opts.launch_mode == 0) {  // K2F: the whole range of half-steps in one persistent fused kernel
-            kmc::tc::FusedParams fpar{};
-            fpar.mu = s->dn->d_params;
-            fpar.lognorm = s->dn->params[s->d + (size_t)s->d * s->d];
-            fpar.d = s->d;
-            const size_t smem = sizeof(kmc::tc::FusedSmem) + 1024;
-            const void *kern = replay ? (const void *)kmc::tc::gaussian_fused_kernel<true>
-                                      : (const void *)kmc::tc::gaussian_fused_kernel<false>;
-            CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const long long ntiles = (s->scnt + kmc::tc::BM - 1) / kmc::tc::BM;
-            const unsigned fgrid = (unsigned)std::min<long long>(ntiles, s->dn->nsm);
-            set_range(hbeg, hend);
-            void *fargs[] = {(void *)&s->dn->mapA, &p, &fpar};
-            CU_TRY(cudaLaunchCooperativeKernel(kern, dim3(fgrid), dim3(kmc::tc::kFusedThreads), fargs, smem, s->stream));
-            s->bar_base += (unsigned long long)(hend - hbeg - 1) * fgrid;
-            s->last_launches += 1;
-            CU_TRY(cudaEventRecord(s->ev1, s->stream));
-            s->timed = true;
-            s->hdone = hend;
-            return KMC_OK;
-        }
-        if (gtc) CU_TRY(gauss_pieces_reserve(s->bsc, *s->dn, s->scnt));
-        const long long wpad = ((s->scnt + kmc::tc::BM - 1) / kmc::tc::BM) * kmc::tc::BM;
-        const unsigned gridp = (unsigned)((wpad * 32 + 255) / 256);
-        for (long long h = hbeg; h < hend; ++h) {
-            set_range(h, h + 1);
-            const int store = (p.n0 > 0 && p.phase0 == 0) ? 1 : 0;
-            if (gtc) {
-                if (replay)
-                    kmc::propose_pieces_kernel<true><<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, s->dn->d_params,
-                                                                                   s->bsc.pieces, wpad);
-                else
-                    kmc::propose_pieces_kernel<false><<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, s->dn->d_params,
-                                                                                    s->bsc.pieces, wpad);
-                CU_TRY(launch_gauss_tc(*s->dn, s->bsc, s->scnt, s->bb.p1, s->stream));
-                if (replay)
-                    kmc::accept_recompute_kernel<true><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
-                else
-                    kmc::accept_recompute_kernel<false><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
-                s->last_launches += 3;
-                continue;
+    return run_range(s, s->hdone, 2 * s->opts.niter_walker, nhalfsteps, 2,
+                     [s](long long hbeg, long long hend, long long &launches) -> int32_t {
+        kmc::RunParams p{};
+        p.x = s->x;
+        p.lp = s->lp;
+        p.nacc = s->nacc;
+        p.chain_x = s->chain_x;
+        p.chain_lp = s->chain_lp;
+        p.rp_partner = s->rp_partner;
+        p.rp_z = s->rp_z;
+        p.rp_u = s->rp_u;
+        p.rp_t0 = s->rp_t0;
+        p.nw = s->nw;
+        p.nhalf = (unsigned)s->nhalf;
+        p.shard_begin = (unsigned)s->sbeg;
+        p.shard_end = (unsigned)(s->sbeg + s->scnt);
+        p.chain_nw = s->nl;
+        p.nthin = s->opts.nthin;
+        p.ns = s->ns;
+        const double a = s->opts.a_scale;
+        p.sia = std::sqrt(1.0 / a);
+        p.span = std::sqrt(a) - p.sia;
+        p.nm1 = (double)(s->d - 1);
+        p.nm1f = (float)(s->d - 1);
+        p.margin = (float)((p.nm1 + 64.0) * 2e-6);
+        p.keys = kmc::philox_keys(s->opts.seed);
+        p.id_base[0] = (unsigned)s->opts.walker_id_base;
+        p.id_base[1] = (unsigned)(s->opts.walker_id_base + s->nhalf);
+        const unsigned nh = (unsigned)s->nhalf;
+        p.lemire_t = (unsigned)(0u - nh) % nh;
+        p.barrier = s->barrier;
+        p.per_cta = s->per_cta;
+        if (s->npeers >= 1) {  // set_peers was called (a single rank exercises the bulk-copy gathers alone)
+            if (s->opts.mode == KMC_MODE_REPLAY || s->dn->ops.batch || s->opts.launch_mode != 0 || !s->dn->ops.run_peer)
+                return fail(KMC_ERR_UNSUPPORTED, "peer mode needs a fused (non-batched) plugin, Philox draws and launch_mode 0");
+            // The ranks meet at a flag barrier BETWEEN the half-steps of one launch only: a second launch could gather from a
+            // peer that is still writing the last half-step of the first.  The pull mode therefore runs the whole job in ONE
+            // launch (the push exchange, kmc_emcee_window_*, has no such restriction).
+            if (s->npeers > 1 && (hbeg != 0 || hend != 2 * s->opts.niter_walker))
+                return fail(KMC_ERR_STATE, "peer (pull) mode runs the whole job in one launch: call kmc_emcee_run(s, -1) once");
+            for (int r = 0; r < s->npeers; ++r) {
+                p.peer_x[r] = s->peer_x[r];
+                p.peer_flags[r] = s->peer_flags[r];
             }
-            if (replay) kmc::propose_kernel<true><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d);
-            else kmc::propose_kernel<false><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d);
-            CU_TRY(launch_batch_logp(*s->dn, s->bb.Y, s->scnt, s->bb.p1, s->bsc, s->stream));
-            if (replay) kmc::accept_kernel<true><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
-            else kmc::accept_kernel<false><<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
-            s->last_launches += s->dn->ops.batch == 2 ? 4 : 3;
+            p.npeers = s->npeers;
+            p.rank = s->rank;
+            p.epoch_base = s->epoch;
         }
-        CU_TRY(cudaGetLastError());
-    } else if (s->opts.launch_mode == 1) {
-        const void *kern = s->dn->ops.run[replay ? 1 : 0][0];
-        const int blk = s->dn->ops.block >= 256 ? 256 : s->dn->ops.block;
-        p.per_cta = (unsigned)blk;  // one walker per thread, one half-step per launch
-        const unsigned grid = (unsigned)((s->scnt + blk - 1) / blk);
-        for (long long h = hbeg; h < hend; ++h) {
-            set_range(h, h + 1);
-            CU_TRY(cudaLaunchKernel(kern, dim3(grid), dim3(blk), args, 0, s->stream));
-            ++s->last_launches;
-        }
-    } else {
-        const void *kern = s->use_bulk ? s->dn->ops.run_bulk[peer ? 1 : 0]
-                           : peer      ? s->dn->ops.run_peer
-                                       : s->dn->ops.run[replay ? 1 : 0][s->use_smem ? 1 : 0];
-        set_range(hbeg, hend);
-        CU_TRY(cudaLaunchCooperativeKernel(kern, dim3(s->grid), dim3(s->block), args,
-                                           (s->use_bulk || (!peer && s->use_smem)) ? s->smem_bytes : 0, s->stream));
-        s->bar_base += (unsigned long long)(hend - hbeg - 1) * s->grid * (peer ? 2 : 1);
-        if (peer) s->epoch += (unsigned long long)(hend - hbeg - 1);
-        ++s->last_launches;
-    }
-    CU_TRY(cudaEventRecord(s->ev1, s->stream));
-    s->timed = true;
-    s->hdone = hend;
-    return KMC_OK;
+        if (s->push) return run_push(s, p, hbeg, hend, launches);
+        if (s->dn->ops.batch == BATCH_GAUSSIAN && s->dn->tc() && s->opts.launch_mode == 0)
+            return run_fused_gauss(s, p, hbeg, hend, launches);
+        if (s->dn->ops.batch) return run_batched(s, p, hbeg, hend, launches);
+        if (s->opts.launch_mode == 1) return run_per_half(s, p, hbeg, hend, launches);
+        return run_persistent(s, p, hbeg, hend, launches);
+    });
 }
 
 int32_t kmc_emcee_run(kmc_sampler_t s, int64_t niters) {

@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -70,6 +71,8 @@ struct kmc_density_s {
     int fused_variant = 2;       // dense Gaussian, launch_mode 0: 2 = K2G (matrix in TMEM, default), 1 = K2F (matrix in shared memory)
     CUtensorMap mapA;
     double *d_At = nullptr;  // FP64 kernel: A transposed and padded to 128 rows, [d][128]
+
+    bool tc() const { return tc_ok && tc_on; }  // the tcgen05 path is available and opted in
 };
 
 
@@ -160,7 +163,42 @@ cudaError_t eval_on_device(const kmc_density_s &dn, const double *X, long long n
 // Kernels eval_on_device launches for this density.
 int eval_launches(const kmc_density_s &dn);
 
+// A sampler under construction, deleted by kmc_emcee_destroy: every exit of a create call frees what was allocated.
+using SamplerPtr = std::unique_ptr<kmc_sampler_s, int32_t (*)(kmc_sampler_t)>;
+
+// Device state of both samplers, from the sizes the create call set (nstate, nl, ns, scnt): the stream and the timing
+// events, x (a push sampler's x already lies in its window), lp, zeroed nacc, the statistics scratch, the chain store,
+// the batched plugins' proposal buffers, theta0 and its log-densities.  The caller synchronises the stream once its
+// own buffers are set up.
+int32_t sampler_init(kmc_sampler_s *s, const double *theta0s);
+
 // kmc_emcee_run of a Metropolis handle (kmc_metro.cu).
 int32_t metro_run(kmc_sampler_s *s, long long nsteps);
+
+// The run of both samplers over [done, done + n), n clamped to the `total` steps left (half-steps for emcee, per = 2 of
+// them per replay iteration; Metropolis steps, per = 1).  path(t0, t1, launches) enqueues the range, recording ev0 where
+// its timed window starts, and reports its kernel launches; the run then closes the window and advances `done`.
+template <class Path>
+int32_t run_range(kmc_sampler_s *s, long long &done, long long total, long long n, int per, Path &&path) {
+    const long long remaining = total - done;
+    if (n < 0 || n > remaining) n = remaining;
+    s->last_launches = 0;
+    s->timed = false;
+    if (n <= 0) return KMC_OK;
+    const long long t0 = done, t1 = done + n;
+    if (s->opts.mode == KMC_MODE_REPLAY && (t0 < per * s->rp_t0 || t1 > per * (s->rp_t0 + s->rp_niters)))
+        return fail(KMC_ERR_STATE, "replay draws cover %s [%lld, %lld), asked to run %s [%lld, %lld)",
+                    per == 2 ? "iterations" : "steps", s->rp_t0, s->rp_t0 + s->rp_niters, per == 2 ? "half-steps" : "steps",
+                    t0, t1);
+    CU_TRY(cudaSetDevice(s->opts.device));
+    long long launches = 0;
+    const int32_t rc = path(t0, t1, launches);
+    if (rc != KMC_OK) return rc;
+    s->last_launches = launches;
+    CU_TRY(cudaEventRecord(s->ev1, s->stream));
+    s->timed = true;
+    done = t1;
+    return KMC_OK;
+}
 
 }  // namespace kmc_host

@@ -11,72 +11,76 @@ using namespace kmc_host;
 
 namespace kmc_host {
 
-int32_t metro_run(kmc_sampler_s *s, long long nsteps) {
-    const long long remaining = s->opts.niter_walker - s->tdone;
-    if (nsteps < 0 || nsteps > remaining) nsteps = remaining;
-    s->last_launches = 0;
-    s->timed = false;
-    if (nsteps <= 0) return KMC_OK;
+namespace {
+
+// The Metropolis run paths: each enqueues steps [t0, t1) of p, recording ev0 where its timed window starts, and reports
+// its kernel launches.
+
+// Fused plugins: the whole range in one launch, state in registers.
+int32_t mh_run_fused(kmc_sampler_s *s, kmc::MhParams &p, long long t0, long long t1, long long &launches) {
     const bool replay = s->opts.mode == KMC_MODE_REPLAY;
-    const long long t0 = s->tdone, t1 = s->tdone + nsteps;
-    if (replay && (t0 < s->rp_t0 || t1 > s->rp_t0 + s->rp_niters))
-        return fail(KMC_ERR_STATE, "replay draws cover steps [%lld, %lld), asked to run steps [%lld, %lld)", s->rp_t0,
-                    s->rp_t0 + s->rp_niters, t0, t1);
-    CU_TRY(cudaSetDevice(s->opts.device));
-    kmc::MhParams p{};
-    p.x = s->x;
-    p.lp = s->lp;
-    p.nacc = s->nacc;
-    p.chain_x = s->chain_x;
-    p.chain_lp = s->chain_lp;
-    p.rp_n = s->rp_n;
-    p.rp_u = s->rp_u;
-    p.rp_t0 = s->rp_t0;
-    p.nchains = s->nw;
-    p.nburnin = s->opts.nburnin_walker;
-    p.nthin = s->opts.nthin;
-    p.keys = kmc::philox_keys(s->opts.seed);
-    p.id_base = (unsigned)s->opts.walker_id_base;
+    CU_TRY(cudaEventRecord(s->ev0, s->stream));
+    p.t0 = t0;
+    p.t1 = t1;
+    void *args[] = {&p, s->dn->params.data(), s->chol ? s->chol_packed.data() : s->sigma.data()};
+    const unsigned grid = (unsigned)((s->nw + kmc::kMhThreads - 1) / kmc::kMhThreads);
+    const void *k = s->chol ? s->dn->ops.mh_chol[replay ? 1 : 0] : s->dn->ops.mh[replay ? 1 : 0];
+    CU_TRY(cudaLaunchKernel(k, dim3(grid), dim3(kmc::kMhThreads), args, 0, s->stream));
+    launches = 1;
+    return KMC_OK;
+}
+
+// Batched plugins: propose -> batched log-density -> accept, per step.
+int32_t mh_run_batched(kmc_sampler_s *s, kmc::MhParams &p, long long t0, long long t1, long long &launches) {
+    const bool replay = s->opts.mode == KMC_MODE_REPLAY;
     const int d = s->d;
     CU_TRY(cudaEventRecord(s->ev0, s->stream));
-    if (!s->dn->ops.batch) {  // the whole range in one launch, state in registers
-        p.t0 = t0;
-        p.t1 = t1;
-        void *args[] = {&p, s->dn->params.data(), s->chol ? s->chol_packed.data() : s->sigma.data()};
-        const unsigned grid = (unsigned)((s->nw + kmc::kMhThreads - 1) / kmc::kMhThreads);
-        const void *k = s->chol ? s->dn->ops.mh_chol[replay ? 1 : 0] : s->dn->ops.mh[replay ? 1 : 0];
-        CU_TRY(cudaLaunchKernel(k, dim3(grid), dim3(kmc::kMhThreads), args, 0, s->stream));
-        s->last_launches = 1;
-    } else {  // propose -> batched log-density -> accept, per step
-        const long long npair = (d + 1) / 2;
-        const unsigned gp = (unsigned)((s->nw * npair + 255) / 256), ga = (unsigned)((s->nw * 32 + 255) / 256);
-        const dim3 gt((unsigned)((s->nw + kmc::kMhTri - 1) / kmc::kMhTri), (unsigned)((d + kmc::kMhTri - 1) / kmc::kMhTri));
-        const int per_step = (s->chol ? 3 : 2) + eval_launches(*s->dn);
-        for (long long t = t0; t < t1; ++t) {
-            p.t0 = t;
-            p.t1 = t + 1;
-            const long long ni = t + 1 - s->opts.nburnin_walker;
-            const int store = (ni > 0 && ni % s->opts.nthin == 0) ? 1 : 0;
-            const long long sidx = store ? ni / s->opts.nthin - 1 : 0;
-            if (s->chol) {  // Z, U; then Y = X + L Z
-                if (replay) kmc::mh_normals_kernel<true><<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
-                else kmc::mh_normals_kernel<false><<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
-                kmc::mh_chol_kernel<<<gt, dim3(kmc::kMhTri, 8), 0, s->stream>>>(s->x, s->d_chol, s->d_z, s->nw, d, s->bb.Y);
-            } else if (replay) {
-                kmc::mh_propose_kernel<true><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
-            } else {
-                kmc::mh_propose_kernel<false><<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
-            }
-            CU_TRY(eval_on_device(*s->dn, s->bb.Y, s->nw, s->bb.p1, s->bsc, s->stream));
-            kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, ni, store, sidx);
-            s->last_launches += per_step;
+    const long long npair = (d + 1) / 2;
+    const unsigned gp = (unsigned)((s->nw * npair + 255) / 256), ga = (unsigned)((s->nw * 32 + 255) / 256);
+    const dim3 gt((unsigned)((s->nw + kmc::kMhTri - 1) / kmc::kMhTri), (unsigned)((d + kmc::kMhTri - 1) / kmc::kMhTri));
+    auto normals = replay ? kmc::mh_normals_kernel<true> : kmc::mh_normals_kernel<false>;
+    auto propose = replay ? kmc::mh_propose_kernel<true> : kmc::mh_propose_kernel<false>;
+    for (long long t = t0; t < t1; ++t) {
+        p.t0 = t;
+        p.t1 = t + 1;
+        const long long ni = t + 1 - s->opts.nburnin_walker;
+        const int store = (ni > 0 && ni % s->opts.nthin == 0) ? 1 : 0;
+        const long long sidx = store ? ni / s->opts.nthin - 1 : 0;
+        if (s->chol) {  // Z, U; then Y = X + L Z
+            normals<<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
+            kmc::mh_chol_kernel<<<gt, dim3(kmc::kMhTri, 8), 0, s->stream>>>(s->x, s->d_chol, s->d_z, s->nw, d, s->bb.Y);
+        } else {
+            propose<<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
         }
-        CU_TRY(cudaGetLastError());
+        CU_TRY(eval_on_device(*s->dn, s->bb.Y, s->nw, s->bb.p1, s->bsc, s->stream));
+        kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, ni, store, sidx);
     }
-    CU_TRY(cudaEventRecord(s->ev1, s->stream));
-    s->timed = true;
-    s->tdone = t1;
+    CU_TRY(cudaGetLastError());
+    launches = (t1 - t0) * ((s->chol ? 3 : 2) + eval_launches(*s->dn));
     return KMC_OK;
+}
+
+}  // namespace
+
+int32_t metro_run(kmc_sampler_s *s, long long nsteps) {
+    return run_range(s, s->tdone, s->opts.niter_walker, nsteps, 1,
+                     [s](long long t0, long long t1, long long &launches) -> int32_t {
+        kmc::MhParams p{};
+        p.x = s->x;
+        p.lp = s->lp;
+        p.nacc = s->nacc;
+        p.chain_x = s->chain_x;
+        p.chain_lp = s->chain_lp;
+        p.rp_n = s->rp_n;
+        p.rp_u = s->rp_u;
+        p.rp_t0 = s->rp_t0;
+        p.nchains = s->nw;
+        p.nburnin = s->opts.nburnin_walker;
+        p.nthin = s->opts.nthin;
+        p.keys = kmc::philox_keys(s->opts.seed);
+        p.id_base = (unsigned)s->opts.walker_id_base;
+        return s->dn->ops.batch ? mh_run_batched(s, p, t0, t1, launches) : mh_run_fused(s, p, t0, t1, launches);
+    });
 }
 
 }  // namespace kmc_host
@@ -123,7 +127,7 @@ static int32_t metro_create(kmc_density_t density, const double *theta0s, int64_
                     density->device, opts->device);
 
     CU_TRY(cudaSetDevice(opts->device));
-    auto *s = new kmc_sampler_s;
+    SamplerPtr s(new kmc_sampler_s, kmc_emcee_destroy);
     s->metro = true;
     s->dn = density;
     s->opts = *opts;
@@ -140,47 +144,18 @@ static int32_t metro_create(kmc_density_t density, const double *theta0s, int64_
     } else {
         for (int k = 0; k < d; ++k) s->sigma[k] = sigma[nsigma == 1 ? 0 : k];
     }
-
-    auto bail = [&](int32_t rc) {
-        kmc_emcee_destroy(s);
-        return rc;
-    };
-#define CU_TRY_S(expr)                                                                                                    \
-    do {                                                                                                                  \
-        cudaError_t e_ = (expr);                                                                                          \
-        if (e_ != cudaSuccess)                                                                                            \
-            return bail(fail(KMC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__)); \
-    } while (0)
-    CU_TRY_S(cudaStreamCreateWithFlags(&s->own_stream, cudaStreamNonBlocking));
-    s->stream = s->own_stream;
-    CU_TRY_S(cudaEventCreate(&s->ev0));
-    CU_TRY_S(cudaEventCreate(&s->ev1));
-    CU_TRY_S(dev_alloc(&s->x, sizeof(double) * nchains * d, opts->device));
-    CU_TRY_S(dev_alloc(&s->lp, sizeof(double) * nchains, opts->device));
-    CU_TRY_S(dev_alloc(&s->nacc, sizeof(unsigned) * nchains, opts->device));
-    CU_TRY_S(dev_alloc(&s->scratch, 4 * sizeof(unsigned long long), opts->device));
-    if (s->ns > 0) {
-        CU_TRY_S(dev_alloc(&s->chain_x, sizeof(double) * s->ns * nchains * d, opts->device));
-        CU_TRY_S(dev_alloc(&s->chain_lp, sizeof(double) * s->ns * nchains, opts->device));
-    }
-    CU_TRY_S(cudaMemsetAsync(s->nacc, 0, sizeof(unsigned) * nchains, s->stream));
-    CU_TRY_S(cudaMemcpyAsync(s->x, theta0s, sizeof(double) * nchains * d, cudaMemcpyHostToDevice, s->stream));  // deep copy
-    if (density->ops.batch) {  // per-step buffers: proposals, their log-densities, accept uniforms
-        CU_TRY_S(dev_alloc(&s->bb.Y, sizeof(double) * nchains * d, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.u, sizeof(double) * nchains, opts->device));
-        CU_TRY_S(dev_alloc(&s->bb.p1, sizeof(double) * nchains, opts->device));
-        CU_TRY_S(dev_alloc(&s->d_sigma, sizeof(double) * d, opts->device));
-        CU_TRY_S(cudaMemcpyAsync(s->d_sigma, s->sigma.data(), sizeof(double) * d, cudaMemcpyHostToDevice, s->stream));
+    if (const int32_t rc = sampler_init(s.get(), theta0s); rc != KMC_OK) return rc;
+    if (density->ops.batch) {  // the proposal in device memory
+        CU_TRY(dev_alloc(&s->d_sigma, sizeof(double) * d, opts->device));
+        CU_TRY(cudaMemcpyAsync(s->d_sigma, s->sigma.data(), sizeof(double) * d, cudaMemcpyHostToDevice, s->stream));
         if (chol) {
-            CU_TRY_S(dev_alloc(&s->d_chol, sizeof(double) * d * d, opts->device));
-            CU_TRY_S(dev_alloc(&s->d_z, sizeof(double) * nchains * d, opts->device));
-            CU_TRY_S(cudaMemcpyAsync(s->d_chol, chol, sizeof(double) * d * d, cudaMemcpyHostToDevice, s->stream));
+            CU_TRY(dev_alloc(&s->d_chol, sizeof(double) * d * d, opts->device));
+            CU_TRY(dev_alloc(&s->d_z, sizeof(double) * nchains * d, opts->device));
+            CU_TRY(cudaMemcpyAsync(s->d_chol, chol, sizeof(double) * d * d, cudaMemcpyHostToDevice, s->stream));
         }
     }
-    CU_TRY_S(eval_on_device(*density, s->x, nchains, s->lp, s->bsc, s->stream));  // p0 = pdf(theta0)
-    CU_TRY_S(cudaStreamSynchronize(s->stream));
-#undef CU_TRY_S
-    *out = s;
+    CU_TRY(cudaStreamSynchronize(s->stream));
+    *out = s.release();
     return KMC_OK;
 }
 

@@ -6,6 +6,15 @@
 
 namespace kmc_host {
 
+// How a plugin evaluates its log-density; the values are what kmc_density_get_info("batched") reports.  BATCH_FUSED is 0,
+// so `if (ops.batch)` reads "a batched plugin".
+enum Batch : int {
+    BATCH_FUSED = 0,     // fused thread-per-walker kernels
+    BATCH_GAUSSIAN = 1,  // dense Gaussian contraction (kmc_batched.cuh; tcgen05 in kmc_tc.cuh)
+    BATCH_LOGISTIC = 2,  // logistic regression over a data set
+    BATCH_EXP = 3,       // exponential at a d with no fused kernel: thread-per-point sum
+};
+
 struct Ops {
     const void *run[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [replay][smem-resident state]
     const void *run_peer = nullptr;  // general kernel with cross-GPU partner gathers (Philox mode)
@@ -15,7 +24,7 @@ struct Ops {
     size_t smem_per_walker = 0;  // bytes of shared memory per owned walker (SMEM mode)
     int block = 0;               // max threads per CTA of the run kernels
     int min_blocks = 1;          // CTAs per SM the kernels are compiled for
-    int batch = 0;               // 0: fused thread-per-walker kernels; 1: wide Gaussian; 2: logistic (kmc_batched.cuh)
+    Batch batch = BATCH_FUSED;
     const void *eval = nullptr;
     const void *mh[2] = {nullptr, nullptr};  // [replay] metropolis_kernel (kmc_metropolis.cuh)
     const void *mh_chol[2] = {nullptr, nullptr};  // [replay] metropolis_chol_kernel: correlated proposal
