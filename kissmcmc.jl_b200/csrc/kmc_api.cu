@@ -424,17 +424,16 @@ int32_t sampler_init(kmc_sampler_s *s, const double *theta0s) {
 
 namespace {
 
-// Half-steps [h0, h1) in p: the burn-in and thinning phase of h0, and the barrier epochs used so far.
-void set_range(kmc::RunParams &p, const kmc_sampler_s *s, long long h0, long long h1) {
+// Half-steps [h0, h1) in p: the burn-in and thinning phase of h0 (returned too), and the barrier epochs used so far.
+kmc::ThinClock<> set_range(kmc::RunParams &p, const kmc_sampler_s *s, long long h0, long long h1) {
     p.h0 = h0;
     p.h1 = h1;
-    const long long t = h0 >> 1;
-    p.n0 = t + 1 - s->opts.nburnin_walker;  // :245  n = (1-nburnin_walker) + t
-    long long ph = p.n0 % p.nthin;
-    if (ph < 0) ph += p.nthin;
-    p.phase0 = ph;
-    p.sidx0 = p.n0 >= 1 ? (p.n0 - 1) / p.nthin : 0;
+    const auto clk = kmc::ThinClock<>::at(h0 >> 1, s->opts.nburnin_walker, p.nthin);
+    p.n0 = clk.n;
+    p.phase0 = clk.phase;
+    p.sidx0 = clk.sidx;
     p.bar_base = s->bar_base;
+    return clk;
 }
 
 // The emcee run paths.  Each enqueues half-steps [h0, h1) of p, recording ev0 where its timed window starts, advances the
@@ -517,16 +516,16 @@ int32_t run_batched(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long
     auto propose_pieces = replay ? kmc::propose_pieces_kernel<true> : kmc::propose_pieces_kernel<false>;
     auto accept_recompute = replay ? kmc::accept_recompute_kernel<true> : kmc::accept_recompute_kernel<false>;
     for (long long h = h0; h < h1; ++h) {
-        set_range(p, s, h, h + 1);
-        const int store = (p.n0 > 0 && p.phase0 == 0) ? 1 : 0;
+        const auto clk = set_range(p, s, h, h + 1);
+        const int store = clk.store() ? 1 : 0;
         if (gtc) {
             propose_pieces<<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, dn.d_params, s->bsc.pieces, wpad);
             CU_TRY(launch_gauss_tc(dn, s->bsc, s->scnt, s->bb.p1, s->stream));
-            accept_recompute<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
+            accept_recompute<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, clk.n, store, clk.sidx);
         } else {
             propose<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d);
             CU_TRY(eval_on_device(dn, s->bb.Y, s->scnt, s->bb.p1, s->bsc, s->stream));
-            accept<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, p.n0, store, p.sidx0);
+            accept<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, clk.n, store, clk.sidx);
         }
     }
     CU_TRY(cudaGetLastError());

@@ -39,7 +39,7 @@ static __global__ void __launch_bounds__(256) propose_kernel(const RunParams p, 
     const double *xk = p.x + ((size_t)(batch ? p.nhalf : 0u) + i) * d;
     const double *xj = p.x + (size_t)j * d;
     double *y = b.Y + (size_t)w * d;
-    for (int c = lane; c < d; c += 32) y[c] = dadd(xj[c], dmul(z, dsub(xk[c], xj[c])));  // :255
+    for (int c = lane; c < d; c += 32) y[c] = stretch_coord(xj[c], xk[c], z);  // :255
     if (lane == 0) {
         b.z[w] = z;
         b.u[w] = u;
@@ -107,8 +107,8 @@ static __global__ void __launch_bounds__(256) propose_pieces_kernel(const RunPar
     const double *xj = p.x + (size_t)j * d;
     for (int c = 2 * lane; c < 128; c += 64) {  // column pairs: one 4-byte store per piece
         double v0 = 0.0, v1 = 0.0;
-        if (c < d) v0 = dadd(xj[c], dmul(z, dsub(xk[c], xj[c]))) - mu[c];  // :255, centred
-        if (c + 1 < d) v1 = dadd(xj[c + 1], dmul(z, dsub(xk[c + 1], xj[c + 1]))) - mu[c + 1];
+        if (c < d) v0 = stretch_coord(xj[c], xk[c], z) - mu[c];  // :255, centred
+        if (c + 1 < d) v1 = stretch_coord(xj[c + 1], xk[c + 1], z) - mu[c + 1];
         unsigned pk[3];
         split3_pair(v0, v1, pk);
 #pragma unroll
@@ -138,7 +138,7 @@ static __global__ void __launch_bounds__(256) accept_recompute_kernel(const RunP
     if (acc || store) {
         for (int c = lane; c < d; c += 32) {
             const double xo = xk[c];
-            const double v = acc ? dadd(xj[c], dmul(z, dsub(xo, xj[c]))) : xo;  // :255 again, same bits
+            const double v = acc ? stretch_coord(xj[c], xo, z) : xo;  // :255 again, same bits
             if (acc) xk[c] = v;                                                  // :261
             if (store) __stcs(p.chain_x + o * d + c, v);                         // :268-272
         }

@@ -18,6 +18,35 @@ __device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a,
 __device__ __forceinline__ double dsub(double a, double b) { return __dsub_rn(a, b); }
 __device__ __forceinline__ double ddiv(double a, double b) { return __ddiv_rn(a, b); }
 
+// One coordinate of the stretch proposal y = xj + z (xk - xj) (src/samplers.jl:255): every kernel that forms or
+// recomputes a proposal uses this one spelling, so they all produce the same bits.
+__device__ __forceinline__ double stretch_coord(double xj, double xk, double z) { return dadd(xj, dmul(z, dsub(xk, xj))); }
+
+// The reference's thinning clock (src/samplers.jl:245, :268): its loop variable n = t + 1 - nburnin (0 at the last
+// burn-in iteration), rem(n, nthin) and the number of samples stored before n.  Phase is the type the phase is kept
+// in (a kernel may keep it in 32 bits).
+template <class Phase = long long>
+struct ThinClock {
+    long long n;
+    Phase phase;
+    long long sidx;
+    // the clock at 0-based iteration t
+    __host__ __device__ static ThinClock at(long long t, long long nburnin, long long nthin) {
+        const long long n = t + 1 - nburnin;
+        long long ph = n % nthin;  // floored: n < 0 during burn-in
+        if (ph < 0) ph += nthin;
+        return ThinClock{n, (Phase)ph, n >= 1 ? (n - 1) / nthin : 0};
+    }
+    __host__ __device__ bool store() const { return n > 0 && phase == 0; }  // :268  n>0 && rem(n,nthin)==0
+    __host__ __device__ bool burnin_end() const { return n == 0; }          // :285-288 accept counters restart
+    // to the next iteration; `stored` is store() of this one
+    __host__ __device__ void advance(bool stored, Phase nthin) {
+        if (stored) ++sidx;
+        ++n;
+        if (++phase == nthin) phase = 0;
+    }
+};
+
 // ------------------------------------------------------------------ FP64 -> three bf16 pieces (tcgen05 operands)
 // Walker coordinates for the tensor-core log-densities: v is rounded ONCE to FP32 (24 significant
 // bits) and that value is split exactly: h0 = RN_bf16(f), r1 = f - h0, h1 = RN_bf16(r1),

@@ -62,6 +62,69 @@ __device__ __forceinline__ unsigned sw128_chunk_offset(unsigned r, unsigned ck) 
     return kh * (GPIECE_BYTES / 2) + (r >> 3) * 1024 + (r & 7) * 128 + ((c8 ^ (r & 7)) << 4);
 }
 
+// Columns 2 cp, 2 cp + 1 (column pairs cp = ck + 16 e, e = 0..3) of a walker's own row xk and, when load_j, of its partner's
+// row xj (an L2 load: other CTAs write it), zero past d.  Even d: one 16-byte load per column pair.
+__device__ __forceinline__ void fused_row_load(const double *xk, const double *xj, bool load_j, int d, unsigned ck,
+                                               double2 (&xa)[4], double2 (&xb)[4]) {
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const int c = 2 * (ck + 16 * e);
+        xa[e] = make_double2(0.0, 0.0);
+        xb[e] = make_double2(0.0, 0.0);
+        if ((d & 1) == 0) {
+            if (c < d) {
+                xa[e] = *reinterpret_cast<const double2 *>(xk + c);
+                if (load_j) xb[e] = __ldcg(reinterpret_cast<const double2 *>(xj + c));
+            }
+        } else {
+            if (c < d) {
+                xa[e].x = xk[c];
+                if (load_j) xb[e].x = __ldcg(xj + c);
+            }
+            if (c + 1 < d) {
+                xa[e].y = xk[c + 1];
+                if (load_j) xb[e].y = __ldcg(xj + c + 1);
+            }
+        }
+    }
+}
+
+// P3 of listed row rr of the tile whose first walker is w0: an accepted row recomputes its proposal with the same three
+// operations as P1 (:255, same bits) and writes it back (:261); in a stored iteration the row goes to the chain (:268-272).
+// A half-warp per row, lane ck owns the column pairs of fused_row_load.
+template <class Smem>
+__device__ __forceinline__ void fused_writeback_row(const RunParams &p, const Smem &sm, unsigned rb, unsigned rr, unsigned w0,
+                                                    size_t a0, int d, unsigned ck, unsigned batch, bool store, long long sidx) {
+    const bool accr = sm.acc[rb][rr] != 0;
+    const unsigned i = p.shard_begin + w0 + rr;
+    double *xk = p.x + (a0 + i) * d;
+    double2 xa[4], xb[4];
+    fused_row_load(xk, p.x + (size_t)sm.j[rb][rr] * d, accr, d, ck, xa, xb);
+    const double z = sm.z[rb][rr];
+    const size_t o = store ? chain_row(p, sidx, batch, i) : 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const int c = 2 * (ck + 16 * e);
+        const double v0 = accr ? stretch_coord(xb[e].x, xa[e].x, z) : xa[e].x;
+        const double v1 = accr ? stretch_coord(xb[e].y, xa[e].y, z) : xa[e].y;
+        if ((d & 1) == 0) {  // even d: rows are 16-byte aligned, one 16-byte store per column pair
+            if (c < d) {
+                if (accr) *reinterpret_cast<double2 *>(xk + c) = make_double2(v0, v1);
+                if (store) __stcs(reinterpret_cast<double2 *>(p.chain_x + o * d + c), make_double2(v0, v1));
+            }
+        } else {
+            if (c < d) {
+                if (accr) xk[c] = v0;
+                if (store) __stcs(p.chain_x + o * d + c, v0);
+            }
+            if (c + 1 < d) {
+                if (accr) xk[c + 1] = v1;
+                if (store) __stcs(p.chain_x + o * d + c + 1, v1);
+            }
+        }
+    }
+}
+
 template <bool REPLAY>
 __global__ void __launch_bounds__(kFusedThreads, 1)
 gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams p, const FusedParams fp) {
@@ -108,7 +171,7 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
     const unsigned half16 = lane >> 4;   // which of the warp's two walkers
     const unsigned ck = lane & 15;       // 16-byte chunk = columns 8*ck .. 8*ck+7
     unsigned mma_phase = 0, tpar = 0;  // tpar: parity of the tile counter of this CTA
-    long long n = p.n0, phase = p.phase0, sidx = p.sidx0;
+    ThinClock<> clk{p.n0, p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
 #ifdef KMC_K2F_PROF
     long long pt[6] = {0, 0, 0, 0, 0, 0}, pc0 = clock64();
@@ -119,7 +182,7 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
 
     for (long long h = p.h0; h < p.h1; ++h) {
         const unsigned batch = (unsigned)(h & 1);
-        const bool store = (n > 0) && (phase == 0);  // :268
+        const bool store = clk.store();
         const size_t a0 = batch ? (size_t)p.nhalf : 0;
 
         // draws (src/samplers.jl:250,:252,:260) of one tile: one thread per walker row, into parity `par`
@@ -153,28 +216,7 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                 auto row_live = [&](unsigned r) { return r < tr && w0 + r < W; };
                 auto row_load = [&](unsigned r, double2 (&xa)[4], double2 (&xb)[4]) {
                     const unsigned i = p.shard_begin + w0 + r;
-                    const double *xk = p.x + (a0 + i) * d, *xj = p.x + (size_t)sm.j[tpar][r] * d;
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const int c = 2 * (ck + 16 * e);
-                        xa[e] = make_double2(0.0, 0.0);
-                        xb[e] = make_double2(0.0, 0.0);
-                        if ((d & 1) == 0) {
-                            if (c < d) {
-                                xa[e] = *reinterpret_cast<const double2 *>(xk + c);
-                                xb[e] = __ldcg(reinterpret_cast<const double2 *>(xj + c));
-                            }
-                        } else {
-                            if (c < d) {
-                                xa[e].x = xk[c];
-                                xb[e].x = __ldcg(xj + c);
-                            }
-                            if (c + 1 < d) {
-                                xa[e].y = xk[c + 1];
-                                xb[e].y = __ldcg(xj + c + 1);
-                            }
-                        }
-                    }
+                    fused_row_load(p.x + (a0 + i) * d, p.x + (size_t)sm.j[tpar][r] * d, true, d, ck, xa, xb);
                 };
                 auto row_emit = [&](unsigned r, const double2 (&xa)[4], const double2 (&xb)[4]) {
                     const double zz = sm.z[tpar][r];
@@ -183,8 +225,8 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                         const int c = 2 * (ck + 16 * e);
                         const double2 m = *reinterpret_cast<const double2 *>(sm.mu + c);  // zero past d
                         // :255, centred; columns past d were loaded as zeros and stay zero
-                        const double v0 = dadd(xb[e].x, dmul(zz, dsub(xa[e].x, xb[e].x))) - m.x;
-                        const double v1 = dadd(xb[e].y, dmul(zz, dsub(xa[e].y, xb[e].y))) - m.y;
+                        const double v0 = stretch_coord(xb[e].x, xa[e].x, zz) - m.x;
+                        const double v1 = stretch_coord(xb[e].y, xa[e].y, zz) - m.y;
                         unsigned pk[PIECES];
                         split3_pair(v0, v1, pk);
                         const unsigned cp = ck + 16 * e;  // column pair -> 4 bytes inside chunk cp/4
@@ -281,13 +323,13 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                     if (acc || store) sm.list[tpar][atomicAdd(&sm.nlist[tpar], 1u)] = (unsigned char)r;
                     if (acc) {
                         p.lp[k] = p1;
-                        if (!(batch == 1 && n == 0)) atomicAdd(p.nacc + k, 1u);  // fire-and-forget; only this thread touches the counter
+                        if (!(batch == 1 && clk.burnin_end())) atomicAdd(p.nacc + k, 1u);  // fire-and-forget; only this thread touches the counter
                     }
-                    if (batch == 1 && n == 0) {  // :285-288
+                    if (batch == 1 && clk.burnin_end()) {  // :285-288
                         p.nacc[i] = 0u;
                         p.nacc[(size_t)p.nhalf + i] = 0u;
                     }
-                    if (store) __stcs(p.chain_lp + chain_row(p, sidx, batch, i), acc ? p1 : p0);
+                    if (store) __stcs(p.chain_lp + chain_row(p, clk.sidx, batch, i), acc ? p1 : p0);
                 }
             }
             else if (warp < 8) {  // idle during the GEMM: the NEXT tile's draws, into the other parity
@@ -317,27 +359,7 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                     if (!live[t]) continue;
                     const double *xk = p.x + (a0 + p.shard_begin + w0 + rr[t]) * d;
                     const double *xj = p.x + (size_t)sm.j[tpar][rr[t]] * d;
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const int c = 2 * (ck + 16 * e);
-                        xa[t][e] = make_double2(0.0, 0.0);
-                        xb[t][e] = make_double2(0.0, 0.0);
-                        if ((d & 1) == 0) {
-                            if (c < d) {
-                                xa[t][e] = *reinterpret_cast<const double2 *>(xk + c);
-                                if (accr[t]) xb[t][e] = __ldcg(reinterpret_cast<const double2 *>(xj + c));
-                            }
-                        } else {
-                            if (c < d) {
-                                xa[t][e].x = xk[c];
-                                if (accr[t]) xb[t][e].x = __ldcg(xj + c);
-                            }
-                            if (c + 1 < d) {
-                                xa[t][e].y = xk[c + 1];
-                                if (accr[t]) xb[t][e].y = __ldcg(xj + c + 1);
-                            }
-                        }
-                    }
+                    fused_row_load(xk, xj, accr[t], d, ck, xa[t], xb[t]);
                 }
 #pragma unroll
                 for (int t = 0; t < 1; ++t) {
@@ -345,12 +367,12 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                     const unsigned i = p.shard_begin + w0 + rr[t];
                     double *xk = p.x + (a0 + i) * d;
                     const double z = sm.z[tpar][rr[t]];
-                    const size_t o = store ? chain_row(p, sidx, batch, i) : 0;
+                    const size_t o = store ? chain_row(p, clk.sidx, batch, i) : 0;
 #pragma unroll
                     for (int e = 0; e < 4; ++e) {
                         const int c = 2 * (ck + 16 * e);
-                        const double v0 = accr[t] ? dadd(xb[t][e].x, dmul(z, dsub(xa[t][e].x, xb[t][e].x))) : xa[t][e].x;  // :255, same bits
-                        const double v1 = accr[t] ? dadd(xb[t][e].y, dmul(z, dsub(xa[t][e].y, xb[t][e].y))) : xa[t][e].y;
+                        const double v0 = accr[t] ? stretch_coord(xb[t][e].x, xa[t][e].x, z) : xa[t][e].x;  // :255, same bits
+                        const double v1 = accr[t] ? stretch_coord(xb[t][e].y, xa[t][e].y, z) : xa[t][e].y;
                         if ((d & 1) == 0) {  // even d: rows are 16-byte aligned, one 16-byte store per column pair
                             if (c < d) {
                                 if (accr[t]) *reinterpret_cast<double2 *>(xk + c) = make_double2(v0, v1);                  // :261
@@ -372,11 +394,7 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
             tpar ^= 1;
             K2F_TICK(3);
         }
-        if (batch == 1) {
-            if (store) ++sidx;
-            ++n;
-            if (++phase == p.nthin) phase = 0;
-        }
+        if (batch == 1) clk.advance(store, p.nthin);
         if (h + 1 < p.h1) {  // the reference's join between the two half-ensemble sweeps (:248/:273)
             target += gridDim.x;
             __syncthreads();

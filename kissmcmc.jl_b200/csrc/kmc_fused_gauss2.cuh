@@ -149,7 +149,7 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
     const int nk = (d + 15) / 16;               // k-steps that hold data
     const unsigned half16 = lane >> 4, ck = lane & 15;
     unsigned mph = 0;                           // bit b: phase of mma_done[b]
-    long long n = p.n0, phase = p.phase0, sidx = p.sidx0;
+    ThinClock<> clk{p.n0, p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
 
 #ifdef KMC_K2F_PROF
@@ -161,7 +161,7 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
 
     for (long long h = p.h0; h < p.h1; ++h) {
         const unsigned batch = (unsigned)(h & 1);
-        const bool store = (n > 0) && (phase == 0);  // :268
+        const bool store = clk.store();
         const size_t a0 = batch ? (size_t)p.nhalf : 0;
 
         // draws (src/samplers.jl:250,:252,:260) of one tile: one thread per walker row, into row buffer rb
@@ -244,13 +244,13 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
                 if (acc || store) sm.list[rb][atomicAdd(&sm.nlist[rb], 1u)] = (unsigned char)r;
                 if (acc) {
                     p.lp[k] = p1;
-                    if (!(batch == 1 && n == 0)) atomicAdd(p.nacc + k, 1u);
+                    if (!(batch == 1 && clk.burnin_end())) atomicAdd(p.nacc + k, 1u);
                 }
-                if (batch == 1 && n == 0) {  // :285-288
+                if (batch == 1 && clk.burnin_end()) {  // :285-288
                     p.nacc[i] = 0u;
                     p.nacc[(size_t)p.nhalf + i] = 0u;
                 }
-                if (store) __stcs(p.chain_lp + chain_row(p, sidx, batch, i), acc ? p1 : p0);
+                if (store) __stcs(p.chain_lp + chain_row(p, clk.sidx, batch, i), acc ? p1 : p0);
             }
         };
 
@@ -259,58 +259,8 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
             const unsigned rb = kk % kRowBufs;
             const unsigned w0 = (blockIdx.x + kk * gridDim.x) * tr;
             const unsigned nl = warp == 0 ? 0u : sm.nlist[rb];
-            for (unsigned l = (warp - 1) * 2 + half16; l < nl; l += kWorkHalfWarps) {
-                const unsigned rr = sm.list[rb][l];
-                const bool accr = sm.acc[rb][rr] != 0;
-                const unsigned i = p.shard_begin + w0 + rr;
-                double *xk = p.x + (a0 + i) * d;
-                const double *xj = p.x + (size_t)sm.j[rb][rr] * d;
-                double2 xa[4], xb[4];
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const int c = 2 * (ck + 16 * e);
-                    xa[e] = make_double2(0.0, 0.0);
-                    xb[e] = make_double2(0.0, 0.0);
-                    if ((d & 1) == 0) {
-                        if (c < d) {
-                            xa[e] = *reinterpret_cast<const double2 *>(xk + c);
-                            if (accr) xb[e] = __ldcg(reinterpret_cast<const double2 *>(xj + c));
-                        }
-                    } else {
-                        if (c < d) {
-                            xa[e].x = xk[c];
-                            if (accr) xb[e].x = __ldcg(xj + c);
-                        }
-                        if (c + 1 < d) {
-                            xa[e].y = xk[c + 1];
-                            if (accr) xb[e].y = __ldcg(xj + c + 1);
-                        }
-                    }
-                }
-                const double z = sm.z[rb][rr];
-                const size_t o = store ? chain_row(p, sidx, batch, i) : 0;
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const int c = 2 * (ck + 16 * e);
-                    const double v0 = accr ? dadd(xb[e].x, dmul(z, dsub(xa[e].x, xb[e].x))) : xa[e].x;  // :255, same bits
-                    const double v1 = accr ? dadd(xb[e].y, dmul(z, dsub(xa[e].y, xb[e].y))) : xa[e].y;
-                    if ((d & 1) == 0) {
-                        if (c < d) {
-                            if (accr) *reinterpret_cast<double2 *>(xk + c) = make_double2(v0, v1);                     // :261
-                            if (store) __stcs(reinterpret_cast<double2 *>(p.chain_x + o * d + c), make_double2(v0, v1));  // :268-272
-                        }
-                    } else {
-                        if (c < d) {
-                            if (accr) xk[c] = v0;
-                            if (store) __stcs(p.chain_x + o * d + c, v0);
-                        }
-                        if (c + 1 < d) {
-                            if (accr) xk[c + 1] = v1;
-                            if (store) __stcs(p.chain_x + o * d + c + 1, v1);
-                        }
-                    }
-                }
-            }
+            for (unsigned l = (warp - 1) * 2 + half16; l < nl; l += kWorkHalfWarps)
+                fused_writeback_row(p, sm, rb, sm.list[rb][l], w0, a0, d, ck, batch, store, clk.sidx);
         };
 
         K2G_TICK(0);
@@ -325,28 +275,7 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
                     auto row_live = [&](unsigned r) { return r < tr && w0 + r < W; };
                     auto row_load = [&](unsigned r, double2 (&xa)[4], double2 (&xb)[4]) {
                         const unsigned i = p.shard_begin + w0 + r;
-                        const double *xk = p.x + (a0 + i) * d, *xj = p.x + (size_t)sm.j[rb][r] * d;
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const int c = 2 * (ck + 16 * e);
-                            xa[e] = make_double2(0.0, 0.0);
-                            xb[e] = make_double2(0.0, 0.0);
-                            if ((d & 1) == 0) {
-                                if (c < d) {
-                                    xa[e] = *reinterpret_cast<const double2 *>(xk + c);
-                                    xb[e] = __ldcg(reinterpret_cast<const double2 *>(xj + c));
-                                }
-                            } else {
-                                if (c < d) {
-                                    xa[e].x = xk[c];
-                                    xb[e].x = __ldcg(xj + c);
-                                }
-                                if (c + 1 < d) {
-                                    xa[e].y = xk[c + 1];
-                                    xb[e].y = __ldcg(xj + c + 1);
-                                }
-                            }
-                        }
+                        fused_row_load(p.x + (a0 + i) * d, p.x + (size_t)sm.j[rb][r] * d, true, d, ck, xa, xb);
                     };
                     auto row_emit = [&](unsigned r, const double2 (&xa)[4], const double2 (&xb)[4]) {
                         const double zz = sm.z[rb][r];
@@ -354,8 +283,8 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
                         for (int e = 0; e < 4; ++e) {
                             const int c = 2 * (ck + 16 * e);
                             const double2 m = *reinterpret_cast<const double2 *>(sm.mu + c);  // zero past d
-                            const double v0 = dadd(xb[e].x, dmul(zz, dsub(xa[e].x, xb[e].x))) - m.x;  // :255, centred
-                            const double v1 = dadd(xb[e].y, dmul(zz, dsub(xa[e].y, xb[e].y))) - m.y;
+                            const double v0 = stretch_coord(xb[e].x, xa[e].x, zz) - m.x;  // :255, centred
+                            const double v1 = stretch_coord(xb[e].y, xa[e].y, zz) - m.y;
                             unsigned pk[PIECES];
                             split3_pair(v0, v1, pk);
                             const unsigned cp = ck + 16 * e;
@@ -435,11 +364,7 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
                 K2G_TICK(4);
             }
         }
-        if (batch == 1) {
-            if (store) ++sidx;
-            ++n;
-            if (++phase == p.nthin) phase = 0;
-        }
+        if (batch == 1) clk.advance(store, p.nthin);
         if (h + 1 < p.h1) {  // the reference's join between the two half-ensemble sweeps (:248/:273)
             target += gridDim.x;
             __syncthreads();

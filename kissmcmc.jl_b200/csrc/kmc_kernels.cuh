@@ -108,6 +108,45 @@ __device__ __forceinline__ void barrier_wait_acquire(const unsigned long long *c
     } while (v < target);
 }
 
+// The join between two half-steps of a persistent kernel (the reference's join after each sweep, :248/:273), local to
+// this GPU.  The CTA's stores are done before thread 0 arrives; shadow() is work independent of the other CTAs, run
+// between arrive and wait (without it thread 0 arrives and waits at once).  The barrier is polled by thread 0 with
+// relaxed loads and one fence, or, with LAST_WARP_ACQUIRE, by the last warp with acquire loads (thread 0's warp is
+// still behind its release).
+struct NoShadow {
+    __device__ void operator()() const {}
+};
+template <bool LAST_WARP_ACQUIRE = false, class Shadow = NoShadow>
+__device__ __forceinline__ void grid_join(const RunParams &p, unsigned long long &target, Shadow shadow = {}) {
+    auto arrive = [&] { barrier_arrive(p.barrier); };
+    auto wait = [&] {
+        if constexpr (LAST_WARP_ACQUIRE) {
+            if (threadIdx.x == blockDim.x - 32) barrier_wait_acquire(p.barrier, target);
+        } else {
+            if (threadIdx.x == 0) barrier_wait(p.barrier, target);
+        }
+    };
+    target += gridDim.x;
+    __syncthreads();
+    if constexpr (std::is_same<Shadow, NoShadow>::value) {
+        static_assert(!LAST_WARP_ACQUIRE, "without shadow work thread 0 arrives and polls");
+        if (gridDim.x > 1) {
+            if (threadIdx.x == 0) {
+                arrive();
+                wait();
+            }
+            __syncthreads();
+        }
+    } else {
+        if (gridDim.x > 1 && threadIdx.x == 0) arrive();
+        shadow();
+        if (gridDim.x > 1) {
+            wait();
+            __syncthreads();
+        }
+    }
+}
+
 // ------------------------------------------------------------------ accept test
 // Decides  ((N-1)*log(z) + p1) - p0 >= log(u)   (src/samplers.jl:260).
 // Fast filter: t = (p1-p0) + ln2*q,  q = (N-1)*lg2f(z) - lg2f(u)  with FP32 MUFU logs.  The
@@ -256,6 +295,12 @@ __device__ __forceinline__ void cross_gpu_barrier(const RunParams &p, unsigned l
     }
 }
 
+// Peer mode, after the local join of half-step h: every GPU has finished the half-step before anyone gathers from it.
+__device__ __forceinline__ void peer_join(const RunParams &p, unsigned long long &target, long long h) {
+    if (blockIdx.x == 0) cross_gpu_barrier(p, p.epoch_base + (unsigned long long)(h - p.h0) + 1);
+    grid_join(p, target);
+}
+
 // ------------------------------------------------------------------ general kernel
 // Owned state stays in L2/HBM; any ensemble size.  U walkers in flight per thread.
 template <template <int> class Dn, int D, bool REPLAY, bool PEER = false>
@@ -291,11 +336,11 @@ static __global__ void __launch_bounds__(max_threads<D>(), min_blocks<D>()) emce
         if (l < cnt) make_draws(p.h0, l, dr[q]);
     }
 
-    long long n = p.n0, phase = p.phase0, sidx = p.sidx0;
+    ThinClock<> clk{p.n0, p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
     for (long long h = p.h0; h < p.h1; ++h) {
         const int batch = (int)(h & 1);
-        const bool store = (n > 0) && (phase == 0);  // :268  n>0 && rem(n,nthin)==0
+        const bool store = clk.store();
         const unsigned a0 = batch ? p.nhalf : 0u;    // :247 active half
 
         for (unsigned g = 0; g * nthr < cnt; g += U) {  // groups of U walkers in flight
@@ -356,9 +401,9 @@ static __global__ void __launch_bounds__(max_threads<D>(), min_blocks<D>()) emce
                 const double z = dr[q].z;
                 double y[D];
 #pragma unroll
-                for (int c = 0; c < D; ++c) y[c] = dadd(xj[q][c], dmul(z, dsub(xk[q][c], xj[q][c])));  // :255
-                const double p1 = dn.logpdf(y);                                                          // :257
-                const double tt = (p1 - lpk[q]) + (double)dr[q].q * 0.6931471805599453;                  // :260
+                for (int c = 0; c < D; ++c) y[c] = stretch_coord(xj[q][c], xk[q][c], z);  // :255
+                const double p1 = dn.logpdf(y);                                            // :257
+                const double tt = (p1 - lpk[q]) + (double)dr[q].q * 0.6931471805599453;  // :260
                 bool acc;
                 if (tt > (double)p.margin) acc = true;
                 else if (tt < -(double)p.margin) acc = false;
@@ -368,45 +413,27 @@ static __global__ void __launch_bounds__(max_threads<D>(), min_blocks<D>()) emce
                     p.lp[k] = p1;
                     p.nacc[k] += 1u;
                 }
-                if (store) chain_store<D>(p, chain_row(p, sidx, (unsigned)batch, base + l), acc, y, xk[q], p1, lpk[q]);
+                if (store) chain_store<D>(p, chain_row(p, clk.sidx, (unsigned)batch, base + l), acc, y, xk[q], p1, lpk[q]);
             }
         }
         if (batch == 1) {
-            if (n == 0) {  // :285-288 burn-in counters are discarded
+            if (clk.burnin_end()) {  // :285-288 burn-in counters are discarded
                 for (unsigned l = tid; l < cnt; l += nthr) {
                     p.nacc[base + l] = 0u;
                     p.nacc[(size_t)p.nhalf + base + l] = 0u;
                 }
             }
-            if (store) ++sidx;
-            ++n;
-            if (++phase == p.nthin) phase = 0;
+            clk.advance(store, p.nthin);
         }
         if (h + 1 < p.h1) {
-            target += gridDim.x;
-            __syncthreads();
-            if (gridDim.x > 1 && tid == 0) barrier_arrive(p.barrier);
+            grid_join(p, target, [&] {
 #pragma unroll
-            for (int q = 0; q < U; ++q) {  // next half-step's first group of draws, in the barrier's shadow
-                const unsigned l = tid + q * nthr;
-                if (l < cnt) make_draws(h + 1, l, dr[q]);
-            }
-            if (gridDim.x > 1) {
-                if (tid == 0) barrier_wait(p.barrier, target);
-                __syncthreads();
-            }
-            if constexpr (PEER) {  // every GPU has finished the half-step before anyone gathers from it
-                if (blockIdx.x == 0) cross_gpu_barrier(p, p.epoch_base + (unsigned long long)(h - p.h0) + 1);
-                target += gridDim.x;
-                __syncthreads();
-                if (gridDim.x > 1) {
-                    if (tid == 0) {
-                        barrier_arrive(p.barrier);
-                        barrier_wait(p.barrier, target);
-                    }
-                    __syncthreads();
+                for (int q = 0; q < U; ++q) {  // next half-step's first group of draws, in the barrier's shadow
+                    const unsigned l = tid + q * nthr;
+                    if (l < cnt) make_draws(h + 1, l, dr[q]);
                 }
-            }
+            });
+            if constexpr (PEER) peer_join(p, target, h);
         }
     }
 }
@@ -468,11 +495,11 @@ static __global__ void __launch_bounds__(kBulkThreads, KMC_BULK_CTAS) emcee_bulk
     };
     if (tid < cnt) make_draw(p.h0, tid);
 
-    long long n = p.n0, phase = p.phase0, sidx = p.sidx0;
+    ThinClock<> clk{p.n0, p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
     for (long long h = p.h0; h < p.h1; ++h) {
         const unsigned batch = (unsigned)(h & 1);
-        const bool store = (n > 0) && (phase == 0);
+        const bool store = clk.store();
         const size_t a0 = batch ? (size_t)p.nhalf : 0;
         for (unsigned g = 0; g < ngroups; ++g, ++gcount) {
             const unsigned rows = min(T, cnt - g * T);
@@ -508,9 +535,9 @@ static __global__ void __launch_bounds__(kBulkThreads, KMC_BULK_CTAS) emcee_bulk
                 }
                 const double z = dr.z;
 #pragma unroll
-                for (int c = 0; c < D; ++c) y[c] = dadd(xj[c], dmul(z, dsub(xk[c], xj[c])));  // :255
-                const double p1 = dn.logpdf(y);                                                // :257
-                const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;             // :260
+                for (int c = 0; c < D; ++c) y[c] = stretch_coord(xj[c], xk[c], z);  // :255
+                const double p1 = dn.logpdf(y);                                      // :257
+                const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;   // :260
                 bool acc;
                 if (tt > (double)p.margin) acc = true;
                 else if (tt < -(double)p.margin) acc = false;
@@ -526,7 +553,7 @@ static __global__ void __launch_bounds__(kBulkThreads, KMC_BULK_CTAS) emcee_bulk
                     p.lp[k] = p1;
                     p.nacc[k] += 1u;
                 }
-                if (store) chain_store<D>(p, chain_row(p, sidx, batch, base + l), acc, y, xk, p1, lpk);
+                if (store) chain_store<D>(p, chain_row(p, clk.sidx, batch, base + l), acc, y, xk, p1, lpk);
             }
 #if KMC_BULK_STORE_ALL
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // smem writes -> bulk store
@@ -535,15 +562,13 @@ static __global__ void __launch_bounds__(kBulkThreads, KMC_BULK_CTAS) emcee_bulk
 #endif
         }
         if (batch == 1) {
-            if (n == 0) {  // :285-288
+            if (clk.burnin_end()) {  // :285-288
                 for (unsigned l = tid; l < cnt; l += T) {
                     p.nacc[base + l] = 0u;
                     p.nacc[(size_t)p.nhalf + base + l] = 0u;
                 }
             }
-            if (store) ++sidx;
-            ++n;
-            if (++phase == p.nthin) phase = 0;
+            clk.advance(store, p.nthin);
         }
 #if KMC_BULK_STORE_ALL
         if (tid == 0) {  // all of this CTA's row stores are complete and ordered before the barrier
@@ -692,14 +717,12 @@ static __global__ void __launch_bounds__(kSmemThreads, kSmemCtas) emcee_smem_ker
 
     // launch-local 32-bit bookkeeping of the reference's n (:245), rem(n, nthin) and the sample index
     const unsigned nh = (unsigned)(p.h1 - p.h0);
-    long long n = p.n0;
-    unsigned phase = (unsigned)p.phase0;
-    long long sidx = p.sidx0;
+    ThinClock<unsigned> clk{p.n0, (unsigned)p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
     for (unsigned hh = 0; hh < nh; ++hh) {
         const long long h = p.h0 + hh;
         const unsigned batch = (unsigned)(h & 1);
-        const bool store = (n > 0) && (phase == 0);  // :268  n>0 && rem(n,nthin)==0
+        const bool store = clk.store();
         const unsigned hslot = batch ? p.per_cta : 0u;            // first slot of the active half
         const size_t hrow = batch ? (size_t)p.nhalf : (size_t)0;  // first global row of the active half (:247)
 
@@ -719,7 +742,7 @@ static __global__ void __launch_bounds__(kSmemThreads, kSmemCtas) emcee_smem_ker
             const double lpk = lds_f64(sbase + 8u * (D * L + sl));
             const double z = dr[q].z;
 #pragma unroll
-            for (int c = 0; c < D; ++c) y[c] = dadd(xj[q % kAhead][c], dmul(z, dsub(xk[c], xj[q % kAhead][c])));  // :255
+            for (int c = 0; c < D; ++c) y[c] = stretch_coord(xj[q % kAhead][c], xk[c], z);  // :255
             if (q + kAhead < kRounds && q + kAhead < nv)  // partner row kAhead rounds ahead, before this round's stores
                 load_row_cg<D>(p.x + (size_t)dr[(q + kAhead) % kRounds].j * D, xj[q % kAhead]);
             const double p1 = dn.logpdf(y);                                        // :257
@@ -735,29 +758,18 @@ static __global__ void __launch_bounds__(kSmemThreads, kSmemCtas) emcee_smem_ker
                 sts_f64(sbase + 8u * (D * L + sl), p1);
                 sts_u32(nbase + 4u * sl, lds_u32(nbase + 4u * sl) + 1u);
             }
-            if (store) chain_store<D>(p, chain_row(p, sidx, batch, wid + q * nthr), acc, y, xk, p1, lpk);
+            if (store) chain_store<D>(p, chain_row(p, clk.sidx, batch, wid + q * nthr), acc, y, xk, p1, lpk);
         }
         if (batch == 1) {
-            if (n == 0)  // :285-288 burn-in counters are discarded
+            if (clk.burnin_end())  // :285-288 burn-in counters are discarded
                 for (unsigned q = 0; q < nv; ++q) {
                     sts_u32(nbase + 4u * (q * nthr), 0u);
                     sts_u32(nbase + 4u * (p.per_cta + q * nthr), 0u);
                 }
-            if (store) ++sidx;
-            ++n;
-            if (++phase == (unsigned)p.nthin) phase = 0;
+            clk.advance(store, (unsigned)p.nthin);
         }
-        if (hh + 1 < nh) {
-            target += gridDim.x;
-            __syncthreads();
-            if (gridDim.x > 1 && threadIdx.x == 0) barrier_arrive(p.barrier);
-            make_draws(h + 1, SplitLo{}, SplitMid{});  // in the barrier's shadow: independent of the other CTAs
-            if (gridDim.x > 1) {
-                // the LAST warp polls: thread 0's warp is still behind its release (a membar over the CTA's row stores)
-                if (threadIdx.x == blockDim.x - 32) barrier_wait_acquire(p.barrier, target);
-                __syncthreads();
-            }
-        }
+        if (hh + 1 < nh)  // the draws in the barrier's shadow are independent of the other CTAs
+            grid_join<true>(p, target, [&] { make_draws(h + 1, SplitLo{}, SplitMid{}); });
     }
 
     for (unsigned b = 0; b < 2; ++b)  // write back what only lived in shared memory

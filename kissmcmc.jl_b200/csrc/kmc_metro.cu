@@ -43,9 +43,8 @@ int32_t mh_run_batched(kmc_sampler_s *s, kmc::MhParams &p, long long t0, long lo
     for (long long t = t0; t < t1; ++t) {
         p.t0 = t;
         p.t1 = t + 1;
-        const long long ni = t + 1 - s->opts.nburnin_walker;
-        const int store = (ni > 0 && ni % s->opts.nthin == 0) ? 1 : 0;
-        const long long sidx = store ? ni / s->opts.nthin - 1 : 0;
+        const auto clk = kmc::ThinClock<>::at(t, s->opts.nburnin_walker, s->opts.nthin);
+        const int store = clk.store() ? 1 : 0;
         if (s->chol) {  // Z, U; then Y = X + L Z
             normals<<<gp, 256, 0, s->stream>>>(p, t, d, s->d_z, s->bb.u);
             kmc::mh_chol_kernel<<<gt, dim3(kmc::kMhTri, 8), 0, s->stream>>>(s->x, s->d_chol, s->d_z, s->nw, d, s->bb.Y);
@@ -53,7 +52,7 @@ int32_t mh_run_batched(kmc_sampler_s *s, kmc::MhParams &p, long long t0, long lo
             propose<<<gp, 256, 0, s->stream>>>(p, s->d_sigma, t, d, s->bb.Y, s->bb.u);
         }
         CU_TRY(eval_on_device(*s->dn, s->bb.Y, s->nw, s->bb.p1, s->bsc, s->stream));
-        kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, ni, store, sidx);
+        kmc::mh_accept_kernel<<<ga, 256, 0, s->stream>>>(p, s->bb.Y, s->bb.p1, s->bb.u, d, clk.n, store, clk.sidx);
     }
     CU_TRY(cudaGetLastError());
     launches = (t1 - t0) * ((s->chol ? 3 : 2) + eval_launches(*s->dn));

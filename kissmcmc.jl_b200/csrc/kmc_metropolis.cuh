@@ -122,10 +122,10 @@ __device__ __forceinline__ void metropolis_chain(const MhParams &p, const Dn<D> 
     double lp = p.lp[c];
     unsigned na = p.nacc[c];
     const unsigned cid = p.id_base + (unsigned)c;
-    long long ni = p.t0 + 1 - p.nburnin;  // the reference's loop variable at step t0
-    long long ph = ni % p.nthin;
-    if (ph < 0) ph += p.nthin;
-    long long sidx = ni >= 1 ? (ni - 1) / p.nthin : 0;  // samples stored before ni
+    // the reference's loop variable at step t0, its phase and the samples stored before it; the loop below advances its
+    // own copy (ThinClock::advance here does not compile to the same code)
+    const ThinClock<> clk0 = ThinClock<>::at(p.t0, p.nburnin, p.nthin);
+    long long ni = clk0.n, ph = clk0.phase, sidx = clk0.sidx;
     for (long long t = p.t0; t < p.t1; ++t) {
         double y[D], u;
         if constexpr (REPLAY) {

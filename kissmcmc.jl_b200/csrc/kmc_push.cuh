@@ -336,14 +336,14 @@ __global__ void __launch_bounds__(kPushThreads, KMC_PUSH_CTAS) emcee_push_kernel
 #else
 #define PUSH_TICK(i) do { } while (0)
 #endif
-    long long n = p.n0, phase = p.phase0, sidx = p.sidx0;
+    ThinClock<> clk{p.n0, p.phase0, p.sidx0};
     unsigned long long target = p.bar_base;
     unsigned long long next = 0;
 
     for (long long h = p.h0; h < p.h1; ++h) {
         const unsigned batch = (unsigned)(h & 1);
-        const bool store = (n > 0) && (phase == 0);      // :268
-        const bool reset = (batch == 1) && (n == 0);     // :285-288
+        const bool store = clk.store();
+        const bool reset = (batch == 1) && clk.burnin_end();
         const size_t act = batch ? (size_t)S : 0;         // first local row of the active half
         const size_t pas = batch ? 0 : (size_t)S;         // first local row of the passive half
         const unsigned par = (unsigned)(h & 1);           // ring parity
@@ -596,9 +596,9 @@ __global__ void __launch_bounds__(kPushThreads, KMC_PUSH_CTAS) emcee_push_kernel
                     }
                     const double z = dr.z;
 #pragma unroll
-                    for (int cc = 0; cc < D; ++cc) y[cc] = dadd(xj[cc], dmul(z, dsub(xk[cc], xj[cc])));  // :255
-                    const double p1 = dn.logpdf(y);                                                    // :257
-                    const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;                 // :260
+                    for (int cc = 0; cc < D; ++cc) y[cc] = stretch_coord(xj[cc], xk[cc], z);  // :255
+                    const double p1 = dn.logpdf(y);                                          // :257
+                    const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;       // :260
                     bool acc;
                     if (tt > (double)p.margin) acc = true;
                     else if (tt < -(double)p.margin) acc = false;
@@ -612,7 +612,7 @@ __global__ void __launch_bounds__(kPushThreads, KMC_PUSH_CTAS) emcee_push_kernel
                         p.nacc[l] = 0u;
                         p.nacc[(size_t)S + l] = 0u;
                     }
-                    if (store) chain_store<D>(p, chain_row(p, sidx, batch, me * S + l), acc, y, xk, p1, lpk);
+                    if (store) chain_store<D>(p, chain_row(p, clk.sidx, batch, me * S + l), acc, y, xk, p1, lpk);
                 }
                 PUSH_TICK(7);
 #ifdef KMC_PUSH_PROF
@@ -628,11 +628,7 @@ __global__ void __launch_bounds__(kPushThreads, KMC_PUSH_CTAS) emcee_push_kernel
             PUSH_TICK(8);
         }
 
-        if (batch == 1) {
-            if (store) ++sidx;
-            ++n;
-            if (++phase == p.nthin) phase = 0;
-        }
+        if (batch == 1) clk.advance(store, p.nthin);
         PUSH_TICK(9);
         if (tid == 0) {  // all of this CTA's messages are complete: the last notes go out
             service();
