@@ -109,10 +109,12 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
 int32_t kmc_density_destroy(kmc_density_t h);
 /* Options: "tensor_cores" = 0/1.  Every plugin is exact FP64 by default.  1 opts in to the tcgen05 kernels, which are
  * APPROXIMATE with a stated tolerance: the dense Gaussian with 16 < d <= 128 (|logp - logp_fp64| <= 1e-5 (1 + |y|^2))
- * and logistic regression with d <= 64 and bf16-representable data (log-density DIFFERENCES between nearby points --
- * what the accept test sees -- within 2e-3 at N = 10^6; the value itself carries a common offset of up to ~1e-7 N
- * that cancels in every accept test but is present in the stored log-densities).  Returns KMC_ERR_UNSUPPORTED if the
- * density has no tensor-core path.
+ * and logistic regression with d <= 64 and bf16-representable data, whose error grows with the size of the logits:
+ * per point |logp - logp_fp64| <= u [(0.5 + 1.05 m) sum_n sum_k |theta_k x_nk| + 8.5 sum_n |theta . x_n|] + 5 u N,
+ * u = 2^-24, m = ceil(d/16) (at most 13.2 u sum_n sum_k |theta_k x_nk| + 5 u N), and the sum of two points' bounds on
+ * their difference.  At d = 32, N = 10^6 and theta* ~ N(0, 1/d) (mean |logit| 0.7) that is ~1.3 per point (measured:
+ * a common offset of ~3e-2 that cancels in every accept test, 2e-3 on differences); with the data drawn from 16 theta*
+ * (mean |logit| 11), ~13.  Returns KMC_ERR_UNSUPPORTED if the density has no tensor-core path.
  * "fused_variant" = 2/1: which fused persistent kernel the tensor-core dense Gaussian uses in
  * launch_mode 0 -- 2 (default): matrix pieces resident in TMEM; 1: matrix pieces in shared memory
  * (bit-identical to the three-kernel pipeline of launch_mode 1).

@@ -118,9 +118,13 @@ def logistic(X, y, prior_sigma: float = 10.0, device: int = 0, tensor_cores: boo
 
     Exact FP64 by default.  Any d <= 512.  tensor_cores=True opts in to the tcgen05 kernel (needs d <= 64 and every X value
     bf16-representable, else KmcError): theta split into three bf16 pieces, FP32 accumulation, FP32 softplus.
-    It is APPROXIMATE: log-density differences between nearby points (what the accept test sees) agree with FP64 to
-    2e-3 at N = 10^6 (6e-4 rms); the value itself -- the stored `logdensities` and the initial p0s -- carries a common
-    offset of about +3e-8 per data row (+3e-2 at N = 10^6) that cancels in every accept test."""
+    It is APPROXIMATE, and its error grows with the size of the logits.  Per point, with u = 2^-24 and m = ceil(d/16):
+        |logp - logp_fp64| <= u [(0.5 + 1.05 m) sum_n sum_k |theta_k x_nk| + 8.5 sum_n |theta . x_n|] + 5 u N
+    (at most 13.2 u sum_n sum_k |theta_k x_nk| + 5 u N), and the sum of the two bounds on a difference of two points.
+    At d = 32, N = 10^6, theta* ~ N(0, 1/d) (mean |logit| 0.7) that is ~1.3 per point; a B200 shows a common offset of
+    about +3e-2 (+3e-8 per data row, in the stored `logdensities` and the initial p0s, cancelling in every accept test)
+    and 2e-3 on differences between nearby points.  With the data drawn from 16 theta* (mean |logit| 11) the bound is
+    ~13 per point."""
     X = np.ascontiguousarray(X, dtype=np.float32)
     y = np.ascontiguousarray(y, dtype=np.float32).ravel()
     assert X.ndim == 2 and y.size == X.shape[0]

@@ -10,9 +10,15 @@
 //
 //   * operands: X is bf16 (the plugin requires bf16-representable data, checked at creation, so
 //     this is exact); theta (FP64) is split into three bf16 pieces hi+mid+lo (24 significant
-//     bits).  bf16 x bf16 products are exact in FP32, the accumulation is FP32 in TMEM:
-//     logits carry ~1e-6 absolute error, the row sum over 1e6 data points ~3e-4 (stated
-//     tolerance on the log-density DIFFERENCE in the tests: 2e-3 at N = 1e6).
+//     bits).  bf16 x bf16 products are exact in FP32, the accumulation is FP32 in TMEM, so a
+//     logit carries an absolute error of a few 2^-24 sum_k |theta_k x_nk| and the N rows add
+//     theirs up.  Bound per point, derived in tests/test_tc_error_model.py (u = 2^-24,
+//     m = ceil(d/16)):  |R_tc - R| <= u [(0.5 + 1.05 m) sum_n sum_k |theta_k x_nk|
+//     + 8.5 sum_n |theta . x_n|] + 5 u N  <=  13.2 u sum_n sum_k |theta_k x_nk| + 5 u N;
+//     a difference of two points, the sum of their bounds.  It grows with the logit scale:
+//     ~1.3 per point at the bench problem (d = 32, N = 1e6, theta*), ~13 with the data drawn
+//     from 16 theta*; on the bench problem a B200 shows ~3e-2 (a common offset) per point and
+//     2e-3 on differences.
 //   * one CTA per SM, persistent over work items (walker tile of 128, chunk of data tiles):
 //       warp 0     TMA producer: A = 3 theta pieces [128 x 32] once per item, B = X tile
 //                  [256 x 32] per stage (4 stages), SWIZZLE_64B K-major, mbarrier complete_tx
@@ -453,7 +459,9 @@ __global__ void logistic_tc_finish_kernel(const double *__restrict__ TH, const d
 //   Both operands are FP64 on the host side and are split into three bf16 pieces each; the six
 //   piece pairs whose product is above 2^-24 relative are accumulated in FP32 in TMEM, smallest
 //   first:  (lo,hi) (hi,lo) (mid,mid) (mid,hi) (hi,mid) (hi,hi)   [C piece, A piece].
-//   Stated tolerance vs the FP64 kernel: |logp_tc - logp_fp64| <= 1e-5 * (1 + |y|^2).
+//   Stated tolerance vs the FP64 kernel: |logp_tc - logp_fp64| <= 1e-5 * (1 + |y|^2); the bound derived
+//   from the arithmetic (tests/test_tc_error_model.py), P = |A| |x - mu|:
+//   21 u sum_i |y_i| P_i + 16 u |y|^2 + (21 u)^2 |P|^2 / 2, u = 2^-24.
 //
 //   smem: A pieces 3 x 32 KB resident for the whole kernel + C pieces 3 x 32 KB per walker tile,
 //   each piece = 2 k-halves of [128 rows x 128 B], SWIZZLE_128B K-major (TMA box 64 x 128).

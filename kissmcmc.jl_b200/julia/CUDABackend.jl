@@ -106,7 +106,10 @@ lognormal(mu=0.0, sigma=1.0; device=0) =
 
 Bayesian logistic regression (BASELINE.json configs[3]): `X` is N x d, `y` in {0,1}, prior N(0, sigma^2 I).
 Exact FP64 by default; `tensor_cores=true` opts in to the tcgen05 kernel (d <= 64 and bf16-representable X; FP64: any d <= 512), which is
-approximate: log-density differences within 2e-3 at N = 10^6, the value itself carries a common offset of ~3e-8 N.
+approximate, with an error that grows with the size of the logits: per point, with u = 2^-24 and m = ceil(d/16),
+`|logp - logp_fp64| <= u [(0.5 + 1.05 m) sum_n sum_k |theta_k x_nk| + 8.5 sum_n |theta . x_n|] + 5 u N`, and the sum of
+two points' bounds on their difference.  At d = 32, N = 10^6, theta* ~ N(0, 1/d) that is ~1.3 per point (a B200 shows
+a common offset of ~3e-8 N and 2e-3 on differences); with the data drawn from 16 theta*, ~13.
 """
 function logistic(X::AbstractMatrix, y::AbstractVector; prior_sigma=10.0, device=0, tensor_cores=false)
     N, d = size(X)
