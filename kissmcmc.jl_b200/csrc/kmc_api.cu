@@ -26,7 +26,6 @@ thread_local std::string g_err;
 }
 
 const std::string &last_error() { return g_err; }
-void set_last_error(const std::string &msg) { g_err = msg; }
 
 int32_t fail(int32_t code, const char *fmt, ...) {
     char buf[512];
@@ -74,10 +73,12 @@ cudaError_t dev_alloc_raw(void **out, size_t bytes, int device) {
         g_cache.cached_bytes = 0;
         e = cudaMalloc(out, bytes);
     }
-    if (e == cudaSuccess) {
-        std::lock_guard<std::mutex> lk(g_cache.mu);
-        g_cache.live[*out] = {device, bytes};
+    if (e != cudaSuccess) {
+        cudaGetLastError();  // the failure is returned here, not left for a later cudaGetLastError check to report
+        return e;
     }
+    std::lock_guard<std::mutex> lk(g_cache.mu);
+    g_cache.live[*out] = {device, bytes};
     return e;
 }
 
@@ -222,35 +223,17 @@ cudaError_t batch_scratch_reserve(BatchScratch &sc, const kmc_density_s &dn, lon
     const TcPlan pl = tcp ? tc_plan(dn, npts) : TcPlan{};
     if (tcp) {
         const size_t pneed = sizeof(__nv_bfloat16) * kmc::tc::PIECES * (size_t)pl.lp.wpad * dn.kp;
-        if (pneed > sc.pieces_bytes) {
-            dev_free(sc.pieces);
-            sc.pieces = nullptr;
-            sc.pieces_bytes = 0;
-            cudaError_t e = dev_alloc(&sc.pieces, pneed, dn.device);
-            if (e != cudaSuccess) return e;
-            sc.pieces_bytes = pneed;
-        }
+        const cudaError_t e = reserve(sc.pieces, sc.pieces_bytes, pneed, dn.device);
+        if (e != cudaSuccess) return e;
     }
     const size_t need = sizeof(double) * (size_t)(tcp ? pl.lp.nchunks : kLogitChunks) * (size_t)npts;
-    if (need <= sc.bytes) return cudaSuccess;
-    dev_free(sc.part);
-    sc.part = nullptr;
-    sc.bytes = 0;
-    cudaError_t e = dev_alloc(&sc.part, need, dn.device);
-    if (e == cudaSuccess) sc.bytes = need;
-    return e;
+    return reserve(sc.part, sc.bytes, need, dn.device);
 }
 
 cudaError_t gauss_pieces_reserve(BatchScratch &sc, const kmc_density_s &dn, long long npts) {
     const long long wpad = ((npts + kmc::tc::BM - 1) / kmc::tc::BM) * kmc::tc::BM;
     const size_t pneed = sizeof(__nv_bfloat16) * kmc::tc::PIECES * (size_t)wpad * kmc::tc::GK;
-    if (pneed <= sc.pieces_bytes) return cudaSuccess;
-    dev_free(sc.pieces);
-    sc.pieces = nullptr;
-    sc.pieces_bytes = 0;
-    cudaError_t e = dev_alloc(&sc.pieces, pneed, dn.device);
-    if (e == cudaSuccess) sc.pieces_bytes = pneed;
-    return e;
+    return reserve(sc.pieces, sc.pieces_bytes, pneed, dn.device);
 }
 
 // The tcgen05 Mahalanobis GEMM on centred bf16 pieces [3][wpad][128] already in sc.pieces.
@@ -264,7 +247,7 @@ cudaError_t launch_gauss_tc(const kmc_density_s &dn, BatchScratch &sc, long long
     gp.lognorm = dn.params[d + (size_t)d * d];
     gp.out = out;
     CUtensorMap mapC;
-    if (!make_map_bf16_k128(&mapC, sc.pieces, (unsigned long long)kmc::tc::PIECES * gp.wpad, kmc::tc::BM))
+    if (!make_map_bf16_k128(&mapC, sc.pieces.get(), (unsigned long long)kmc::tc::PIECES * gp.wpad, kmc::tc::BM))
         return cudaErrorInvalidValue;
     const size_t smem = sizeof(kmc::tc::GaussSmem) + 1024;
     cudaError_t e = cudaFuncSetAttribute(kmc::tc::gaussian_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -283,8 +266,8 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
         if (e != cudaSuccess) return e;
         const long long wpad = ((npts + kmc::tc::BM - 1) / kmc::tc::BM) * kmc::tc::BM;
         const long long ne = wpad * kmc::tc::GK;
-        kmc::tc::split_rows128_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(X, dn.d_params, sc.pieces, npts,
-                                                                                    wpad, d);
+        kmc::tc::split_rows128_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(X, dn.d_params, sc.pieces.get(),
+                                                                                    npts, wpad, d);
         return launch_gauss_tc(dn, sc, npts, out, st);
     }
     if (dn.ops.batch == BATCH_GAUSSIAN && d > kmc::kWideMaxD) {
@@ -319,13 +302,13 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
         cudaError_t e = batch_scratch_reserve(sc, dn, npts);
         if (e != cudaSuccess) return e;
         TcPlan pl = tc_plan(dn, npts);
-        pl.lp.part = sc.part;
+        pl.lp.part = sc.part.get();
         const int kp = dn.kp;  // d zero-padded to the GEMM's K (32 or 64)
         const long long ne = pl.lp.wpad * kp;
-        kmc::tc::split_theta_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(X, sc.pieces, npts, pl.lp.wpad, d, kp,
-                                                                                       1.4426950408889634);
+        kmc::tc::split_theta_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, st>>>(X, sc.pieces.get(), npts, pl.lp.wpad, d,
+                                                                                       kp, 1.4426950408889634);
         CUtensorMap mapA;
-        if (!make_map_bf16_k(&mapA, sc.pieces, (unsigned long long)kmc::tc::PIECES * pl.lp.wpad, kmc::tc::BM, kp))
+        if (!make_map_bf16_k(&mapA, sc.pieces.get(), (unsigned long long)kmc::tc::PIECES * pl.lp.wpad, kmc::tc::BM, kp))
             return cudaErrorInvalidValue;
         if (kp == 32) {
             const size_t smem = sizeof(kmc::tc::Smem<32>) + 1024;
@@ -340,7 +323,7 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
         }
         const double sg = dn.params[0];
         kmc::tc::logistic_tc_finish_kernel<<<(unsigned)((npts + 255) / 256), 256, 0, st>>>(
-            X, sc.part, dn.d_xty, out, npts, d, pl.lp.nchunks, 0.5 / (sg * sg));
+            X, sc.part.get(), dn.d_xty, out, npts, d, pl.lp.nchunks, 0.5 / (sg * sg));
         return cudaGetLastError();
     }
     if (dn.ops.batch == BATCH_LOGISTIC) {
@@ -353,9 +336,9 @@ cudaError_t launch_batch_logp(const kmc_density_s &dn, const double *X, long lon
             e = cudaFuncSetAttribute(kmc::logistic_logp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
         }
-        kmc::logistic_logp_kernel<<<grid, 256, smem, st>>>(X, sc.part, npts, d, dn.d_X, dn.d_y, dn.ndata, rows);
+        kmc::logistic_logp_kernel<<<grid, 256, smem, st>>>(X, sc.part.get(), npts, d, dn.d_X, dn.d_y, dn.ndata, rows);
         const double sg = dn.params[0];
-        kmc::logistic_finish_kernel<<<(unsigned)((npts + 255) / 256), 256, 0, st>>>(X, sc.part, out, npts, d,
+        kmc::logistic_finish_kernel<<<(unsigned)((npts + 255) / 256), 256, 0, st>>>(X, sc.part.get(), out, npts, d,
                                                                                      kLogitChunks, 0.5 / (sg * sg));
         return cudaGetLastError();
     }
@@ -419,6 +402,36 @@ int32_t sampler_init(kmc_sampler_s *s, const double *theta0s) {
         CU_TRY(dev_alloc(&s->bb.p1, sizeof(double) * s->scnt, dev));
     }
     CU_TRY(eval_on_device(*s->dn, s->x, s->nstate, s->lp, s->bsc, s->stream));  // p0 = pdf(theta0), :209-210
+    return KMC_OK;
+}
+
+int32_t chain_gather(kmc_sampler_s *s, const unsigned *idx, long long nk, double *thetas, double *logp) {
+    const long long ns = s->ns, nl = s->nl;
+    const int d = s->d;
+    // walkers per staging chunk: <= 64 MiB of [wc][ns][d] doubles
+    const long long wc = std::min(nk, std::max<long long>(32, (64LL << 20) / (sizeof(double) * ns * d)));
+    DevBuf<double> stage;
+    CU_TRY(dev_alloc(stage, sizeof(double) * wc * ns * d, s->opts.device));
+    auto transpose = idx ? kmc::chain_transpose_kernel<true> : kmc::chain_transpose_kernel<false>;
+    const dim3 blk(32, 8);
+    for (long long w0 = 0; w0 < nk; w0 += wc) {
+        const long long cur = std::min(wc, nk - w0);
+        for (int what = 0; what < 2; ++what) {
+            double *host = what == 0 ? thetas : logp;
+            if (!host) continue;
+            const int dd = what == 0 ? d : 1;
+            const double *src = what == 0 ? s->chain_x : s->chain_lp;
+            for (long long s0 = 0; s0 < ns; s0 += kmc::kTransposeMaxSamples) {
+                const long long sc = std::min(kmc::kTransposeMaxSamples, ns - s0);
+                const dim3 grd((unsigned)((cur + 31) / 32), (unsigned)((sc + 31) / 32), (unsigned)dd);
+                transpose<<<grd, blk, 0, s->stream>>>(src, stage.get(), ns, nl, w0, cur, dd, s0, idx);
+            }
+            CU_TRY(cudaMemcpyAsync(host + w0 * ns * dd, stage.get(), sizeof(double) * cur * ns * dd,
+                                   cudaMemcpyDeviceToHost, s->stream));
+        }
+    }
+    CU_TRY(cudaStreamSynchronize(s->stream));
+    CU_TRY(cudaGetLastError());
     return KMC_OK;
 }
 
@@ -519,7 +532,7 @@ int32_t run_batched(kmc_sampler_s *s, kmc::RunParams &p, long long h0, long long
         const auto clk = set_range(p, s, h, h + 1);
         const int store = clk.store() ? 1 : 0;
         if (gtc) {
-            propose_pieces<<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, dn.d_params, s->bsc.pieces, wpad);
+            propose_pieces<<<gridp, 256, 0, s->stream>>>(p, s->bb, h, s->d, dn.d_params, s->bsc.pieces.get(), wpad);
             CU_TRY(launch_gauss_tc(dn, s->bsc, s->scnt, s->bb.p1, s->stream));
             accept_recompute<<<grid, 256, 0, s->stream>>>(p, s->bb, h, s->d, clk.n, store, clk.sidx);
         } else {
@@ -610,7 +623,8 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
     if (nparams != ops.nparams)
         return fail(KMC_ERR_INVALID, "plugin '%s' with d=%d takes %d parameters, got %lld", name, d,
                     ops.nparams, (long long)nparams);
-    auto *h = new kmc_density_s;
+    // the density under construction, deleted by kmc_density_destroy on every exit but the last
+    std::unique_ptr<kmc_density_s, int32_t (*)(kmc_density_t)> h(new kmc_density_s, kmc_density_destroy);
     h->kind = kind;
     h->d = d;
     h->device = device;
@@ -623,52 +637,43 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
     }
     if (ops.batch) {  // batched plugins keep parameters (and data) in device memory
         if (nparams) h->params.assign(params, params + nparams);
-        cudaError_t e = cudaSetDevice(device);
-        if (e == cudaSuccess) {
-            int nsm = 0;
-            cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
-            h->nsm = nsm > 0 ? nsm : 148;
+        CU_TRY(cudaSetDevice(device));
+        int nsm = 0;
+        cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device);
+        h->nsm = nsm > 0 ? nsm : 148;
+        if (nparams) {
+            CU_TRY(dev_alloc(&h->d_params, sizeof(double) * nparams, device));
+            CU_TRY(cudaMemcpy(h->d_params, params, sizeof(double) * nparams, cudaMemcpyHostToDevice));
         }
-        if (e == cudaSuccess && nparams) e = dev_alloc(&h->d_params, sizeof(double) * nparams, device);
-        if (e == cudaSuccess && nparams) e = cudaMemcpy(h->d_params, params, sizeof(double) * nparams, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && ops.batch == BATCH_GAUSSIAN) {  // A^T padded to a multiple of 128 rows for the FP64 kernels
+        if (ops.batch == BATCH_GAUSSIAN) {  // A^T padded to a multiple of 128 rows for the FP64 kernels
             const size_t dpad = (size_t)(d + 127) / 128 * 128;
             std::vector<double> At((size_t)d * dpad, 0.0);
             for (int i = 0; i < d; ++i)
                 for (int j = 0; j < d; ++j) At[(size_t)j * dpad + i] = params[d + (size_t)i * d + j];
-            e = dev_alloc(&h->d_At, sizeof(double) * At.size(), device);
-            if (e == cudaSuccess) e = cudaMemcpy(h->d_At, At.data(), sizeof(double) * At.size(), cudaMemcpyHostToDevice);
+            CU_TRY(dev_alloc(&h->d_At, sizeof(double) * At.size(), device));
+            CU_TRY(cudaMemcpy(h->d_At, At.data(), sizeof(double) * At.size(), cudaMemcpyHostToDevice));
         }
-        if (e == cudaSuccess && ops.batch == BATCH_GAUSSIAN && d <= kmc::kWideMaxD) {  // matrix pieces for the tcgen05 Mahalanobis GEMM
-            e = dev_alloc(&h->d_Abf, sizeof(__nv_bfloat16) * kmc::tc::PIECES * kmc::tc::GN * kmc::tc::GK, device);
-            if (e == cudaSuccess) {
-                const long long ne = (long long)kmc::tc::GN * kmc::tc::GK;
-                kmc::tc::split_rows128_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(h->d_params + d, nullptr, h->d_Abf, d,
-                                                                                    kmc::tc::GN, d);
-                e = cudaDeviceSynchronize();
-            }
-            if (e == cudaSuccess)
-                h->tc_ok = make_map_bf16_k128(&h->mapA, h->d_Abf, (unsigned long long)kmc::tc::PIECES * kmc::tc::GN,
-                                              kmc::tc::GN);
+        if (ops.batch == BATCH_GAUSSIAN && d <= kmc::kWideMaxD) {  // matrix pieces for the tcgen05 Mahalanobis GEMM
+            CU_TRY(dev_alloc(&h->d_Abf, sizeof(__nv_bfloat16) * kmc::tc::PIECES * kmc::tc::GN * kmc::tc::GK, device));
+            const long long ne = (long long)kmc::tc::GN * kmc::tc::GK;
+            kmc::tc::split_rows128_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(h->d_params + d, nullptr, h->d_Abf, d,
+                                                                                kmc::tc::GN, d);
+            CU_TRY(cudaDeviceSynchronize());
+            h->tc_ok = make_map_bf16_k128(&h->mapA, h->d_Abf, (unsigned long long)kmc::tc::PIECES * kmc::tc::GN,
+                                          kmc::tc::GN);
         }
-        if (e == cudaSuccess && ops.batch == BATCH_LOGISTIC) {
+        if (ops.batch == BATCH_LOGISTIC) {
             const long long N = data_bytes / (long long)(sizeof(float) * (d + 1));
-            if (!data || N < 1 || N * (long long)(sizeof(float) * (d + 1)) != data_bytes) {
-                kmc_density_destroy(h);
+            if (!data || N < 1 || N * (long long)(sizeof(float) * (d + 1)) != data_bytes)
                 return fail(KMC_ERR_INVALID, "logistic needs data = float32 X[N][d] then y[N] (%d+1 floats per row)", d);
-            }
-            if (!(params[0] > 0.0)) {
-                kmc_density_destroy(h);
-                return fail(KMC_ERR_INVALID, "logistic prior_sigma must be > 0");
-            }
+            if (!(params[0] > 0.0)) return fail(KMC_ERR_INVALID, "logistic prior_sigma must be > 0");
             h->ndata = N;
-            e = dev_alloc(&h->d_X, sizeof(float) * N * d, device);
-            if (e == cudaSuccess) e = dev_alloc(&h->d_y, sizeof(float) * N, device);
-            if (e == cudaSuccess) e = cudaMemcpy(h->d_X, data, sizeof(float) * N * d, cudaMemcpyHostToDevice);
-            if (e == cudaSuccess)
-                e = cudaMemcpy(h->d_y, (const float *)data + N * d, sizeof(float) * N, cudaMemcpyHostToDevice);
+            CU_TRY(dev_alloc(&h->d_X, sizeof(float) * N * d, device));
+            CU_TRY(dev_alloc(&h->d_y, sizeof(float) * N, device));
+            CU_TRY(cudaMemcpy(h->d_X, data, sizeof(float) * N * d, cudaMemcpyHostToDevice));
+            CU_TRY(cudaMemcpy(h->d_y, (const float *)data + N * d, sizeof(float) * N, cudaMemcpyHostToDevice));
             // tcgen05 path: d <= 64 (zero-padded to K = 32 or 64) and every X value exactly representable in bf16
-            if (e == cudaSuccess && d <= 64) {
+            if (d <= 64) {
                 h->kp = d <= 32 ? 32 : 64;
                 const uint32_t *xb = reinterpret_cast<const uint32_t *>(data);
                 bool exact = true;
@@ -682,24 +687,17 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
                         const double yc = (double)yh[n] - 0.5;
                         for (int c = 0; c < d; ++c) xty[c] += yc * (double)Xh[n * d + c];
                     }
-                    e = dev_alloc(&h->d_Xbf, sizeof(__nv_bfloat16) * N * h->kp, device);
-                    if (e == cudaSuccess) e = dev_alloc(&h->d_xty, sizeof(double) * d, device);
-                    if (e == cudaSuccess) e = cudaMemcpy(h->d_xty, xty.data(), sizeof(double) * d, cudaMemcpyHostToDevice);
-                    if (e == cudaSuccess) {
-                        kmc::tc::f32_to_bf16_kernel<<<(unsigned)((N * h->kp + 255) / 256), 256>>>(h->d_X, h->d_Xbf, N, d, h->kp);
-                        e = cudaDeviceSynchronize();
-                    }
-                    if (e == cudaSuccess)
-                        h->tc_ok = make_map_bf16_k(&h->mapX, h->d_Xbf, (unsigned long long)N, kmc::tc::BN, h->kp);
+                    CU_TRY(dev_alloc(&h->d_Xbf, sizeof(__nv_bfloat16) * N * h->kp, device));
+                    CU_TRY(dev_alloc(&h->d_xty, sizeof(double) * d, device));
+                    CU_TRY(cudaMemcpy(h->d_xty, xty.data(), sizeof(double) * d, cudaMemcpyHostToDevice));
+                    kmc::tc::f32_to_bf16_kernel<<<(unsigned)((N * h->kp + 255) / 256), 256>>>(h->d_X, h->d_Xbf, N, d, h->kp);
+                    CU_TRY(cudaDeviceSynchronize());
+                    h->tc_ok = make_map_bf16_k(&h->mapX, h->d_Xbf, (unsigned long long)N, kmc::tc::BN, h->kp);
                 }
             }
         }
-        if (e != cudaSuccess) {
-            kmc_density_destroy(h);
-            return fail(KMC_ERR_CUDA, "density upload failed: %s", cudaGetErrorString(e));
-        }
     }
-    *out = h;
+    *out = h.release();
     return KMC_OK;
 }
 
@@ -758,19 +756,14 @@ int32_t kmc_density_eval(kmc_density_t h, const double *thetas, int64_t nw, doub
     if (!h || !thetas || !logp_out || nw < 0) return fail(KMC_ERR_INVALID, "bad argument");
     if (nw == 0) return KMC_OK;
     CU_TRY(cudaSetDevice(h->device));
-    double *dx = nullptr, *dl = nullptr;
-    CU_TRY(dev_alloc(&dx, sizeof(double) * nw * h->d, h->device));
-    cudaError_t e = dev_alloc(&dl, sizeof(double) * nw, h->device);
-    if (e == cudaSuccess) e = cudaMemcpy(dx, thetas, sizeof(double) * nw * h->d, cudaMemcpyHostToDevice);
+    DevBuf<double> dx, dl;
     BatchScratch sc;
-    if (e == cudaSuccess) e = eval_on_device(*h, dx, nw, dl, sc, nullptr);
-    if (e == cudaSuccess) e = cudaMemcpy(logp_out, dl, sizeof(double) * nw, cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();
-    dev_free(dx);
-    dev_free(dl);
-    dev_free(sc.part);
-    dev_free(sc.pieces);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "density eval failed: %s", cudaGetErrorString(e));
+    CU_TRY(dev_alloc(dx, sizeof(double) * nw * h->d, h->device));
+    CU_TRY(dev_alloc(dl, sizeof(double) * nw, h->device));
+    CU_TRY(cudaMemcpy(dx.get(), thetas, sizeof(double) * nw * h->d, cudaMemcpyHostToDevice));
+    CU_TRY(eval_on_device(*h, dx.get(), nw, dl.get(), sc, nullptr));
+    CU_TRY(cudaMemcpy(logp_out, dl.get(), sizeof(double) * nw, cudaMemcpyDeviceToHost));
+    CU_TRY(cudaDeviceSynchronize());
     return KMC_OK;
 }
 
@@ -802,8 +795,6 @@ int32_t kmc_emcee_destroy(kmc_sampler_t s) {
     dev_free(s->bb.u);
     dev_free(s->bb.p1);
     dev_free(s->bb.j);
-    dev_free(s->bsc.part);
-    dev_free(s->bsc.pieces);
     if (s->ev0) cudaEventDestroy(s->ev0);
     if (s->ev1) cudaEventDestroy(s->ev1);
     if (s->own_stream) cudaStreamDestroy(s->own_stream);
@@ -1231,43 +1222,9 @@ int32_t kmc_emcee_copy_results(kmc_sampler_t s, double *thetas, double *logp, do
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
     CU_TRY(cudaSetDevice(s->opts.device));
     CU_TRY(cudaStreamSynchronize(s->stream));
-    const long long ns = s->ns, nl = s->nl;
-    const int d = s->d;
-    if (ns > 0 && (thetas || logp)) {
-        // walkers per staging chunk: <= 64 MiB of [wc][ns][d] doubles
-        long long wc = std::max<long long>(32, (64LL << 20) / (sizeof(double) * ns * d));
-        wc = std::min(wc, nl);
-        double *stage = nullptr;
-        CU_TRY(dev_alloc(&stage, sizeof(double) * wc * ns * d, s->opts.device));
-        cudaError_t e = cudaSuccess;
-        for (long long w0 = 0; w0 < nl && e == cudaSuccess; w0 += wc) {
-            const long long cur = std::min(wc, nl - w0);
-            const dim3 blk(32, 8);
-            if (thetas) {
-                for (long long s0 = 0; s0 < ns; s0 += kmc::kTransposeMaxSamples) {
-                    const long long sc = std::min(kmc::kTransposeMaxSamples, ns - s0);
-                    const dim3 grd((unsigned)((cur + 31) / 32), (unsigned)((sc + 31) / 32), (unsigned)d);
-                    kmc::chain_transpose_kernel<<<grd, blk, 0, s->stream>>>(s->chain_x, stage, ns, nl, w0, cur, d, s0);
-                }
-                e = cudaMemcpyAsync(thetas + w0 * ns * d, stage, sizeof(double) * cur * ns * d,
-                                    cudaMemcpyDeviceToHost, s->stream);
-                if (e != cudaSuccess) break;
-            }
-            if (logp) {
-                for (long long s0 = 0; s0 < ns; s0 += kmc::kTransposeMaxSamples) {
-                    const long long sc = std::min(kmc::kTransposeMaxSamples, ns - s0);
-                    const dim3 grd((unsigned)((cur + 31) / 32), (unsigned)((sc + 31) / 32), 1);
-                    kmc::chain_transpose_kernel<<<grd, blk, 0, s->stream>>>(s->chain_lp, stage, ns, nl, w0, cur, 1, s0);
-                }
-                e = cudaMemcpyAsync(logp + w0 * ns, stage, sizeof(double) * cur * ns, cudaMemcpyDeviceToHost,
-                                    s->stream);
-            }
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
-        if (e == cudaSuccess) e = cudaGetLastError();
-        dev_free(stage);
-        if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "copy_results failed: %s", cudaGetErrorString(e));
-    }
+    const long long nl = s->nl;
+    if (s->ns > 0 && (thetas || logp))
+        if (const int32_t rc = chain_gather(s, nullptr, nl, thetas, logp); rc != KMC_OK) return rc;
     if (accept_ratio) {  // this sampler's walkers: its slice of half 0, then of half 1 (Metropolis: every chain)
         std::vector<unsigned> h(nl);
         if (s->metro) {
@@ -1290,19 +1247,15 @@ int32_t kmc_emcee_chain_moments(kmc_sampler_t s, double *mean, double *var, int6
     if (count) *count = nrows;
     if (nrows < 1) return fail(KMC_ERR_STATE, "no samples stored");
     CU_TRY(cudaSetDevice(s->opts.device));
-    double *sums = nullptr;
-    CU_TRY(dev_alloc(&sums, sizeof(double) * 2 * d, s->opts.device));
+    DevBuf<double> sums;
+    CU_TRY(dev_alloc(sums, sizeof(double) * 2 * d, s->opts.device));
     std::vector<double> h(2 * d), shift(d);
-    cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * 2 * d, s->stream);
-    if (e == cudaSuccess) {
-        const unsigned grid = (unsigned)std::min<long long>((nrows * d + 255) / 256, 148 * 8);
-        kmc::chain_moments_kernel<<<grid, 256, sizeof(double) * 2 * d, s->stream>>>(s->chain_x, nrows, d, sums);
-        e = cudaMemcpyAsync(h.data(), sums, sizeof(double) * 2 * d, cudaMemcpyDeviceToHost, s->stream);
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
-    dev_free(sums);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "chain moments failed: %s", cudaGetErrorString(e));
+    CU_TRY(cudaMemsetAsync(sums.get(), 0, sizeof(double) * 2 * d, s->stream));
+    const unsigned grid = (unsigned)std::min<long long>((nrows * d + 255) / 256, 148 * 8);
+    kmc::chain_moments_kernel<<<grid, 256, sizeof(double) * 2 * d, s->stream>>>(s->chain_x, nrows, d, sums.get());
+    CU_TRY(cudaMemcpyAsync(h.data(), sums.get(), sizeof(double) * 2 * d, cudaMemcpyDeviceToHost, s->stream));
+    CU_TRY(cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream));
+    CU_TRY(cudaStreamSynchronize(s->stream));
     const double n = (double)nrows;
     for (int c = 0; c < d; ++c) {
         if (mean) mean[c] = shift[c] + h[c] / n;

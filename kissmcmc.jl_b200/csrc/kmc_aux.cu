@@ -43,17 +43,12 @@ int32_t kmc_emcee_create_multi(const kmc_density_t *densities, const double *the
         if (!densities[r]) return fail(KMC_ERR_INVALID, "densities[%d] is NULL", r);
     if (mode == KMC_MULTI_SHARDED && (nwalkers < 2 || (nwalkers & 1) || (nwalkers / 2) % ndev))
         return fail(KMC_ERR_INVALID, "nwalkers/2 must be a multiple of the number of devices");
-    auto *m = new kmc_multi_s;
+    // the handle under construction, deleted by kmc_multi_destroy (which sets no error) on every exit but the last
+    std::unique_ptr<kmc_multi_s, int32_t (*)(kmc_multi_t)> m(new kmc_multi_s, kmc_multi_destroy);
     m->mode = mode;
     m->nw = nwalkers;
     m->d = d;
     m->subs.assign(ndev, nullptr);
-    auto bail = [&](int32_t rc) {
-        const std::string keep = last_error();
-        kmc_multi_destroy(m);
-        set_last_error(keep);
-        return rc;
-    };
     const long long S = nwalkers / 2 / ndev;
     for (int r = 0; r < ndev; ++r) {
         kmc_emcee_opts o = *opts;
@@ -70,7 +65,7 @@ int32_t kmc_emcee_create_multi(const kmc_density_t *densities, const double *the
         }
         const double *th = mode == KMC_MULTI_SHARDED ? theta0s : theta0s + (size_t)r * nwalkers * d;
         const int32_t rc = kmc_emcee_create(densities[r], th, nwalkers, d, &o, &m->subs[r]);
-        if (rc != KMC_OK) return bail(rc);
+        if (rc != KMC_OK) return rc;
     }
     if (mode == KMC_MULTI_SHARDED) {
         for (int a = 0; a < ndev; ++a) {
@@ -80,16 +75,16 @@ int32_t kmc_emcee_create_multi(const kmc_density_t *densities, const double *the
             sa->share = share;  // sub-samplers of one GPU must all be co-resident: split the CTA slots
             sa->grid = std::max(1u, sa->grid / (unsigned)share);
             sa->lag = push_default_lag(sa->nchunks, opts->push_lag);
-            if (cudaSetDevice(devices[a]) != cudaSuccess) return bail(fail(KMC_ERR_CUDA, "cudaSetDevice(%d) failed", devices[a]));
+            CU_TRY(cudaSetDevice(devices[a]));
             for (int b = 0; b < ndev; ++b) {
                 if (devices[b] != devices[a]) {
                     int can = 0;
                     cudaDeviceCanAccessPeer(&can, devices[a], devices[b]);
-                    if (!can) return bail(fail(KMC_ERR_CUDA, "device %d cannot access device %d's memory", devices[a], devices[b]));
+                    if (!can) return fail(KMC_ERR_CUDA, "device %d cannot access device %d's memory", devices[a], devices[b]);
                     const cudaError_t e = cudaDeviceEnablePeerAccess(devices[b], 0);
                     if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled)
-                        return bail(fail(KMC_ERR_CUDA, "cudaDeviceEnablePeerAccess(%d -> %d) failed: %s", devices[a], devices[b],
-                                         cudaGetErrorString(e)));
+                        return fail(KMC_ERR_CUDA, "cudaDeviceEnablePeerAccess(%d -> %d) failed: %s", devices[a], devices[b],
+                                    cudaGetErrorString(e));
                     cudaGetLastError();
                 }
                 push_set_peer(sa, b, m->subs[b]->window);
@@ -97,7 +92,7 @@ int32_t kmc_emcee_create_multi(const kmc_density_t *densities, const double *the
             sa->attached = true;
         }
     }
-    *out = m;
+    *out = m.release();
     return KMC_OK;
 }
 
@@ -219,13 +214,11 @@ int32_t kmc_sample_g(double a_scale, uint64_t seed, int64_t n, int32_t device, d
     if (!(a_scale > 1.0)) return fail(KMC_ERR_INVALID, "a_scale must be > 1");
     if (n == 0) return KMC_OK;
     CU_TRY(cudaSetDevice(device));
-    double *dz = nullptr;
-    CU_TRY(dev_alloc(&dz, sizeof(double) * n, device));
+    DevBuf<double> dz;
+    CU_TRY(dev_alloc(dz, sizeof(double) * n, device));
     const double sia = std::sqrt(1.0 / a_scale), span = std::sqrt(a_scale) - sia;
-    sample_g_kernel<<<(unsigned)((n + 255) / 256), 256>>>(kmc::philox_keys(seed), sia, span, n, dz);
-    cudaError_t e = cudaMemcpy(out, dz, sizeof(double) * n, cudaMemcpyDeviceToHost);
-    dev_free(dz);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "sample_g failed: %s", cudaGetErrorString(e));
+    sample_g_kernel<<<(unsigned)((n + 255) / 256), 256>>>(kmc::philox_keys(seed), sia, span, n, dz.get());
+    CU_TRY(cudaMemcpy(out, dz.get(), sizeof(double) * n, cudaMemcpyDeviceToHost));
     return KMC_OK;
 }
 
@@ -236,11 +229,17 @@ int32_t kmc_sample_g(double a_scale, uint64_t seed, int64_t n, int32_t device, d
 // concatenation (:398-399) and the time ordering (:415-426) without copying the per-walker chains to the host first.
 namespace {
 
+// counter i of this sampler's walkers: its slice of half 0 (the first na), then of half 1
+__device__ __forceinline__ unsigned counter_at(const unsigned *__restrict__ a, const unsigned *__restrict__ b, long long na,
+                                               long long i) {
+    return i < na ? a[i] : b[i - na];
+}
+
 // histogram of (v >> shift) & 0xFFFF over the counters whose upper bits (v >> (shift + 16)) equal `prefix`
 __global__ void nacc_hist_kernel(const unsigned *__restrict__ a, const unsigned *__restrict__ b, long long na, long long n,
                                  int shift, unsigned prefix, unsigned *__restrict__ hist) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const unsigned v = i < na ? a[i] : b[i - na];
+        const unsigned v = counter_at(a, b, na, i);
         if (shift == 16 || (v >> 16) == prefix) atomicAdd(hist + ((v >> shift) & 0xFFFFu), 1u);
     }
 }
@@ -250,7 +249,7 @@ __global__ void nacc_sums_kernel(const unsigned *__restrict__ a, const unsigned 
                                  unsigned long long *__restrict__ out /* sum, sq_lo, sq_hi */) {
     unsigned long long s = 0, lo = 0, hi = 0;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
-        const unsigned long long v = i < na ? a[i] : b[i - na];
+        const unsigned long long v = counter_at(a, b, na, i);
         s += v;
         const unsigned long long sq = v * v, nl = lo + sq;
         hi += nl < lo ? 1ull : 0ull;
@@ -262,70 +261,69 @@ __global__ void nacc_sums_kernel(const unsigned *__restrict__ a, const unsigned 
     if (hi) atomicAdd(out + 2, hi);
 }
 
-constexpr int kKeepBlock = 1024;  // walkers per block of the keep scan
+// ---- ordered compaction: the kept threads' items in thread order, by blocks of kKeepBlock threads.  Each block
+// counts its kept threads (compact_count), the host scans the counts into block offsets (compact_offsets), and a
+// second launch of the same grid writes each kept item to its slot (compact_slot).
+constexpr int kKeepBlock = 1024;
 
-// keep[w] = accept_ratio[w] > thr (:384-391: dropped iff ratio <= median - drop_fact*std); per-block kept counts and the
-// exact sum of the kept counters
-__global__ void __launch_bounds__(kKeepBlock) keep_count_kernel(const unsigned *__restrict__ a, const unsigned *__restrict__ b,
-                                                                long long na, long long n, double den, double thr, int drop,
-                                                                unsigned *__restrict__ blk_cnt, unsigned long long *__restrict__ kept_sum) {
-    __shared__ unsigned wc[kKeepBlock / 32];
-    const long long w = (long long)blockIdx.x * kKeepBlock + threadIdx.x;
-    bool keep = false;
-    unsigned v = 0;
-    if (w < n) {
-        v = w < na ? a[w] : b[w - na];
-        keep = !drop || !((double)v / den <= thr);
-    }
-    const unsigned bl = __ballot_sync(0xffffffffu, keep);
-    unsigned long long sv = keep ? v : 0u;
-    for (int o = 16; o > 0; o >>= 1) sv += __shfl_xor_sync(0xffffffffu, sv, o);
-    if ((threadIdx.x & 31) == 0) {
-        wc[threadIdx.x >> 5] = __popc(bl);
-        if (sv) atomicAdd(kept_sum, sv);
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        unsigned t = 0;
-        for (int k = 0; k < kKeepBlock / 32; ++k) t += wc[k];
-        blk_cnt[blockIdx.x] = t;
-    }
+__device__ __forceinline__ void compact_count(bool keep, unsigned *__restrict__ blk_cnt) {
+    const int c = __syncthreads_count(keep);
+    if (threadIdx.x == 0) blk_cnt[blockIdx.x] = (unsigned)c;
 }
 
-// kept walker indices in walker order: idx[blk_off[block] + rank inside the block] = w
-__global__ void __launch_bounds__(kKeepBlock) keep_index_kernel(const unsigned *__restrict__ a, const unsigned *__restrict__ b,
-                                                                long long na, long long n, double den, double thr, int drop,
-                                                                const unsigned *__restrict__ blk_off, unsigned *__restrict__ idx) {
+// the slot of a kept thread: its block's offset, the kept threads of the lower warps and the kept lanes below it
+__device__ __forceinline__ unsigned compact_slot(bool keep, const unsigned *__restrict__ blk_off) {
     __shared__ unsigned wc[kKeepBlock / 32];
-    const long long w = (long long)blockIdx.x * kKeepBlock + threadIdx.x;
-    bool keep = false;
-    if (w < n) {
-        const unsigned v = w < na ? a[w] : b[w - na];
-        keep = !drop || !((double)v / den <= thr);
-    }
     const unsigned bl = __ballot_sync(0xffffffffu, keep), lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
     if (lane == 0) wc[wp] = __popc(bl);
     __syncthreads();
     unsigned off = blk_off[blockIdx.x];
     for (unsigned k = 0; k < wp; ++k) off += wc[k];
-    if (keep) idx[off + __popc(bl & ((1u << lane) - 1u))] = (unsigned)w;
+    return off + __popc(bl & ((1u << lane) - 1u));
 }
 
-// walker-major gather of kept walkers [k0, k0+kc): out[(k*ns + s)*d + c] = in[(s*nl + idx[k0+k])*d + c]  (:398-399)
-__global__ void squash_walker_major_kernel(const double *__restrict__ in, double *__restrict__ out, long long ns, long long nl,
-                                           const unsigned *__restrict__ idx, long long k0, long long kc, int d, long long s0) {
-    __shared__ double tile[32][33];
-    const int c = blockIdx.z;
-    const long long kb = (long long)blockIdx.x * 32, sb = s0 + (long long)blockIdx.y * 32;
-    for (int r = threadIdx.y; r < 32; r += blockDim.y) {
-        const long long s = sb + r, k = kb + threadIdx.x;
-        if (s < ns && k < kc) tile[r][threadIdx.x] = in[(s * nl + idx[k0 + k]) * d + c];
+// d_blk[0, nblk) holds the blocks' counts: their exclusive scan goes to d_blk[nblk, 2 nblk), their sum to `total`
+int32_t compact_offsets(unsigned *d_blk, long long nblk, cudaStream_t st, long long &total) {
+    std::vector<unsigned> blk(2 * nblk);
+    CU_TRY(cudaMemcpyAsync(blk.data(), d_blk, sizeof(unsigned) * nblk, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    total = 0;
+    for (long long b = 0; b < nblk; ++b) {
+        blk[nblk + b] = (unsigned)total;
+        total += blk[b];
     }
-    __syncthreads();
-    for (int r = threadIdx.y; r < 32; r += blockDim.y) {
-        const long long k = kb + r, s = sb + threadIdx.x;
-        if (s < ns && k < kc) out[(k * ns + s) * d + c] = tile[threadIdx.x][r];
-    }
+    CU_TRY(cudaMemcpyAsync(d_blk + nblk, blk.data() + nblk, sizeof(unsigned) * nblk, cudaMemcpyHostToDevice, st));
+    return KMC_OK;
+}
+
+// walker w is kept unless drop is on and its accept ratio is <= thr (:384-391); v = its counter (0 past the end)
+__device__ __forceinline__ bool walker_kept(const unsigned *__restrict__ a, const unsigned *__restrict__ b, long long na,
+                                            long long n, long long w, double den, double thr, int drop, unsigned &v) {
+    v = w < n ? counter_at(a, b, na, w) : 0u;
+    return w < n && (!drop || !((double)v / den <= thr));
+}
+
+// per-block kept counts and the exact sum of the kept counters
+__global__ void __launch_bounds__(kKeepBlock) keep_count_kernel(const unsigned *__restrict__ a, const unsigned *__restrict__ b,
+                                                                long long na, long long n, double den, double thr, int drop,
+                                                                unsigned *__restrict__ blk_cnt, unsigned long long *__restrict__ kept_sum) {
+    unsigned v;
+    const bool keep = walker_kept(a, b, na, n, (long long)blockIdx.x * kKeepBlock + threadIdx.x, den, thr, drop, v);
+    unsigned long long sv = keep ? v : 0u;
+    for (int o = 16; o > 0; o >>= 1) sv += __shfl_xor_sync(0xffffffffu, sv, o);
+    if ((threadIdx.x & 31) == 0 && sv) atomicAdd(kept_sum, sv);
+    compact_count(keep, blk_cnt);
+}
+
+// kept walker indices in walker order
+__global__ void __launch_bounds__(kKeepBlock) keep_index_kernel(const unsigned *__restrict__ a, const unsigned *__restrict__ b,
+                                                                long long na, long long n, double den, double thr, int drop,
+                                                                const unsigned *__restrict__ blk_off, unsigned *__restrict__ idx) {
+    const long long w = (long long)blockIdx.x * kKeepBlock + threadIdx.x;
+    unsigned v;
+    const bool keep = walker_kept(a, b, na, n, w, den, thr, drop, v);
+    const unsigned slot = compact_slot(keep, blk_off);
+    if (keep) idx[slot] = (unsigned)w;
 }
 
 // time-major gather (order=true, :415-426: the stable sortperm of (1:ns, 1:ns, ...) = sample-major, walkers in kept
@@ -351,7 +349,8 @@ cudaError_t select_kth(const unsigned *a, const unsigned *b, long long na, long 
         if (e != cudaSuccess) return e;
         nacc_hist_kernel<<<grid, 256, 0, st>>>(a, b, na, n, pass == 0 ? 16 : 0, prefix, d_hist);
         e = cudaMemcpyAsync(h_hist.data(), d_hist, sizeof(unsigned) * 65536, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return e;
+        e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) return e;
         long long acc = 0;
         unsigned bin = 0;
@@ -383,43 +382,29 @@ int32_t kmc_emcee_squash(kmc_sampler_t s, int32_t drop_low_accept_ratio, double 
     const double den = (double)(s->opts.niter_walker - s->opts.nburnin_walker);  // :291
     const long long nblk = (nl + kKeepBlock - 1) / kKeepBlock;
 
-    unsigned *d_hist = nullptr, *d_blk = nullptr, *d_idx = nullptr;
-    unsigned long long *d_sums = nullptr;
-    double *stage = nullptr;
-    auto cleanup = [&]() {
-        dev_free(d_hist);
-        dev_free(d_blk);
-        dev_free(d_idx);
-        dev_free(d_sums);
-        dev_free(stage);
-    };
-#define CU_TRY_Q(expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t e_ = (expr);                                                                         \
-        if (e_ != cudaSuccess) {                                                                         \
-            cleanup();                                                                                   \
-            return fail(KMC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-        }                                                                                                \
-    } while (0)
-    CU_TRY_Q(dev_alloc(&d_hist, sizeof(unsigned) * 65536, s->opts.device));
-    CU_TRY_Q(dev_alloc(&d_blk, sizeof(unsigned) * 2 * nblk, s->opts.device));
-    CU_TRY_Q(dev_alloc(&d_idx, sizeof(unsigned) * nl, s->opts.device));
-    CU_TRY_Q(dev_alloc(&d_sums, sizeof(unsigned long long) * 4, s->opts.device));
+    DevBuf<unsigned> d_hist, d_blk, d_idx;
+    DevBuf<unsigned long long> d_sums;
+    DevBuf<double> stage;
+    CU_TRY(dev_alloc(d_hist, sizeof(unsigned) * 65536, s->opts.device));
+    CU_TRY(dev_alloc(d_blk, sizeof(unsigned) * 2 * nblk, s->opts.device));
+    CU_TRY(dev_alloc(d_idx, sizeof(unsigned) * nl, s->opts.device));
+    CU_TRY(dev_alloc(d_sums, sizeof(unsigned long long) * 4, s->opts.device));
 
     // ---- :385  median and std (n-1) of the accept ratios, from exact integer statistics of the counters
     double med = 0.0, sd = 0.0, thr = 0.0;
     {
         std::vector<unsigned> h_hist(65536);
         unsigned c1 = 0, c2 = 0;
-        CU_TRY_Q(select_kth(na, nb, S, nl, (nl - 1) / 2, d_hist, h_hist, st, &c1));
-        CU_TRY_Q(select_kth(na, nb, S, nl, nl / 2, d_hist, h_hist, st, &c2));
+        CU_TRY(select_kth(na, nb, S, nl, (nl - 1) / 2, d_hist.get(), h_hist, st, &c1));
+        CU_TRY(select_kth(na, nb, S, nl, nl / 2, d_hist.get(), h_hist, st, &c2));
         med = ((double)c1 / den + (double)c2 / den) / 2.0;  // median of an even count = mean of the two middle values
         if (c1 == c2) med = (double)c1 / den;
         unsigned long long hs[3] = {0, 0, 0};
-        CU_TRY_Q(cudaMemsetAsync(d_sums, 0, sizeof(unsigned long long) * 4, st));
-        nacc_sums_kernel<<<(unsigned)std::min<long long>((nl + 255) / 256, 1184), 256, 0, st>>>(na, nb, S, nl, d_sums);
-        CU_TRY_Q(cudaMemcpyAsync(hs, d_sums, sizeof hs, cudaMemcpyDeviceToHost, st));
-        CU_TRY_Q(cudaStreamSynchronize(st));
+        CU_TRY(cudaMemsetAsync(d_sums.get(), 0, sizeof(unsigned long long) * 4, st));
+        nacc_sums_kernel<<<(unsigned)std::min<long long>((nl + 255) / 256, 1184), 256, 0, st>>>(na, nb, S, nl,
+                                                                                                d_sums.get());
+        CU_TRY(cudaMemcpyAsync(hs, d_sums.get(), sizeof hs, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
         const unsigned __int128 sum = hs[0], sq = ((unsigned __int128)hs[2] << 64) | hs[1];
         const unsigned __int128 num = (unsigned __int128)nl * sq - sum * sum;  // n * sum(c^2) - (sum c)^2 >= 0, exact
         const long double var = nl > 1 ? (long double)num / ((long double)nl * (long double)(nl - 1)) : 0.0L;
@@ -431,69 +416,39 @@ int32_t kmc_emcee_squash(kmc_sampler_t s, int32_t drop_low_accept_ratio, double 
 
     // ---- :380-396  walkers to keep, in walker order
     const int drop = drop_low_accept_ratio ? 1 : 0;
-    CU_TRY_Q(cudaMemsetAsync(d_sums, 0, sizeof(unsigned long long) * 4, st));
-    keep_count_kernel<<<(unsigned)nblk, kKeepBlock, 0, st>>>(na, nb, S, nl, den, thr, drop, d_blk, d_sums);
-    std::vector<unsigned> blk(2 * nblk);
+    CU_TRY(cudaMemsetAsync(d_sums.get(), 0, sizeof(unsigned long long) * 4, st));
+    keep_count_kernel<<<(unsigned)nblk, kKeepBlock, 0, st>>>(na, nb, S, nl, den, thr, drop, d_blk.get(), d_sums.get());
     unsigned long long kept_sum = 0;
-    CU_TRY_Q(cudaMemcpyAsync(blk.data(), d_blk, sizeof(unsigned) * nblk, cudaMemcpyDeviceToHost, st));
-    CU_TRY_Q(cudaMemcpyAsync(&kept_sum, d_sums, sizeof kept_sum, cudaMemcpyDeviceToHost, st));
-    CU_TRY_Q(cudaStreamSynchronize(st));
+    CU_TRY(cudaMemcpyAsync(&kept_sum, d_sums.get(), sizeof kept_sum, cudaMemcpyDeviceToHost, st));
     long long nk = 0;
-    for (long long bi = 0; bi < nblk; ++bi) {
-        blk[nblk + bi] = (unsigned)nk;
-        nk += blk[bi];
-    }
-    CU_TRY_Q(cudaMemcpyAsync(d_blk + nblk, blk.data() + nblk, sizeof(unsigned) * nblk, cudaMemcpyHostToDevice, st));
-    keep_index_kernel<<<(unsigned)nblk, kKeepBlock, 0, st>>>(na, nb, S, nl, den, thr, drop, d_blk + nblk, d_idx);
+    if (const int32_t rc = compact_offsets(d_blk.get(), nblk, st, nk); rc != KMC_OK) return rc;
+    keep_index_kernel<<<(unsigned)nblk, kKeepBlock, 0, st>>>(na, nb, S, nl, den, thr, drop, d_blk.get() + nblk,
+                                                             d_idx.get());
     if (nkept) *nkept = nk;
     if (accept_mean) *accept_mean = nk > 0 ? (double)kept_sum / den / (double)nk : 0.0;  // :427 mean(accept_ratio[keep])
 
     // ---- :398-399 / :415-426  the kept chains, walker-major or time-major, staged through <= 64 MiB
     if (ns > 0 && nk > 0 && (thetas || logp)) {
-        const long long row_bytes = (long long)sizeof(double) * d;
-        if (!order) {
-            long long kc = std::max<long long>(32, (64LL << 20) / (row_bytes * ns));
-            kc = std::min(kc, nk);
-            CU_TRY_Q(dev_alloc(&stage, sizeof(double) * kc * ns * d, s->opts.device));
-            const dim3 blkdim(32, 8);
-            for (long long k0 = 0; k0 < nk; k0 += kc) {
-                const long long cur = std::min(kc, nk - k0);
-                for (int what = 0; what < 2; ++what) {
-                    double *host = what == 0 ? thetas : logp;
-                    if (!host) continue;
-                    const int dd = what == 0 ? d : 1;
-                    const double *src = what == 0 ? s->chain_x : s->chain_lp;
-                    for (long long s0 = 0; s0 < ns; s0 += kmc::kTransposeMaxSamples) {
-                        const long long sc = std::min(kmc::kTransposeMaxSamples, ns - s0);
-                        const dim3 grd((unsigned)((cur + 31) / 32), (unsigned)((sc + 31) / 32), (unsigned)dd);
-                        squash_walker_major_kernel<<<grd, blkdim, 0, st>>>(src, stage, ns, nl, d_idx, k0, cur, dd, s0);
-                    }
-                    CU_TRY_Q(cudaMemcpyAsync(host + k0 * ns * dd, stage, sizeof(double) * cur * ns * dd, cudaMemcpyDeviceToHost, st));
-                    CU_TRY_Q(cudaStreamSynchronize(st));
-                }
-            }
-        } else {
-            long long sc = std::max<long long>(1, (64LL << 20) / (row_bytes * nk));
-            sc = std::min(sc, ns);
-            CU_TRY_Q(dev_alloc(&stage, sizeof(double) * sc * nk * d, s->opts.device));
-            for (long long s0 = 0; s0 < ns; s0 += sc) {
-                const long long cur = std::min(sc, ns - s0);
-                for (int what = 0; what < 2; ++what) {
-                    double *host = what == 0 ? thetas : logp;
-                    if (!host) continue;
-                    const int dd = what == 0 ? d : 1;
-                    const double *src = what == 0 ? s->chain_x : s->chain_lp;
-                    const unsigned grid = (unsigned)std::min<long long>((cur * nk * dd + 255) / 256, 148 * 16);
-                    squash_time_major_kernel<<<grid, 256, 0, st>>>(src, stage, nl, nk, d_idx, s0, cur, dd);
-                    CU_TRY_Q(cudaMemcpyAsync(host + s0 * nk * dd, stage, sizeof(double) * cur * nk * dd, cudaMemcpyDeviceToHost, st));
-                    CU_TRY_Q(cudaStreamSynchronize(st));
-                }
+        if (!order) return chain_gather(s, d_idx.get(), nk, thetas, logp);
+        long long sc = std::max<long long>(1, (64LL << 20) / ((long long)sizeof(double) * d * nk));
+        sc = std::min(sc, ns);
+        CU_TRY(dev_alloc(stage, sizeof(double) * sc * nk * d, s->opts.device));
+        for (long long s0 = 0; s0 < ns; s0 += sc) {
+            const long long cur = std::min(sc, ns - s0);
+            for (int what = 0; what < 2; ++what) {
+                double *host = what == 0 ? thetas : logp;
+                if (!host) continue;
+                const int dd = what == 0 ? d : 1;
+                const double *src = what == 0 ? s->chain_x : s->chain_lp;
+                const unsigned grid = (unsigned)std::min<long long>((cur * nk * dd + 255) / 256, 148 * 16);
+                squash_time_major_kernel<<<grid, 256, 0, st>>>(src, stage.get(), nl, nk, d_idx.get(), s0, cur, dd);
+                CU_TRY(cudaMemcpyAsync(host + s0 * nk * dd, stage.get(), sizeof(double) * cur * nk * dd,
+                                       cudaMemcpyDeviceToHost, st));
             }
         }
     }
-    CU_TRY_Q(cudaGetLastError());
-#undef CU_TRY_Q
-    cleanup();
+    CU_TRY(cudaStreamSynchronize(st));  // the blocks go back to the cache idle (the sizing call ends with keep_index)
+    CU_TRY(cudaGetLastError());
     return KMC_OK;
 }
 
@@ -579,28 +534,20 @@ __global__ void found_clear_kernel(unsigned char *__restrict__ found, long long 
     if (i < n) found[i] = 0;
 }
 
-// per-block counts / ordered indices of the found walkers (same two-level scan as the squash keep list)
+// per-block counts / ordered rows of the found walkers (the ordered compaction of the squash keep list)
 __global__ void __launch_bounds__(kKeepBlock) found_count_kernel(const unsigned char *__restrict__ found, long long n,
                                                                  unsigned *__restrict__ blk_cnt) {
     const long long w = (long long)blockIdx.x * kKeepBlock + threadIdx.x;
-    const int c = __syncthreads_count(w < n && found[w]);
-    if (threadIdx.x == 0) blk_cnt[blockIdx.x] = (unsigned)c;
+    compact_count(w < n && found[w], blk_cnt);
 }
 __global__ void __launch_bounds__(kKeepBlock) found_gather_kernel(const unsigned char *__restrict__ found, long long n, int d,
                                                                   const unsigned *__restrict__ blk_off,
                                                                   const double *__restrict__ rows, double *__restrict__ out) {
-    __shared__ unsigned wc[kKeepBlock / 32];
     const long long w = (long long)blockIdx.x * kKeepBlock + threadIdx.x;
     const bool keep = w < n && found[w];
-    const unsigned bl = __ballot_sync(0xffffffffu, keep), lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-    if (lane == 0) wc[wp] = __popc(bl);
-    __syncthreads();
-    unsigned off = blk_off[blockIdx.x];
-    for (unsigned k = 0; k < wp; ++k) off += wc[k];
-    if (keep) {
-        const size_t o = (size_t)(off + __popc(bl & ((1u << lane) - 1u))) * d;
+    const size_t o = (size_t)compact_slot(keep, blk_off) * d;
+    if (keep)
         for (int c = 0; c < d; ++c) out[o + c] = rows[(size_t)w * d + c];
-    }
 }
 
 }  // namespace
@@ -613,13 +560,12 @@ int32_t kmc_ball_randn(uint64_t seed, int64_t walker0, int64_t nwalkers, int32_t
         return fail(KMC_ERR_INVALID, "bad argument");
     if (nwalkers == 0) return KMC_OK;
     CU_TRY(cudaSetDevice(device));
-    double *dz = nullptr;
-    CU_TRY(dev_alloc(&dz, sizeof(double) * nwalkers * d, device));
+    DevBuf<double> dz;
+    CU_TRY(dev_alloc(dz, sizeof(double) * nwalkers * d, device));
     const long long ne = nwalkers * ((d + 1) / 2);
-    ball_randn_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(kmc::philox_keys(seed), nullptr, walker0, nwalkers, k, j, d, dz);
-    cudaError_t e = cudaMemcpy(out, dz, sizeof(double) * nwalkers * d, cudaMemcpyDeviceToHost);
-    dev_free(dz);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "ball_randn failed: %s", cudaGetErrorString(e));
+    ball_randn_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(kmc::philox_keys(seed), nullptr, walker0, nwalkers, k, j, d,
+                                                             dz.get());
+    CU_TRY(cudaMemcpy(out, dz.get(), sizeof(double) * nwalkers * d, cudaMemcpyDeviceToHost));
     return KMC_OK;
 }
 
@@ -638,60 +584,48 @@ int32_t kmc_make_theta0s(kmc_density_t density, const double *theta0, const doub
     const kmc::PhiloxKeys ks = kmc::philox_keys(seed);
     std::vector<double> br(ball_radius, ball_radius + d);
 
-    double *d_th0 = nullptr, *d_br = nullptr, *d_cand = nullptr, *d_lp = nullptr, *d_rows = nullptr, *d_out = nullptr;
-    unsigned *d_pend[2] = {nullptr, nullptr}, *d_cnt = nullptr, *d_blk = nullptr;
-    unsigned char *d_found = nullptr;
+    DevBuf<double> d_th0, d_br, d_cand, d_lp, d_rows, d_out;
+    DevBuf<unsigned> d_pend[2], d_cnt, d_blk;
+    DevBuf<unsigned char> d_found;
     BatchScratch sc;
-    auto cleanup = [&]() {
-        for (void *q : {(void *)d_th0, (void *)d_br, (void *)d_cand, (void *)d_lp, (void *)d_rows, (void *)d_out,
-                        (void *)d_pend[0], (void *)d_pend[1], (void *)d_cnt, (void *)d_blk, (void *)d_found, (void *)sc.part,
-                        (void *)sc.pieces})
-            dev_free(q);
-    };
-#define CU_TRY_M(expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t e_ = (expr);                                                                         \
-        if (e_ != cudaSuccess) {                                                                         \
-            cleanup();                                                                                   \
-            return fail(KMC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, __LINE__); \
-        }                                                                                                \
-    } while (0)
     const long long nblk = (nw + kKeepBlock - 1) / kKeepBlock;
-    CU_TRY_M(dev_alloc(&d_th0, sizeof(double) * d, dev));
-    CU_TRY_M(dev_alloc(&d_br, sizeof(double) * d, dev));
-    CU_TRY_M(dev_alloc(&d_cand, sizeof(double) * nw * d, dev));
-    CU_TRY_M(dev_alloc(&d_lp, sizeof(double) * nw, dev));
-    CU_TRY_M(dev_alloc(&d_rows, sizeof(double) * nw * d, dev));
-    CU_TRY_M(dev_alloc(&d_pend[0], sizeof(unsigned) * nw, dev));
-    CU_TRY_M(dev_alloc(&d_pend[1], sizeof(unsigned) * nw, dev));
-    CU_TRY_M(dev_alloc(&d_cnt, sizeof(unsigned) * 2, dev));
-    CU_TRY_M(dev_alloc(&d_blk, sizeof(unsigned) * 2 * nblk, dev));
-    CU_TRY_M(dev_alloc(&d_found, (size_t)nw, dev));
-    CU_TRY_M(cudaMemcpy(d_th0, theta0, sizeof(double) * d, cudaMemcpyHostToDevice));
-    CU_TRY_M(cudaMemset(d_found, 0, (size_t)nw));
+    CU_TRY(dev_alloc(d_th0, sizeof(double) * d, dev));
+    CU_TRY(dev_alloc(d_br, sizeof(double) * d, dev));
+    CU_TRY(dev_alloc(d_cand, sizeof(double) * nw * d, dev));
+    CU_TRY(dev_alloc(d_lp, sizeof(double) * nw, dev));
+    CU_TRY(dev_alloc(d_rows, sizeof(double) * nw * d, dev));
+    CU_TRY(dev_alloc(d_pend[0], sizeof(unsigned) * nw, dev));
+    CU_TRY(dev_alloc(d_pend[1], sizeof(unsigned) * nw, dev));
+    CU_TRY(dev_alloc(d_cnt, sizeof(unsigned) * 2, dev));
+    CU_TRY(dev_alloc(d_blk, sizeof(unsigned) * 2 * nblk, dev));
+    CU_TRY(dev_alloc(d_found, (size_t)nw, dev));
+    CU_TRY(cudaMemcpy(d_th0.get(), theta0, sizeof(double) * d, cudaMemcpyHostToDevice));
+    CU_TRY(cudaMemset(d_found.get(), 0, (size_t)nw));
 
     // one batched try (k, j) of the walkers in d_pend[cur][0..np): candidates -> plugin -> accept / stay pending
     auto try_round = [&](int cur, long long np, int k, int j, unsigned *np_next) -> cudaError_t {
-        cudaError_t e = cudaMemset(d_cnt, 0, sizeof(unsigned));
+        cudaError_t e = cudaMemset(d_cnt.get(), 0, sizeof(unsigned));
         if (e != cudaSuccess) return e;
         const long long ne = np * ((d + 1) / 2);
-        ball_candidates_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(ks, d_pend[cur], np, k, j, d, d_th0, d_br, d_cand);
-        e = eval_on_device(*density, d_cand, np, d_lp, sc, nullptr);  // :334-336 through the plugin
+        ball_candidates_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(ks, d_pend[cur].get(), np, k, j, d, d_th0.get(),
+                                                                      d_br.get(), d_cand.get());
+        e = eval_on_device(*density, d_cand.get(), np, d_lp.get(), sc, nullptr);  // :334-336 through the plugin
         if (e != cudaSuccess) return e;
-        ball_accept_kernel<<<(unsigned)((np + 255) / 256), 256>>>(d_cand, d_lp, d_pend[cur], np, d, d_rows, d_found,
-                                                                  d_pend[cur ^ 1], d_cnt);
-        return cudaMemcpy(np_next, d_cnt, sizeof(unsigned), cudaMemcpyDeviceToHost);
+        ball_accept_kernel<<<(unsigned)((np + 255) / 256), 256>>>(d_cand.get(), d_lp.get(), d_pend[cur].get(), np, d,
+                                                                  d_rows.get(), d_found.get(), d_pend[cur ^ 1].get(),
+                                                                  d_cnt.get());
+        return cudaMemcpy(np_next, d_cnt.get(), sizeof(unsigned), cudaMemcpyDeviceToHost);
     };
 
     long long i0 = 0;
     while (i0 < nw) {  // :323 walkers i0.. with the CURRENT ball radius
-        CU_TRY_M(cudaMemcpy(d_br, br.data(), sizeof(double) * d, cudaMemcpyHostToDevice));
+        CU_TRY(cudaMemcpy(d_br.get(), br.data(), sizeof(double) * d, cudaMemcpyHostToDevice));
         long long np = nw - i0;
         int cur = 0;
-        iota_kernel<<<(unsigned)((np + 255) / 256), 256>>>(d_pend[0], np, (unsigned)i0);
+        iota_kernel<<<(unsigned)((np + 255) / 256), 256>>>(d_pend[0].get(), np, (unsigned)i0);
         for (int j = 1; j <= ntries && np > 0; ++j) {  // k = 1: radius factor 1/2^0 = 1  (:326-327)
             unsigned nxt = 0;
-            CU_TRY_M(try_round(cur, np, 1, j, &nxt));
+            CU_TRY(try_round(cur, np, 1, j, &nxt));
             np = nxt;
             cur ^= 1;
         }
@@ -699,19 +633,20 @@ int32_t kmc_make_theta0s(kmc_density_t density, const double *theta0, const doub
         // the first walker whose k = 1 tries all failed: the reference now shrinks the ball for it AND, because the
         // radius is never reset (:326), for every later walker -- which must therefore be redone
         unsigned f = 0xFFFFFFFFu;
-        CU_TRY_M(cudaMemset(d_cnt + 1, 0xFF, sizeof(unsigned)));
-        min_u32_kernel<<<(unsigned)std::min<long long>((np + 255) / 256, 1184), 256>>>(d_pend[cur], np, d_cnt + 1);
-        CU_TRY_M(cudaMemcpy(&f, d_cnt + 1, sizeof(unsigned), cudaMemcpyDeviceToHost));
+        CU_TRY(cudaMemset(d_cnt.get() + 1, 0xFF, sizeof(unsigned)));
+        min_u32_kernel<<<(unsigned)std::min<long long>((np + 255) / 256, 1184), 256>>>(d_pend[cur].get(), np,
+                                                                                        d_cnt.get() + 1);
+        CU_TRY(cudaMemcpy(&f, d_cnt.get() + 1, sizeof(unsigned), cudaMemcpyDeviceToHost));
         if ((long long)f + 1 < nw)
-            found_clear_kernel<<<(unsigned)((nw - f - 1 + 255) / 256), 256>>>(d_found, (long long)f + 1, nw);
+            found_clear_kernel<<<(unsigned)((nw - f - 1 + 255) / 256), 256>>>(d_found.get(), (long long)f + 1, nw);
         bool got = false;
         for (int k = 2; k <= ball_radius_halfing_steps && !got; ++k) {  // :324
             for (int c = 0; c < d; ++c) br[c] = br[c] * (1.0 / std::pow(2.0, k - 1));  // :326 cumulative
-            CU_TRY_M(cudaMemcpy(d_br, br.data(), sizeof(double) * d, cudaMemcpyHostToDevice));
+            CU_TRY(cudaMemcpy(d_br.get(), br.data(), sizeof(double) * d, cudaMemcpyHostToDevice));
             for (int j = 1; j <= ntries && !got; ++j) {
                 unsigned nxt = 0;
-                CU_TRY_M(cudaMemcpy(d_pend[0], &f, sizeof(unsigned), cudaMemcpyHostToDevice));
-                CU_TRY_M(try_round(0, 1, k, j, &nxt));
+                CU_TRY(cudaMemcpy(d_pend[0].get(), &f, sizeof(unsigned), cudaMemcpyHostToDevice));
+                CU_TRY(try_round(0, 1, k, j, &nxt));
                 got = nxt == 0;
             }
         }
@@ -719,24 +654,18 @@ int32_t kmc_make_theta0s(kmc_density_t density, const double *theta0, const doub
     }
 
     // :348  the found walkers, in walker order (fewer than nwalkers if some walker exhausted every try)
-    found_count_kernel<<<(unsigned)nblk, kKeepBlock>>>(d_found, nw, d_blk);
-    std::vector<unsigned> blk(2 * nblk);
-    CU_TRY_M(cudaMemcpy(blk.data(), d_blk, sizeof(unsigned) * nblk, cudaMemcpyDeviceToHost));
+    found_count_kernel<<<(unsigned)nblk, kKeepBlock>>>(d_found.get(), nw, d_blk.get());
     long long nf = 0;
-    for (long long b = 0; b < nblk; ++b) {
-        blk[nblk + b] = (unsigned)nf;
-        nf += blk[b];
-    }
+    if (const int32_t rc = compact_offsets(d_blk.get(), nblk, nullptr, nf); rc != KMC_OK) return rc;
     if (nf > 0) {
-        CU_TRY_M(cudaMemcpy(d_blk + nblk, blk.data() + nblk, sizeof(unsigned) * nblk, cudaMemcpyHostToDevice));
-        CU_TRY_M(dev_alloc(&d_out, sizeof(double) * nf * d, dev));
-        found_gather_kernel<<<(unsigned)nblk, kKeepBlock>>>(d_found, nw, d, d_blk + nblk, d_rows, d_out);
-        CU_TRY_M(cudaMemcpy(out, d_out, sizeof(double) * nf * d, cudaMemcpyDeviceToHost));
+        CU_TRY(dev_alloc(d_out, sizeof(double) * nf * d, dev));
+        found_gather_kernel<<<(unsigned)nblk, kKeepBlock>>>(d_found.get(), nw, d, d_blk.get() + nblk, d_rows.get(),
+                                                            d_out.get());
+        CU_TRY(cudaMemcpy(out, d_out.get(), sizeof(double) * nf * d, cudaMemcpyDeviceToHost));
     }
-    CU_TRY_M(cudaGetLastError());
-#undef CU_TRY_M
+    CU_TRY(cudaStreamSynchronize(nullptr));  // the blocks go back to the cache idle (nf = 0: the offsets' upload)
+    CU_TRY(cudaGetLastError());
     *nfound = nf;
-    cleanup();
     return KMC_OK;
 }
 

@@ -20,7 +20,6 @@ namespace kmc_host {
 // status + thread-local message (kmc_last_error)
 int32_t fail(int32_t code, const char *fmt, ...);
 const std::string &last_error();
-void set_last_error(const std::string &msg);
 
 // per-device cache of freed device blocks (kmc_trim releases them)
 cudaError_t dev_alloc_raw(void **out, size_t bytes, int device);
@@ -31,10 +30,38 @@ cudaError_t dev_alloc(T **out, size_t bytes, int device) {
 void dev_free(void *p);
 void cache_trim();
 
+// A device block owned by its scope: it goes back to the cache when the owner is destroyed, so every user must have
+// synchronised the block's stream by then.
+struct DevFree {
+    void operator()(void *p) const { dev_free(p); }
+};
+template <typename T>
+using DevBuf = std::unique_ptr<T, DevFree>;
+
+template <typename T>
+cudaError_t dev_alloc(DevBuf<T> &b, size_t bytes, int device) {
+    T *p = nullptr;
+    const cudaError_t e = dev_alloc(&p, bytes, device);
+    b.reset(p);
+    return e;
+}
+
+// Grows b, which holds `have` bytes, to at least `need` bytes; the contents are not kept.
+template <typename T>
+cudaError_t reserve(DevBuf<T> &b, size_t &have, size_t need, int device) {
+    if (need <= have) return cudaSuccess;
+    b.reset();
+    have = 0;
+    const cudaError_t e = dev_alloc(b, need, device);
+    if (e != cudaSuccess) return e;
+    have = need;
+    return cudaSuccess;
+}
+
 struct BatchScratch {
-    double *part = nullptr;
+    DevBuf<double> part;  // logistic: partial sums [chunks][npts]
     size_t bytes = 0;
-    __nv_bfloat16 *pieces = nullptr;  // tcgen05 path: theta split into 3 bf16 pieces [3][wpad][d]
+    DevBuf<__nv_bfloat16> pieces;  // tcgen05 path: theta split into 3 bf16 pieces [3][wpad][d]
     size_t pieces_bytes = 0;
 };
 
@@ -162,6 +189,10 @@ cudaError_t eval_on_device(const kmc_density_s &dn, const double *X, long long n
                            cudaStream_t st);
 // Kernels eval_on_device launches for this density.
 int eval_launches(const kmc_density_s &dn);
+
+// Walker-major copy of the stored chains to the host: thetas [nk][ns][d] and logp [nk][ns] (either may be NULL) for
+// the stored walkers idx[0, nk), or [0, nk) if idx is NULL, staged through <= 64 MiB.  Synchronises the stream once.
+int32_t chain_gather(kmc_sampler_s *s, const unsigned *idx, long long nk, double *thetas, double *logp);
 
 // A sampler under construction, deleted by kmc_emcee_destroy: every exit of a create call frees what was allocated.
 using SamplerPtr = std::unique_ptr<kmc_sampler_s, int32_t (*)(kmc_sampler_t)>;

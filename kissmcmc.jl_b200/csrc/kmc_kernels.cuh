@@ -794,16 +794,19 @@ static __global__ void __launch_bounds__(256) density_eval_kernel(const double *
 
 // Chain store is sample-major on the device ([ns][nw][D]); the ABI wants walker-major
 // ([nw][ns][D]).  Transposes walkers [w0, w0+wc), samples [s0, s0 + 32*gridDim.y) into a staging buffer.
+// INDEXED: walker w is stored row idx[w] (squash's kept walkers); else row w.
 constexpr long long kTransposeMaxSamples = 65535LL * 32;  // gridDim.y limit: longer chains take several launches
+template <bool INDEXED>
 static __global__ void chain_transpose_kernel(const double *__restrict__ in, double *__restrict__ out, long long ns,
-                                       long long nw, long long w0, long long wc, int d, long long s0) {
+                                       long long nw, long long w0, long long wc, int d, long long s0,
+                                       const unsigned *__restrict__ idx) {
     __shared__ double tile[32][33];
     // element (s, w) is a d-vector; handle one component per blockIdx.z
     const int c = blockIdx.z;
     const long long wb = (long long)blockIdx.x * 32, sb = s0 + (long long)blockIdx.y * 32;
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {
         const long long s = sb + r, w = wb + threadIdx.x;
-        if (s < ns && w < wc) tile[r][threadIdx.x] = in[(s * nw + (w0 + w)) * d + c];
+        if (s < ns && w < wc) tile[r][threadIdx.x] = in[(s * nw + (INDEXED ? (long long)idx[w0 + w] : w0 + w)) * d + c];
     }
     __syncthreads();
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {

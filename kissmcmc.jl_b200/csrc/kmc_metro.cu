@@ -201,19 +201,14 @@ int32_t kmc_metropolis_draws(uint64_t seed, int64_t chain0, int64_t nchains, int
     if (n == 0) return KMC_OK;
     if (!normals || !u) return fail(KMC_ERR_INVALID, "NULL output");
     CU_TRY(cudaSetDevice(device));
-    double *dn = nullptr, *du = nullptr;
-    CU_TRY(dev_alloc(&dn, sizeof(double) * n * d, device));
-    cudaError_t e = dev_alloc(&du, sizeof(double) * n, device);
-    if (e == cudaSuccess) {
-        const long long ne = n * ((d + 1) / 2);
-        kmc::mh_draws_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(kmc::philox_keys(seed), (unsigned)chain0, nchains, t0,
-                                                                     niters, d, dn, du);
-        e = cudaMemcpy(normals, dn, sizeof(double) * n * d, cudaMemcpyDeviceToHost);
-    }
-    if (e == cudaSuccess) e = cudaMemcpy(u, du, sizeof(double) * n, cudaMemcpyDeviceToHost);
-    dev_free(dn);
-    dev_free(du);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "metropolis_draws failed: %s", cudaGetErrorString(e));
+    DevBuf<double> dn, du;
+    CU_TRY(dev_alloc(dn, sizeof(double) * n * d, device));
+    CU_TRY(dev_alloc(du, sizeof(double) * n, device));
+    const long long ne = n * ((d + 1) / 2);
+    kmc::mh_draws_kernel<<<(unsigned)((ne + 255) / 256), 256>>>(kmc::philox_keys(seed), (unsigned)chain0, nchains, t0,
+                                                                 niters, d, dn.get(), du.get());
+    CU_TRY(cudaMemcpy(normals, dn.get(), sizeof(double) * n * d, cudaMemcpyDeviceToHost));
+    CU_TRY(cudaMemcpy(u, du.get(), sizeof(double) * n, cudaMemcpyDeviceToHost));
     return KMC_OK;
 }
 
@@ -226,18 +221,16 @@ int32_t kmc_emcee_chain_covariance(kmc_sampler_t s, double *mean, double *cov, i
     if (nrows < 1) return fail(KMC_ERR_STATE, "no samples stored");
     CU_TRY(cudaSetDevice(s->opts.device));
     const int P = (d + 1) * (d + 2) / 2;  // upper triangle over the d components and the constant column
-    double *part = nullptr, *sums = nullptr;
-    CU_TRY(dev_alloc(&part, sizeof(double) * ((size_t)kmc::kCovGrid + 1) * P, s->opts.device));
-    sums = part + (size_t)kmc::kCovGrid * P;
+    DevBuf<double> part;
+    CU_TRY(dev_alloc(part, sizeof(double) * ((size_t)kmc::kCovGrid + 1) * P, s->opts.device));
+    double *sums = part.get() + (size_t)kmc::kCovGrid * P;
     std::vector<double> h(P), shift(d);
-    kmc::mh_cov_partial_kernel<<<kmc::kCovGrid, kmc::kCovThreads, 0, s->stream>>>(s->chain_x, nrows, d, part);
-    kmc::mh_cov_final_kernel<<<(P + 255) / 256, 256, 0, s->stream>>>(part, P, kmc::kCovGrid, sums);
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(h.data(), sums, sizeof(double) * P, cudaMemcpyDeviceToHost, s->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
-    dev_free(part);
-    if (e != cudaSuccess) return fail(KMC_ERR_CUDA, "chain covariance failed: %s", cudaGetErrorString(e));
+    kmc::mh_cov_partial_kernel<<<kmc::kCovGrid, kmc::kCovThreads, 0, s->stream>>>(s->chain_x, nrows, d, part.get());
+    kmc::mh_cov_final_kernel<<<(P + 255) / 256, 256, 0, s->stream>>>(part.get(), P, kmc::kCovGrid, sums);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaMemcpyAsync(h.data(), sums, sizeof(double) * P, cudaMemcpyDeviceToHost, s->stream));
+    CU_TRY(cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream));
+    CU_TRY(cudaStreamSynchronize(s->stream));
     const int dc = d + 1;
     auto at = [&](int a, int b) { return h[(size_t)a * dc - (size_t)a * (a - 1) / 2 + (b - a)]; };  // a <= b
     const double n = (double)nrows;

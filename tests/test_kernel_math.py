@@ -140,15 +140,20 @@ def test_balanced_tiling_of_the_fused_gaussian_kernels_covers_every_walker_once(
         assert (ntiles - 1) * tr < W <= ntiles * tr
 
 
-def test_chain_transpose_launch_geometry_covers_long_chains():
-    """kmc_emcee_copy_results transposes the sample-major chain in launches of at most kTransposeMaxSamples samples
-    (gridDim.y <= 65535 blocks of 32 samples): every sample exactly once, for chains far beyond 2.09 M samples."""
+def test_chain_gather_launch_geometry_covers_long_chains():
+    """kmc_emcee_copy_results and the walker-major squash transpose the sample-major chain (chain_gather) in launches
+    of at most kTransposeMaxSamples samples (gridDim.y <= 65535 blocks of 32 samples): every sample exactly once, for
+    chains far beyond 2.09 M samples."""
     src = (CSRC / "kmc_kernels.cuh").read_text()
     m = re.search(r"kTransposeMaxSamples = (\d+)LL \* (\d+);", src)
     max_samples = int(m.group(1)) * int(m.group(2))
     assert max_samples == 65535 * 32
     api = (CSRC / "kmc_api.cu").read_text()
-    assert api.count("s0 += kmc::kTransposeMaxSamples") == 2          # thetas and logp both loop over sample chunks
+    gather = api[api.index("int32_t chain_gather("):]
+    gather = gather[:gather.index("\n}\n")]
+    assert api.count("s0 += kmc::kTransposeMaxSamples") == 1 and "s0 += kmc::kTransposeMaxSamples" in gather
+    assert "what == 0 ? s->chain_x : s->chain_lp" in gather            # thetas and logp both loop over sample chunks
+    assert "chain_gather(s, nullptr, nl, thetas, logp)" in api
     for ns in (1, 31, 32, max_samples - 1, max_samples, max_samples + 1, 5_000_000, 3 * max_samples + 7):
         covered = 0
         for s0 in range(0, ns, max_samples):
