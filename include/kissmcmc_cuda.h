@@ -185,14 +185,17 @@ int32_t kmc_emcee_nlocal(kmc_sampler_t s, int64_t *nl);
  * nl = nwalkers, or 2*shard_count for a sharded sampler (its slice of half 0, then of half 1). */
 int32_t kmc_emcee_copy_results(kmc_sampler_t s, double *thetas, double *logp,
                                double *accept_ratio);
-/* Posterior moments of the whole stored chain (all walkers squashed, src/samplers.jl:372-428),
+/* Posterior moments of the samples stored so far (all walkers squashed, src/samplers.jl:372-428),
  * reduced on the device: mean [d], unbiased variance [d], number of samples.  Avoids copying
- * chains of 10^9+ samples to the host. */
+ * chains of 10^9+ samples to the host.  Samples stored so far: those of the iterations run, the
+ * whole chain once the run is complete; an emcee iteration with one half-step left adds none.
+ * KMC_ERR_STATE while none is stored (before the first run, during burn-in). */
 int32_t kmc_emcee_chain_moments(kmc_sampler_t s, double *mean, double *var, int64_t *count);
-/* Covariance of the same rows as kmc_emcee_chain_moments (emcee or Metropolis handle): mean [d], unbiased covariance
- * cov [d][d] (ddof = 1, row-major, symmetric), number of samples; shifted by the first stored sample.  A fixed grid
- * and a fixed-order final sum: the result's bits depend only on the stored chain.  d <= 128, else
- * KMC_ERR_UNSUPPORTED.  The pilot-run estimate a correlated Metropolis proposal is tuned from. */
+/* Covariance of the same rows as kmc_emcee_chain_moments (emcee or Metropolis handle), the samples stored so far:
+ * mean [d], unbiased covariance cov [d][d] (ddof = 1, row-major, symmetric), number of samples; shifted by the first
+ * stored sample.  A fixed grid and a fixed-order final sum: the result's bits depend only on the stored chain.
+ * d <= 128, else KMC_ERR_UNSUPPORTED; KMC_ERR_STATE while no sample is stored.  The pilot-run estimate a correlated
+ * Metropolis proposal is tuned from. */
 int32_t kmc_emcee_chain_covariance(kmc_sampler_t s, double *mean, double *cov, int64_t *count);
 /* Current ensemble: theta [nw][d], logp [nw], naccept [nw]; any may be NULL. */
 int32_t kmc_emcee_copy_state(kmc_sampler_t s, double *theta, double *logp, int64_t *naccept);

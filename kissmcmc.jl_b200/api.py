@@ -255,13 +255,15 @@ class Sampler:
         return th, mean.value, lp, None
 
     def chain_moments(self):
-        """(mean[d], var[d], nsamples) of the whole stored chain, reduced on the device."""
+        """(mean[d], var[d], nsamples) of the samples stored so far (the whole chain once the run is complete; an
+        emcee iteration with one half-step left adds none), reduced on the device.  KmcError (code 4) while none is
+        stored."""
         mean, var, n = np.empty(self.d), np.empty(self.d), C.c_int64()
         check(lib.kmc_emcee_chain_moments(self._h, _ptr(mean), _ptr(var), C.byref(n)))
         return mean, var, n.value
 
     def chain_covariance(self):
-        """(mean[d], cov[d, d], nsamples) of the whole stored chain (the rows of chain_moments; unbiased, ddof=1),
+        """(mean[d], cov[d, d], nsamples) of the samples stored so far (the rows of chain_moments; unbiased, ddof=1),
         reduced on the device in a fixed order: the same chain gives the same bits.  d <= 128."""
         mean, cov, n = np.empty(self.d), np.empty((self.d, self.d)), C.c_int64()
         check(lib.kmc_emcee_chain_covariance(self._h, _ptr(mean), _ptr(cov), C.byref(n)))

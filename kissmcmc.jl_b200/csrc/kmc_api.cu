@@ -1242,7 +1242,7 @@ int32_t kmc_emcee_copy_results(kmc_sampler_t s, double *thetas, double *logp, do
 
 int32_t kmc_emcee_chain_moments(kmc_sampler_t s, double *mean, double *var, int64_t *count) {
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
-    const long long nrows = s->ns * s->nl;
+    const long long nrows = stored_samples(s) * s->nl;
     const int d = s->d;
     if (count) *count = nrows;
     if (nrows < 1) return fail(KMC_ERR_STATE, "no samples stored");
@@ -1252,7 +1252,11 @@ int32_t kmc_emcee_chain_moments(kmc_sampler_t s, double *mean, double *var, int6
     std::vector<double> h(2 * d), shift(d);
     CU_TRY(cudaMemsetAsync(sums.get(), 0, sizeof(double) * 2 * d, s->stream));
     const unsigned grid = (unsigned)std::min<long long>((nrows * d + 255) / 256, 148 * 8);
-    kmc::chain_moments_kernel<<<grid, 256, sizeof(double) * 2 * d, s->stream>>>(s->chain_x, nrows, d, sums.get());
+    const size_t smem = sizeof(double) * 2 * d;  // above 48 KiB (d > 3072) only with the opt-in
+    if (smem > (48u << 10))
+        CU_TRY(cudaFuncSetAttribute(kmc::chain_moments_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kmc::chain_moments_kernel<<<grid, 256, smem, s->stream>>>(s->chain_x, nrows, d, sums.get());
+    CU_TRY(cudaGetLastError());
     CU_TRY(cudaMemcpyAsync(h.data(), sums.get(), sizeof(double) * 2 * d, cudaMemcpyDeviceToHost, s->stream));
     CU_TRY(cudaMemcpyAsync(shift.data(), s->chain_x, sizeof(double) * d, cudaMemcpyDeviceToHost, s->stream));
     CU_TRY(cudaStreamSynchronize(s->stream));

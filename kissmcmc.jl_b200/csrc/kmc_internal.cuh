@@ -194,6 +194,14 @@ int eval_launches(const kmc_density_s &dn);
 // the stored walkers idx[0, nk), or [0, nk) if idx is NULL, staged through <= 64 MiB.  Synchronises the stream once.
 int32_t chain_gather(kmc_sampler_s *s, const unsigned *idx, long long nk, double *thetas, double *logp);
 
+// Complete samples stored so far per walker: the thinning clock after the iterations run (Metropolis: tdone steps;
+// emcee: hdone / 2, so an iteration with one half-step left adds no sample).  The store is sample-major, so they are
+// its first stored_samples(s) * nl rows; the rest of the ns planned samples hold whatever the block held before.
+inline long long stored_samples(const kmc_sampler_s *s) {
+    const long long t = s->metro ? s->tdone : s->hdone / 2;
+    return kmc::ThinClock<>::at(t, s->opts.nburnin_walker, s->opts.nthin).sidx;
+}
+
 // A sampler under construction, deleted by kmc_emcee_destroy: every exit of a create call frees what was allocated.
 using SamplerPtr = std::unique_ptr<kmc_sampler_s, int32_t (*)(kmc_sampler_t)>;
 

@@ -214,7 +214,7 @@ int32_t kmc_metropolis_draws(uint64_t seed, int64_t chain0, int64_t nchains, int
 
 int32_t kmc_emcee_chain_covariance(kmc_sampler_t s, double *mean, double *cov, int64_t *count) {
     if (!s) return fail(KMC_ERR_INVALID, "NULL sampler");
-    const long long nrows = s->ns * s->nl;  // the rows kmc_emcee_chain_moments reduces
+    const long long nrows = stored_samples(s) * s->nl;  // the rows kmc_emcee_chain_moments reduces
     const int d = s->d;
     if (count) *count = nrows;
     if (d > kmc::kCovMaxD) return fail(KMC_ERR_UNSUPPORTED, "chain covariance supports d <= %d, got d=%d", kmc::kCovMaxD, d);
