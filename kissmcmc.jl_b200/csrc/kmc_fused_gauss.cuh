@@ -312,13 +312,12 @@ gaussian_fused_kernel(const __grid_constant__ CUtensorMap mapA, const RunParams 
                     const unsigned i = p.shard_begin + w;
                     const size_t k = a0 + i;
                     const double p1 = fp.lognorm - 0.5 * ss;
-                    // :260 -- the FP32 filter of kmc_kernels.cuh decides exactly like the FP64 expression whenever
-                    // |tt| is above its rigorous margin; everything else takes the FP64 expression itself
+                    // :260 -- the FP32 filter of kmc_kernels.cuh decides exactly like the FP64 expression where
+                    // accept_decide lets it; everything else takes the FP64 expression itself
                     const double tt = (p1 - p0) + (double)sm.q[tpar][r] * 0.6931471805599453;
-                    bool acc;
-                    if (tt > (double)p.margin) acc = true;
-                    else if (tt < -(double)p.margin) acc = false;
-                    else acc = accept_exact<false>(p.nm1, sm.z[tpar][r], p1, p0, sm.u[tpar][r]);
+                    const bool acc = accept_decide(tt, p0, p.margin, [&] {
+                        return accept_exact<false>(p.nm1, sm.z[tpar][r], p1, p0, sm.u[tpar][r]);
+                    });
                     sm.acc[tpar][r] = acc ? 1 : 0;
                     if (acc || store) sm.list[tpar][atomicAdd(&sm.nlist[tpar], 1u)] = (unsigned char)r;
                     if (acc) {

@@ -236,10 +236,8 @@ gaussian_fused2_kernel(const RunParams p, const Fused2Params fp) {
                 const size_t k = a0 + i;
                 const double p1 = fp.lognorm - 0.5 * (double)ssf;
                 const double tt = (p1 - p0) + (double)sm.q[rb][r] * 0.6931471805599453;  // :260, FP32 filter of K1
-                bool acc;
-                if (tt > (double)p.margin) acc = true;
-                else if (tt < -(double)p.margin) acc = false;
-                else acc = accept_exact<false>(p.nm1, sm.z[rb][r], p1, p0, sm.u[rb][r]);
+                const bool acc = accept_decide(
+                    tt, p0, p.margin, [&] { return accept_exact<false>(p.nm1, sm.z[rb][r], p1, p0, sm.u[rb][r]); });
                 sm.acc[rb][r] = acc ? 1 : 0;
                 if (acc || store) sm.list[rb][atomicAdd(&sm.nlist[rb], 1u)] = (unsigned char)r;
                 if (acc) {

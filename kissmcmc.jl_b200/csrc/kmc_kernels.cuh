@@ -153,9 +153,12 @@ __device__ __forceinline__ void grid_join(const RunParams &p, unsigned long long
 // error of t is bounded by `margin` (set by the host: (N-1+64)*2e-6, >3x the worst case of
 // two MUFU.LG2 errors (2^-22.6 absolute on the mantissa part + one FP32 rounding of the
 // result), two FP64->FP32 input roundings and one FP32 fma, for |lg2 z| <= 4 and
-// |lg2 u| <= 100), so |t| > margin decides exactly like the FP64 expression.  Anything closer,
-// non-finite or outside that range (q = NaN) takes the exact FP64 path: the decisions are
-// those of the exact expression, bit for bit.
+// |lg2 u| <= 100).  The FP64 expression rounds too: (N-1)*log(z) + p1 is rounded to the ulp
+// of p1, which exceeds the margin once |p0| ~ 2^40 (the filter sees p1 - p0 exactly).  So
+// |t| > margin decides like the FP64 expression only while |p0| < kFilterMaxLogp = 2^36, where
+// that rounding stays below 2^-17 (tests/test_accept_filter_model.py derives the bound).
+// Anything closer, with a larger |p0|, non-finite or outside the logs' range (q = NaN) takes
+// the exact FP64 path: the decisions are those of the exact expression, bit for bit.
 template <bool SKIP_LOGZ>
 __device__ __forceinline__ bool accept_exact(double nm1, double z, double p1, double p0, double u) {
     double lhs;
@@ -208,6 +211,19 @@ __device__ __forceinline__ bool accept_slow(const RunParams &p, long long h, uns
     double z2, u;
     step_draws<REPLAY>(p, h, i, j, z2, u);
     return accept_exact<SKIP_LOGZ>(p.nm1, z, p1, p0, u);
+}
+
+// The decision of every filtered kernel: tt = (p1 - p0) + ln2*q (q from filter_q) decides alone where the FP64
+// expression provably agrees with it (see accept_exact); everything else calls exact(), accept_slow or accept_exact.
+// The |p0| bound costs the bench line (K1, 2^20 2-D walkers) ~0.2 % on a B200 at 1000 W.
+constexpr double kFilterMaxLogp = 68719476736.0;  // 2^36
+template <class Exact>
+__device__ __forceinline__ bool accept_decide(double tt, double p0, float margin, Exact &&exact) {
+    if (fabs(p0) < kFilterMaxLogp) {  // false for NaN
+        if (tt > (double)margin) return true;
+        if (tt < -(double)margin) return false;
+    }
+    return exact();
 }
 
 struct DrawRec {  // what a walker-step needs from its draws: 4 registers
@@ -404,10 +420,9 @@ static __global__ void __launch_bounds__(max_threads<D>(), min_blocks<D>()) emce
                 for (int c = 0; c < D; ++c) y[c] = stretch_coord(xj[q][c], xk[q][c], z);  // :255
                 const double p1 = dn.logpdf(y);                                            // :257
                 const double tt = (p1 - lpk[q]) + (double)dr[q].q * 0.6931471805599453;  // :260
-                bool acc;
-                if (tt > (double)p.margin) acc = true;
-                else if (tt < -(double)p.margin) acc = false;
-                else acc = accept_slow<REPLAY, (D == 1 && !REPLAY)>(p, h, base + l, z, p1, lpk[q]);
+                const bool acc = accept_decide(tt, lpk[q], p.margin, [&] {
+                    return accept_slow<REPLAY, (D == 1 && !REPLAY)>(p, h, base + l, z, p1, lpk[q]);
+                });
                 if (acc) {  // :261-265
                     store_row<D>(p.x + k * D, y);
                     p.lp[k] = p1;
@@ -538,10 +553,8 @@ static __global__ void __launch_bounds__(kBulkThreads, KMC_BULK_CTAS) emcee_bulk
                 for (int c = 0; c < D; ++c) y[c] = stretch_coord(xj[c], xk[c], z);  // :255
                 const double p1 = dn.logpdf(y);                                      // :257
                 const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;   // :260
-                bool acc;
-                if (tt > (double)p.margin) acc = true;
-                else if (tt < -(double)p.margin) acc = false;
-                else acc = accept_slow<false, false>(p, h, base + l, z, p1, lpk);
+                const bool acc =
+                    accept_decide(tt, lpk, p.margin, [&] { return accept_slow<false, false>(p, h, base + l, z, p1, lpk); });
                 if (acc) {  // :261-265
 #if KMC_BULK_STORE_ALL
 #pragma unroll
@@ -747,10 +760,9 @@ static __global__ void __launch_bounds__(kSmemThreads, kSmemCtas) emcee_smem_ker
                 load_row_cg<D>(p.x + (size_t)dr[(q + kAhead) % kRounds].j * D, xj[q % kAhead]);
             const double p1 = dn.logpdf(y);                                        // :257
             const double tt = (p1 - lpk) + (double)dr[q].q * 0.6931471805599453;  // :260
-            bool acc;
-            if (tt > (double)p.margin) acc = true;
-            else if (tt < -(double)p.margin) acc = false;
-            else acc = accept_slow<REPLAY, (D == 1 && !REPLAY)>(p, h, wid + q * nthr, z, p1, lpk);
+            const bool acc = accept_decide(tt, lpk, p.margin, [&] {
+                return accept_slow<REPLAY, (D == 1 && !REPLAY)>(p, h, wid + q * nthr, z, p1, lpk);
+            });
             if (acc) {  // :261-265
                 store_row<D>(grow + ro * D, y);
 #pragma unroll

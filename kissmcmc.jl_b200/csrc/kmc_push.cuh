@@ -599,10 +599,8 @@ __global__ void __launch_bounds__(kPushThreads, KMC_PUSH_CTAS) emcee_push_kernel
                     for (int cc = 0; cc < D; ++cc) y[cc] = stretch_coord(xj[cc], xk[cc], z);  // :255
                     const double p1 = dn.logpdf(y);                                          // :257
                     const double tt = (p1 - lpk) + (double)dr.q * 0.6931471805599453;       // :260
-                    bool acc;
-                    if (tt > (double)p.margin) acc = true;
-                    else if (tt < -(double)p.margin) acc = false;
-                    else acc = accept_slow<false, false>(p, h, me * S + l, z, p1, lpk);
+                    const bool acc = accept_decide(tt, lpk, p.margin,
+                                                   [&] { return accept_slow<false, false>(p, h, me * S + l, z, p1, lpk); });
                     if (acc) {  // :261-265: only accepted rows are written (the kernel is bound by its DRAM traffic)
                         store_row<D>(p.x + k * D, y);
                         p.lp[k] = p1;
