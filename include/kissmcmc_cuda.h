@@ -102,6 +102,13 @@ int32_t kmc_trim(void);
  *                                           memory up to d = 128 and in L2 beyond)
  *   "lognormal"    test/runtests.jl:56      params: [mu, sigma, log(sigma)+0.5*log(2pi)], d = 1
  *   "logistic"     BASELINE.json config 4   params: [prior_sigma]; data: float32 X[N][d] then y[N]; any d <= 512
+ *   "gaussian_mixture"  sum_k w_k MvNormal(mu_k, Sigma_k)   params: K components of q = d + d(d+1)/2 + 1 doubles,
+ *                                           each [mu_k(d), upper triangle of A_k = chol(Sigma_k^-1)^T row by row (row i
+ *                                           holds j = i..d-1, diagonal > 0), c_k = log(w_k/sum w) + lognorm_k];
+ *                                           logp = logsumexp_k(c_k - 0.5*|A_k (x-mu_k)|^2); d in {1..6, 8, 10, 12, 16},
+ *                                           1 <= K <= Kmax(d) = floor(272/q): 90, 45, 27, 18, 12, 9, 6, 4, 2, 1 for
+ *                                           d = 1, 2, 3, 4, 5, 6, 8, 10, 12, 16 (KMC_ERR_UNSUPPORTED beyond; nparams not a
+ *                                           multiple of q, a non-finite value or a diagonal entry <= 0: KMC_ERR_INVALID)
  * `data` may be NULL.  params/data are copied; the caller may free them on return. */
 int32_t kmc_density_create(const char *name, int32_t d, const double *params, int64_t nparams,
                            const void *data, int64_t data_bytes, int32_t device,

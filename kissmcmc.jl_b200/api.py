@@ -107,6 +107,61 @@ def gaussian(mean, cov, device: int = 0) -> LogDensity:
     return LogDensity("gaussian", mu.size, gaussian_params(mean, cov), device=device)
 
 
+def gaussian_mixture_params(weights, means, covs) -> np.ndarray:
+    """The parameters of the "gaussian_mixture" plugin: per component k, [mu_k, the upper triangle of A_k row by row,
+    log(w_k / sum w) + lognorm_k], with mu_k, A_k and lognorm_k as gaussian_params computes them.
+    weights [K] (finite, > 0; normalised here), means [K, d] (or [K] for d = 1), covs [K, d, d] symmetric positive
+    definite (or [K] variances for d = 1).  ValueError names the offending component."""
+    w = np.asarray(weights, dtype=np.float64)
+    if w.ndim != 1 or w.size < 1:
+        raise ValueError(f"weights must be a non-empty vector, got shape {w.shape}")
+    K = w.size
+    mus = np.asarray(means, dtype=np.float64)
+    mus = mus.reshape(K, 1) if mus.shape == (K,) else mus
+    if mus.ndim != 2 or mus.shape[0] != K:
+        raise ValueError(f"means must have shape [K, d] (or [K] for d = 1) with K = {K}, got {np.shape(means)}")
+    d = mus.shape[1]
+    cv = np.asarray(covs, dtype=np.float64)
+    cv = cv.reshape(K, 1, 1) if d == 1 and cv.shape == (K,) else cv
+    if cv.shape != (K, d, d):
+        raise ValueError(f"covs must have shape [{K}, {d}, {d}]" + (f" (or [{K}] variances)" if d == 1 else "") +
+                         f", got {np.shape(covs)}")
+    total = 0.0
+    for k in range(K):
+        if not (math.isfinite(w[k]) and w[k] > 0.0):
+            raise ValueError(f"component {k}: weight {w[k]} is not finite and > 0")
+        total += w[k]
+    upper = np.triu_indices(d)      # row by row, j = i .. d-1
+    out = []
+    for k in range(K):
+        c = cv[k]
+        if not (np.all(np.isfinite(c)) and np.all(np.isfinite(mus[k]))):
+            raise ValueError(f"component {k}: mean or covariance is not finite")
+        if not np.allclose(c, c.T, rtol=1e-12, atol=1e-14 * np.abs(c).max()):
+            raise ValueError(f"component {k}: covariance is not symmetric")
+        try:
+            np.linalg.cholesky(0.5 * (c + c.T))
+        except np.linalg.LinAlgError:
+            raise ValueError(f"component {k}: covariance is not positive definite") from None
+        g = gaussian_params(mus[k], c)
+        A, lognorm = g[d:d + d * d].reshape(d, d), g[-1]
+        out.append(np.concatenate([mus[k], A[upper], [math.log(w[k] / total) + lognorm]]))
+    return np.concatenate(out)
+
+
+def gaussian_mixture(weights, means, covs, device: int = 0) -> LogDensity:
+    """MixtureModel(MvNormal.(means, covs), weights): logp(x) = logsumexp_k(log w_k + log N(x; mu_k, Sigma_k)), weights
+    normalised to sum 1.  Shapes and checks as gaussian_mixture_params.  Fused kernels for d in {1..6, 8, 10, 12, 16}
+    with at most Kmax(d) = floor(272 / (d + d(d+1)/2 + 1)) components:
+        d     1   2   3   4   5   6   8  10  12  16
+        Kmax 90  45  27  18  12   9   6   4   2   1
+    (KmcError, code 3, at any other d or beyond Kmax).  Exact FP64; with K = 1 it equals gaussian(mean, cov) bit for
+    bit at finite x."""
+    p = gaussian_mixture_params(weights, means, covs)
+    d = np.asarray(means).reshape(len(np.atleast_1d(weights)), -1).shape[1]
+    return LogDensity("gaussian_mixture", d, p, device=device)
+
+
 def lognormal(mu: float = 0.0, sigma: float = 1.0, device: int = 0) -> LogDensity:
     """LogNormal(mu, sigma) (test/runtests.jl:56)."""
     return LogDensity("lognormal", 1, [mu, sigma, math.log(sigma) + 0.5 * math.log(2 * math.pi)], device=device)

@@ -9,7 +9,8 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libkissmcmc_cuda.so"
-SOURCES = ["kmc_api.cu", "kmc_aux.cu", "kmc_metro.cu", "kmc_ops_exp.cu", "kmc_ops_gauss.cu", "kmc_ops_misc.cu"]
+SOURCES = ["kmc_api.cu", "kmc_aux.cu", "kmc_metro.cu", "kmc_ops_exp.cu", "kmc_ops_gauss.cu", "kmc_ops_misc.cu",
+           "kmc_ops_mix.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 LINK_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "static"]
 

@@ -128,6 +128,7 @@ bool find_ops(int kind, int d, Ops &o) {
             return true;
         case kmc::KIND_ROSENBROCK: return ops_rosenbrock(d, o);
         case kmc::KIND_LOGNORMAL: return ops_lognormal(d, o);
+        case kmc::KIND_GAUSSIAN_MIXTURE: return ops_gaussian_mixture(d, o);  // no batched path: other d are unsupported
         default: return false;
     }
 }
@@ -139,7 +140,34 @@ int kind_of(const char *name) {
     if (!strcmp(name, "gaussian")) return kmc::KIND_GAUSSIAN;
     if (!strcmp(name, "lognormal")) return kmc::KIND_LOGNORMAL;
     if (!strcmp(name, "logistic")) return kmc::KIND_LOGISTIC;
+    if (!strcmp(name, "gaussian_mixture")) return kmc::KIND_GAUSSIAN_MIXTURE;
     return -1;
+}
+
+// A mixture's parameters: K whole components of mix_q(d) doubles, 1 <= K <= mix_kmax(d), every value finite and every
+// diagonal entry of every A_k > 0.  On success K is in *ncomp.
+int32_t check_mixture(int d, const double *params, int64_t nparams, int &ncomp) {
+    const int q = kmc::mix_q(d), kmax = kmc::mix_kmax(d);
+    if (nparams < q || nparams % q)
+        return fail(KMC_ERR_INVALID, "gaussian_mixture with d=%d takes K*%d parameters (mu, upper triangle of A, c per "
+                                     "component), got %lld", d, q, (long long)nparams);
+    const int64_t K = nparams / q;
+    if (K > kmax)
+        return fail(KMC_ERR_UNSUPPORTED, "gaussian_mixture with d=%d holds at most Kmax=%d components, got %lld", d, kmax,
+                    (long long)K);
+    for (int64_t i = 0; i < nparams; ++i)
+        if (!std::isfinite(params[i]))
+            return fail(KMC_ERR_INVALID, "gaussian_mixture parameter %lld (component %lld) is not finite", (long long)i,
+                        (long long)(i / q));
+    for (int64_t k = 0; k < K; ++k) {
+        const double *a = params + k * q + d;  // row i of A_k starts with its diagonal entry
+        for (int i = 0; i < d; a += d - i, ++i)
+            if (!(a[0] > 0.0))
+                return fail(KMC_ERR_INVALID, "gaussian_mixture component %lld: diagonal entry %d of A is not > 0",
+                            (long long)k, i);
+    }
+    ncomp = (int)K;
+    return KMC_OK;
 }
 
 // CTAs of `kern` resident per SM, or 0 if the query fails (its error is cleared).
@@ -620,7 +648,10 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
     Ops ops;
     if (!find_ops(kind, d, ops))
         return fail(KMC_ERR_UNSUPPORTED, "no sm_100a kernel for plugin '%s' with d=%d", name, d);
-    if (nparams != ops.nparams)
+    int ncomp = 0;
+    if (kind == kmc::KIND_GAUSSIAN_MIXTURE) {
+        if (const int32_t rc = check_mixture(d, params, nparams, ncomp); rc != KMC_OK) return rc;
+    } else if (nparams != ops.nparams)
         return fail(KMC_ERR_INVALID, "plugin '%s' with d=%d takes %d parameters, got %lld", name, d,
                     ops.nparams, (long long)nparams);
     // the density under construction, deleted by kmc_density_destroy on every exit but the last
@@ -635,6 +666,7 @@ int32_t kmc_density_create(const char *name, int32_t d, const double *params, in
         const double T = std::fabs(params[2]);
         h->params[3] = (T > 0x1p-100 && T < 0x1p100) ? 1.0 / params[2] : 0.0;
     }
+    if (kind == kmc::KIND_GAUSSIAN_MIXTURE) h->params[kmc::kMixSlots] = ncomp;  // K after the component bank
     if (ops.batch) {  // batched plugins keep parameters (and data) in device memory
         if (nparams) h->params.assign(params, params + nparams);
         CU_TRY(cudaSetDevice(device));

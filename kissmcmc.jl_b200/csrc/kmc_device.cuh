@@ -267,6 +267,75 @@ struct LogNormal {
     }
 };
 
+// Gaussian mixture sum_k w_k N(mu_k, Sigma_k), K components in a fixed bank of kMixSlots doubles (the size of
+// Gaussian<16>'s parameters, so every kernel family keeps its parameters under 4 KB) plus K, host-filled.  Component
+// k takes q(D) = D + D(D+1)/2 + 1 doubles: mu_k[D], the upper triangle of A_k = chol(Sigma_k^-1)^T row by row (row i
+// holds j = i .. D-1), c_k = log(w_k / sum w) + lognorm_k.  Operation order (mixture_oracle/ restates it):
+//   y_i = 0; y_i += A_k[i][j] (x_j - mu_k[j]), j ascending;  ss = 0; ss += y_i y_i;  l_k = c_k - 0.5 ss
+//   m = max_k l_k (NaN propagates); m NaN or -Inf: return m;  s = 0; s += exp(l_k - m), k ascending;  m + log(s).
+// With K = 1 this is the Gaussian plugin bit for bit at finite x: its below-diagonal products are +-0 added to +0,
+// exp(0) = 1 and log(1) = 0.
+constexpr int KIND_GAUSSIAN_MIXTURE = 5;
+constexpr int kMixSlots = 272;
+__host__ __device__ constexpr int mix_q(int d) { return d + d * (d + 1) / 2 + 1; }
+__host__ __device__ constexpr int mix_kmax(int d) { return kMixSlots / mix_q(d); }
+
+template <int D>
+struct GaussianMixture {
+    static constexpr int kind = KIND_GAUSSIAN_MIXTURE;
+    static constexpr int nparams = kMixSlots;  // the capacity: the host takes K * mix_q(D) of them, 1 <= K <= kmax
+    static constexpr int Q = mix_q(D);
+    static constexpr int kmax = mix_kmax(D);
+    static_assert(kmax >= 1, "one component must fit the parameter bank");
+    // the first kHeld l_k stay in registers between the two passes; later components are evaluated again (the same
+    // bits), so the register count does not grow with kmax
+    static constexpr int kHeld = kmax < 4 ? kmax : 4;
+    double p[kMixSlots + 1];  // components, then K
+
+    __device__ __forceinline__ double component(int k, const double (&x)[D]) const {
+        const double *pk = p + k * Q;
+        double c[D];
+#pragma unroll
+        for (int j = 0; j < D; ++j) c[j] = dsub(x[j], pk[j]);
+        double ss = 0.0;
+        int a = D;
+#pragma unroll
+        for (int i = 0; i < D; ++i) {
+            double y = 0.0;
+#pragma unroll
+            for (int j = i; j < D; ++j) y = dadd(y, dmul(pk[a++], c[j]));
+            ss = dadd(ss, dmul(y, y));
+        }
+        return dsub(pk[Q - 1], dmul(0.5, ss));
+    }
+
+    __device__ __forceinline__ double logpdf(const double (&x)[D]) const {
+        const int K = (int)p[kMixSlots];
+        double held[kHeld];
+        double m = -CUDART_INF;
+#pragma unroll
+        for (int k = 0; k < kHeld; ++k) {
+            if (k < K) {
+                held[k] = component(k, x);
+                m = (held[k] > m || held[k] != held[k]) ? held[k] : m;
+            }
+        }
+#pragma unroll 1
+        for (int k = kHeld; k < K; ++k) {
+            const double l = component(k, x);
+            m = (l > m || l != l) ? l : m;
+        }
+        if (m != m || m == -CUDART_INF) return m;
+        double s = 0.0;
+#pragma unroll
+        for (int k = 0; k < kHeld; ++k)
+            if (k < K) s = dadd(s, exp(dsub(held[k], m)));
+#pragma unroll 1
+        for (int k = kHeld; k < K; ++k) s = dadd(s, exp(dsub(component(k, x), m)));
+        return dadd(m, log(s));
+    }
+};
+
 // ------------------------------------------------------------------ row access
 // Walker rows are contiguous ([nw][D] row-major): a partner gather touches ceil(8D/32)
 // sectors instead of D sectors with a component-major layout, and for even D the active

@@ -38,6 +38,7 @@ bool ops_exponential(int d, Ops &o);
 bool ops_gaussian(int d, Ops &o);     // the fused FP64 Gaussian, d <= 16
 bool ops_rosenbrock(int d, Ops &o);
 bool ops_lognormal(int d, Ops &o);
+bool ops_gaussian_mixture(int d, Ops &o);  // the same dimensions as ops_gaussian
 
 }  // namespace kmc_host
 

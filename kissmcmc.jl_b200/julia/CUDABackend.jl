@@ -17,7 +17,7 @@
 # and the GPU parity tests.
 module CUDABackend
 
-export LogDensity, exponential, rosenbrock, gaussian, lognormal, logistic, set_option!, info, emcee, emcee_squashed,
+export LogDensity, exponential, rosenbrock, gaussian, gaussian_mixture, lognormal, logistic, set_option!, info, emcee, emcee_squashed,
        make_theta0s, g_pdf, cdf_g_inv, sample_g, NormalProposal, MvNormalProposal, normal_proposal, metropolis
 
 using LinearAlgebra: cholesky, Symmetric, diag, inv
@@ -96,6 +96,38 @@ function gaussian(mean, cov; device=0)
     lognorm = sum(log.(diag(Lc))) - 0.5 * d * log(2pi)
     params = vcat(mu, vec(permutedims(A)), lognorm)          # A row-major
     return LogDensity("gaussian", d, params; device=device)
+end
+"""
+    gaussian_mixture(weights, means, covs; device=0)
+
+`MixtureModel(MvNormal.(means, covs), weights)`: `weights` (K, each > 0, normalised here), `means` (K vectors of length
+d, or K numbers for d = 1), `covs` (K symmetric positive definite d x d matrices, or K variances for d = 1).
+params = per component [mu_k; upper triangle of A_k = chol(inv(Sigma_k))' row by row; log(w_k / sum w) + lognorm_k],
+the per-component math of `gaussian`.  Fused kernels for d in {1..6, 8, 10, 12, 16} with K <= Kmax(d) =
+floor(272 / (d + d(d+1)/2 + 1)): 90, 45, 27, 18, 12, 9, 6, 4, 2, 1 (KmcError 3 otherwise).  Like the rest of this
+module it has not been executed (no Julia in the build image); the Python `gaussian_mixture` packs the same layout.
+"""
+function gaussian_mixture(weights, means, covs; device=0)
+    K = length(weights)
+    (length(means) == K && length(covs) == K) || throw(ArgumentError("weights, means and covs need one entry per component"))
+    all(w -> isfinite(w) && w > 0, weights) || throw(ArgumentError("every weight must be finite and > 0"))
+    total = sum(Float64.(weights))
+    d = length(vcat(means[1]))
+    params = Float64[]
+    for k in 1:K
+        mu = Float64.(vcat(means[k]))
+        length(mu) == d || throw(ArgumentError("component $(k - 1): mean has length $(length(mu)), expected $d"))
+        prec = inv(reshape(Float64.(collect(covs[k])), d, d))
+        Lc = cholesky(Symmetric((prec + prec') / 2)).L      # prec = L L'
+        A = Matrix(Lc')                                      # upper triangular, y = A (x - mu)
+        lognorm = sum(log.(diag(Lc))) - 0.5 * d * log(2pi)
+        append!(params, mu)
+        for i in 1:d, j in i:d                               # row by row, j = i .. d
+            push!(params, A[i, j])
+        end
+        push!(params, log(weights[k] / total) + lognorm)
+    end
+    return LogDensity("gaussian_mixture", d, params; device=device)
 end
 "LogNormal(mu, sigma) (test/runtests.jl:56)"
 lognormal(mu=0.0, sigma=1.0; device=0) =
